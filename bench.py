@@ -22,6 +22,13 @@ One JSON line on stdout (rank 0):
   stack     configs[2]: 512 chained 4096^2 pairs, strong-scaled over the N GPUs (tvl1_stack_run)
   volume    configs[4]-style: chained 6144^2 slices per GPU, matches only (no flow download)
   cpu_baseline  the C oracle (oracle/, OpenMP) on a bounded crop of the same pair
+
+--dump-outputs DIR writes what the timed path returned in its last timed step, so that two builds run
+with the same arguments (hence the same seeded inputs) can be compared output for output:
+  u.npy, v.npy      the flow planes (float32), whole when both fit in DUMP_BYTES, else the same fixed
+                    seeded sample of pixels from each (flat row-major indices, see dump_index)
+  iterations.npy    the iteration count of every (level, warp) (float64)
+Only rank 0 writes.
 """
 import argparse
 import ctypes as C
@@ -43,6 +50,30 @@ from fibsem_optflow_b200 import synth  # noqa: E402
 METRIC = "tvl1_flow_mpx_per_s"
 UNIT = "Mpx/s"
 CPU_CROP = 2048          # the CPU legs run a CPU_CROP^2 crop of the pair (bounded sample)
+DUMP_BYTES = 64 << 20    # --dump-outputs: at most this much in all
+DUMP_SAMPLE = 4 << 20    # pixels drawn per flow plane when the planes are larger than DUMP_BYTES
+
+
+def dump_index(npx):
+    """Flat pixel indices --dump-outputs keeps of an npx-pixel flow plane: None (all of them) when both
+    float32 planes fit in DUMP_BYTES, else a fixed seeded draw, sorted and without repeats."""
+    if 2 * 4 * npx <= DUMP_BYTES:
+        return None
+    return np.unique(np.random.default_rng(0).integers(0, npx, DUMP_SAMPLE))
+
+
+def dump_outputs(d, u, v, iters):
+    """Writes d/u.npy, d/v.npy (float32; u and v are NumPy arrays or torch tensors) and d/iterations.npy."""
+    idx = dump_index(u.numel() if hasattr(u, "numel") else u.size)
+    out = {}
+    for name, a in (("u", u), ("v", v)):
+        if idx is not None:
+            a = a.reshape(-1)[idx]
+        out[name] = np.asarray(a.cpu() if hasattr(a, "cpu") else a, dtype=np.float32)
+    out["iterations"] = np.asarray(iters, dtype=np.float64)
+    os.makedirs(d, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 def workload(args):
@@ -141,10 +172,10 @@ def cpu_leg(args, steps, warmup, crop=CPU_CROP):
     cores = os.cpu_count() or 1
     p = O.default_params(nscales=args.scales, warps=args.warps, nthreads=cores)
     times = []
-    iters = None
+    u = v = iters = None
     for i in range(warmup + steps):
         t = time.perf_counter()
-        _, _, iters, _ = O.tvl1_calc(c0, c1, params=p)
+        u, v, iters, lev = O.tvl1_calc(c0, c1, params=p)
         dt = time.perf_counter() - t
         if i >= warmup:
             times.append(dt)
@@ -153,15 +184,17 @@ def cpu_leg(args, steps, warmup, crop=CPU_CROP):
             "sample": "center %dx%d crop of the %dx%d pair, same parameters, %d step(s), "
                       "%d total iterations" % (n, n, args.size, args.size, len(times),
                                                int(iters[iters >= 0].sum())),
-            "ms_per_step": total / len(times) * 1e3}
+            "ms_per_step": total / len(times) * 1e3, "outputs": (u, v, iters[:lev])}
 
 
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return 0
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, max(0, args.warmup)
     cb = cpu_leg(args, steps, min(warmup, 1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *cb["outputs"])
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT,
             "n_gpus": args.gpus, "steps": steps, "warmup": min(warmup, 1),
             "ms_per_step": cb["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -219,7 +252,7 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.SUM)
         return float(t.item())
 
-    K, W = max(1, args.steps), max(3, args.warmup)
+    K, W = args.steps, max(3, args.warmup)
     S = args.size
     I0, I1 = make_pair(args, rank)
     solver = N.Solver(N.default_params(lambda_=0.15, nscales=args.scales, warps=args.warps,
@@ -273,6 +306,8 @@ def run_ours(args):
     alg_bytes = stats.algorithmic_bytes
     stage_ms = {"total": stats.ms_total, "pyramid": stats.ms_pyramid, "warp": stats.ms_warp,
                 "iterate": stats.ms_iterate, "median": stats.ms_median, "other": stats.ms_other}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, du, dv, iters_last)
 
     # this box's own copy bandwidth, measured the way MEASURED_PEAKS.json was (context only:
     # boxes of the pool differ by ~20 %; roofline.frac stays against the driver-written peak)
@@ -536,7 +571,10 @@ def main():
     ap.add_argument("--stack-size", type=int, default=4096)
     ap.add_argument("--volume-pairs", type=int, default=16, help="configs[4] leg: pairs per GPU, matches only (0 = off)")
     ap.add_argument("--volume-size", type=int, default=6144)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

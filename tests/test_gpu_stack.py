@@ -25,7 +25,7 @@ def test_stack_flows_and_matches(gpu, orc):
             assert np.array_equal(got[j], want[j])
 
 
-def test_stack_debug_stream_continues(gpu, orc):
+def test_stack_debug_stream_continues(gpu, orc, tmp_path):
     """seed < 0: the reference's debug mode never calls srand, so pair k's shuffle starts where
     pair k-1's stopped.  The oracle reproduces that with real glibc rand() in a fresh process."""
     import json, os, subprocess, sys
@@ -33,16 +33,17 @@ def test_stack_debug_stream_continues(gpu, orc):
     s = gpu.Solver(gpu.default_params(lambda_=0.15, nscales=2))
     res = s.run_stack(slices, flows=True, npoints=6, scale=1.0, seed=-1)
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    np.savez("/tmp/_stack_dbg.npz", slices=np.stack(slices), u=np.stack(res["u"]), v=np.stack(res["v"]))
+    npz = str(tmp_path / "stack_dbg.npz")
+    np.savez(npz, slices=np.stack(slices), u=np.stack(res["u"]), v=np.stack(res["v"]))
     code = (
         "import sys, json; sys.path.insert(0, %r)\n"
         "import numpy as np\n"
         "from oracle import oracle as O\n"
-        "d = np.load('/tmp/_stack_dbg.npz'); out = []\n"
+        "d = np.load(%r); out = []\n"
         "for k in range(3):\n"
         "    r = O.random_points(d['slices'][k], d['slices'][k+1], d['u'][k], d['v'][k], scale=1.0, npoints=6, seed=-1)\n"
         "    out.append([a.tolist() for a in r[:5]])\n"
-        "print(json.dumps(out))\n" % root)
+        "print(json.dumps(out))\n" % (root, npz))
     want = json.loads(subprocess.check_output([sys.executable, "-c", code]).decode())
     for k in range(3):
         for j in range(5):
