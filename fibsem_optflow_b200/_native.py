@@ -84,6 +84,7 @@ EXPORTS = [
     "tvl1_mask_flow_u8", "tvl1_finish_flow_u8", "tvl1_sample_matches", "tvl1_sample_matches_skip", "tvl1_sample_matches_ex",
     "tvl1_default_feature_params", "tvl1_find_alignment", "tvl1_warp_affine_u8", "tvl1_warp_affine_f32", "tvl1_stack_run", "tvl1_k_convert_u8", "tvl1_k_resize",
     "tvl1_k_centered_gradient", "tvl1_k_warp", "tvl1_k_iterate", "tvl1_k_iterate_fused2", "tvl1_k_outer", "tvl1_k_iterate_gamma", "tvl1_k_median5", "tvl1_k_median3", "tvl1_k_last_ms",
+    "tvl1_k_gauss7_u8", "tvl1_k_fast_corners", "tvl1_k_describe", "tvl1_k_knn2", "tvl1_features_extract",
     "tvl1_pyramid_sizes", "tvl1_glibc_rand", "tvl1_selftest_arith", "tvl1_dev_count", "tvl1_dev_alloc", "tvl1_dev_free",
     "tvl1_dev_memset", "tvl1_dev_h2d", "tvl1_dev_d2h", "tvl1_dev_sync", "tvl1_set_device", "tvl1_stream_create",
     "tvl1_stream_destroy", "tvl1_stream_sync", "tvl1_stream_query", "tvl1_stream_wait", "tvl1_dev_h2d_async", "tvl1_dev_d2h_async",
@@ -160,6 +161,12 @@ def lib():
     L.tvl1_k_median5.argtypes = [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp]
     L.tvl1_k_median3.argtypes = L.tvl1_k_median5.argtypes
     L.tvl1_k_last_ms.argtypes = [C.POINTER(C.c_float)]
+    L.tvl1_k_gauss7_u8.argtypes = [_vp, _sz, C.c_int, C.c_int, _vp, _sz, _vp]
+    L.tvl1_k_fast_corners.argtypes = [_vp, _sz, C.c_int, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _vp, C.c_int, _vp, _vp, _vp]
+    L.tvl1_k_describe.argtypes = [_vp, _sz, _vp, _sz, _vp, C.c_int, C.c_float, C.c_int, _vp, _vp, _vp]
+    L.tvl1_k_knn2.argtypes = [_vp, C.c_int, _vp, C.c_int, _vp, _vp, _vp, _vp]
+    L.tvl1_features_extract.argtypes = [_vp, _vp, _sz, C.c_int, C.c_int, C.POINTER(FeatureParams), _vp, _vp, C.c_int,
+                                        C.POINTER(C.c_int), _vp]
     L.tvl1_pyramid_sizes.argtypes = [C.c_int, C.c_int, C.c_int, C.c_double, _vp, _vp]
     L.tvl1_glibc_rand.argtypes = [C.c_longlong, C.c_longlong, C.c_int, _vp]
     L.tvl1_selftest_arith.argtypes = [C.c_longlong, C.c_uint, C.c_int, C.c_int, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
@@ -374,31 +381,43 @@ class Solver:
         g = int(add_grid)
         check(lib().tvl1_finish_flow_u8(self.handle, d_f1, pitch1, w, h, d_u, d_v, pitch_out, (g > 0) - (g < 0), stream))
 
-    def find_alignment(self, moving, fixed, **kw):
+    def find_alignment(self, moving, fixed, pitch_moving=None, pitch_fixed=None, pad_value=255, **kw):
         """find_alignment (src/features.cpp:46-167): host uint8 frames in, (affine 2x3 float32 mapping `moving`
-        coordinates to `fixed` coordinates, n_matches, n_good) out.  kw: fields of tvl1_feature_params."""
+        coordinates to `fixed` coordinates, n_matches, n_good) out.  kw: fields of tvl1_feature_params.
+        pitch_*: the frames go up as rows of that many bytes, the padding filled with pad_value."""
         moving = np.ascontiguousarray(moving, np.uint8)
         fixed = np.ascontiguousarray(fixed, np.uint8)
-        p = FeatureParams()
-        lib().tvl1_default_feature_params(C.byref(p))
-        for k, v in kw.items():
-            k = {"scaleFactor": "scale_factor", "edgeThreshold": "edge_threshold", "firstLevel": "first_level",
-                 "patchSize": "patch_size", "fastThreshold": "fast_threshold"}.get(k, k)
-            if not hasattr(p, k):
-                raise KeyError(k)
-            setattr(p, k, v)
-        bm = DevBuf(moving.nbytes, self.device).upload(moving)
-        bf = DevBuf(fixed.nbytes, self.device).upload(fixed)
+        p = feature_params(**kw)
+        bm, pm = upload_u8(moving, pitch_moving, pad_value, self.device)
+        bf, pf = upload_u8(fixed, pitch_fixed, pad_value, self.device)
         aff = np.zeros(6, np.float32)
         nm, ng = C.c_int(0), C.c_int(0)
         try:
-            check(lib().tvl1_find_alignment(self.handle, bm.ptr, moving.shape[1], moving.shape[1], moving.shape[0],
-                                            bf.ptr, fixed.shape[1], fixed.shape[1], fixed.shape[0], C.byref(p),
+            check(lib().tvl1_find_alignment(self.handle, bm.ptr, pm, moving.shape[1], moving.shape[0],
+                                            bf.ptr, pf, fixed.shape[1], fixed.shape[0], C.byref(p),
                                             aff.ctypes.data, C.byref(nm), C.byref(ng), None))
         finally:
             bm.free()
             bf.free()
         return aff.reshape(2, 3), nm.value, ng.value
+
+    def features_extract(self, img, pitch=None, pad_value=255, **kw):
+        """One frame's keypoints (KEYPT_DTYPE) and descriptors ((n, 8) uint32) as tvl1_find_alignment computes
+        them (tvl1_features_extract).  kw: fields of tvl1_feature_params."""
+        img = np.ascontiguousarray(img, np.uint8)
+        p = feature_params(**kw)
+        b, pb = upload_u8(img, pitch, pad_value, self.device)
+        kp = DevBuf(p.nfeatures * KEYPT_DTYPE.itemsize, self.device)
+        desc = DevBuf(p.nfeatures * 32, self.device)
+        n = C.c_int(0)
+        try:
+            check(lib().tvl1_features_extract(self.handle, b.ptr, pb, img.shape[1], img.shape[0], C.byref(p),
+                                              kp.ptr, desc.ptr, p.nfeatures, C.byref(n), None))
+            n = n.value
+            return kp.download(n, KEYPT_DTYPE), desc.download((n, 8), np.uint32)
+        finally:
+            for x in (b, kp, desc):
+                x.free()
 
     def sample_matches_device(self, d_f0, pitch0, d_f1, pitch1, d_u, d_v, pitch_flow, w, h,
                               roi0=(0, 0), roi1=(0, 0), scale=0.5, npoints=25, seed=-1,
@@ -564,27 +583,136 @@ def k_iterate_gamma(I1wx, I1wy, rho_c, u1, u2, u3, p11, p12, p21, p22, p31, p32,
     return tuple(p.get() for p in state) + (errs[:n],)
 
 
-def warp_affine(src, affine, dsize, device=0):
-    """cv::warpAffine(src, affine, dsize = (w, h), INTER_LINEAR, BORDER_CONSTANT 0) on the device; uint8 or float32"""
+def warp_affine(src, affine, dsize, device=0, spitch=None, dpitch=None):
+    """cv::warpAffine(src, affine, dsize = (w, h), INTER_LINEAR, BORDER_CONSTANT 0) on the device; uint8 or float32.
+    spitch / dpitch: row pitches in ELEMENTS of the device copies (default: the widths); padding holds a marker
+    value (255 resp. NaN) that must neither be read nor be overwritten."""
     src = np.ascontiguousarray(src)
     aff = np.ascontiguousarray(affine, np.float32).reshape(6)
     dw, dh = int(dsize[0]), int(dsize[1])
     sh, sw = src.shape
-    bs = DevBuf(src.nbytes, device).upload(src)
+    sp, dp = spitch or sw, dpitch or dw
+    mark = 255 if src.dtype == np.uint8 else np.nan
+    a = np.full((sh, sp), mark, src.dtype)
+    a[:, :sw] = src
+    bs = DevBuf(a.nbytes, device).upload(a)
+    bd = DevBuf(dh * dp * src.itemsize, device).upload(np.full((dh, dp), mark, src.dtype))
+    e = src.itemsize
     if src.dtype == np.uint8:
-        bd = DevBuf(dw * dh, device)
-        check(lib().tvl1_warp_affine_u8(bs.ptr, sw, sw, sh, aff.ctypes.data, bd.ptr, dw, dw, dh, None))
-        check(lib().tvl1_dev_sync(device))
-        out = bd.download((dh, dw), np.uint8)
+        check(lib().tvl1_warp_affine_u8(bs.ptr, sp, sw, sh, aff.ctypes.data, bd.ptr, dp, dw, dh, None))
     else:
         assert src.dtype == np.float32
-        bd = DevBuf(dw * dh * 4, device)
-        check(lib().tvl1_warp_affine_f32(bs.ptr, sw * 4, sw, sh, aff.ctypes.data, bd.ptr, dw * 4, dw, dh, None))
-        check(lib().tvl1_dev_sync(device))
-        out = bd.download((dh, dw), np.float32)
+        check(lib().tvl1_warp_affine_f32(bs.ptr, sp * e, sw, sh, aff.ctypes.data, bd.ptr, dp * e, dw, dh, None))
+    check(lib().tvl1_dev_sync(device))
+    out = bd.download((dh, dp), src.dtype)
     bs.free()
     bd.free()
+    pad = out[:, dw:]
+    assert (pad == 255).all() if src.dtype == np.uint8 else np.isnan(pad).all(), "warp_affine wrote into the row padding"
+    return np.ascontiguousarray(out[:, :dw])
+
+
+# ---- the feature kernels (tvl1_k_gauss7_u8 .. tvl1_features_extract)
+
+CAND_DTYPE = np.dtype([("harris", "<f4"), ("x", "<u2"), ("y", "<u2")])            # struct Cand
+KEYPT_DTYPE = np.dtype([("x", "<f4"), ("y", "<f4"), ("angle", "<f4"), ("level", "<i4")])   # struct KeyPt
+
+
+def feature_params(**kw):
+    """tvl1_default_feature_params with the given fields replaced (OpenCV's ORB names accepted)"""
+    p = FeatureParams()
+    lib().tvl1_default_feature_params(C.byref(p))
+    for k, v in kw.items():
+        k = {"scaleFactor": "scale_factor", "edgeThreshold": "edge_threshold", "firstLevel": "first_level",
+             "patchSize": "patch_size", "fastThreshold": "fast_threshold"}.get(k, k)
+        if not hasattr(p, k):
+            raise KeyError(k)
+        setattr(p, k, v)
+    return p
+
+
+def upload_u8(img, pitch=None, pad_value=255, device=0):
+    """(DevBuf, pitch): an 8-bit image on the device as rows of `pitch` bytes (default: its width), the
+    padding filled with pad_value"""
+    img = np.ascontiguousarray(img, np.uint8)
+    h, w = img.shape
+    pitch = int(pitch or w)
+    a = np.full((h, pitch), pad_value, np.uint8)
+    a[:, :w] = img
+    return DevBuf(a.nbytes, device).upload(a), pitch
+
+
+def k_gauss7_u8(img, spitch=None, dpitch=None, device=0):
+    """7x7 Gaussian (sigma 2) of an 8-bit image; the output's row padding must stay untouched"""
+    img = np.ascontiguousarray(img, np.uint8)
+    h, w = img.shape
+    s, sp = upload_u8(img, spitch, 255, device)
+    dp = int(dpitch or w)
+    d = DevBuf(h * dp, device).upload(np.full((h, dp), 77, np.uint8))
+    check(lib().tvl1_k_gauss7_u8(s.ptr, sp, w, h, d.ptr, dp, None))
+    check(lib().tvl1_dev_sync(device))
+    out = d.download((h, dp), np.uint8)
+    assert (out[:, w:] == 77).all(), "k_gauss7_u8 wrote into the row padding"
+    return np.ascontiguousarray(out[:, :w])
+
+
+def k_fast_corners(img, border, t, pitch=None, spitch=None, cap=None, device=0):
+    """k_fast_score + k_nms_harris: (score plane, candidates (CAND_DTYPE, device order), count, 2048-bin histogram)"""
+    img = np.ascontiguousarray(img, np.uint8)
+    h, w = img.shape
+    b, pb = upload_u8(img, pitch, 255, device)
+    sp = int(spitch or w)
+    cap = int(cap if cap is not None else h * w // 2 + 1)
+    score = DevBuf(h * sp * 4, device).zero()
+    cand = DevBuf(max(cap, 1) * CAND_DTYPE.itemsize, device)
+    cnt = DevBuf((1 + 2048) * 4, device).zero()
+    check(lib().tvl1_k_fast_corners(b.ptr, pb, w, h, border, t, score.ptr, sp, cand.ptr, cap, cnt.ptr, cnt.ptr + 4, None))
+    check(lib().tvl1_dev_sync(device))
+    counters = cnt.download(1 + 2048, np.int32)
+    n = int(counters[0])
+    out = (score.download((h, sp), np.float32)[:, :w].copy(), cand.download(min(n, cap), CAND_DTYPE), n, counters[1:])
+    for x in (b, score, cand, cnt):
+        x.free()
     return out
+
+
+def k_describe(img, blur, cand, scale=1.0, level=0, pitch=None, bpitch=None, device=0):
+    """k_describe of the candidates `cand` (CAND_DTYPE or (x, y) pairs): keypoints (KEYPT_DTYPE), (n, 8) uint32"""
+    img = np.ascontiguousarray(img, np.uint8)
+    h, w = img.shape
+    c = np.asarray(cand)
+    if c.dtype != CAND_DTYPE:
+        xy = np.asarray(c, np.int64).reshape(-1, 2)
+        c = np.zeros(len(xy), CAND_DTYPE)
+        c["x"], c["y"] = xy[:, 0], xy[:, 1]
+    n = len(c)
+    bi, pi = upload_u8(img, pitch, 255, device)
+    bb, pbb = upload_u8(blur, bpitch, 255, device)
+    bc = DevBuf(max(n, 1) * CAND_DTYPE.itemsize, device).upload(c)
+    kp = DevBuf(max(n, 1) * KEYPT_DTYPE.itemsize, device)
+    desc = DevBuf(max(n, 1) * 32, device)
+    check(lib().tvl1_k_describe(bi.ptr, pi, bb.ptr, pbb, bc.ptr, n, scale, level, kp.ptr, desc.ptr, None))
+    check(lib().tvl1_dev_sync(device))
+    out = kp.download(n, KEYPT_DTYPE), desc.download((n, 8), np.uint32)
+    for x in (bi, bb, bc, kp, desc):
+        x.free()
+    return out
+
+
+def k_knn2(q, t, device=0):
+    """Hamming 2-NN of (nq, 8) uint32 query descriptors among (nt, 8) train descriptors: idx1, d1, d2"""
+    q = np.ascontiguousarray(q, np.uint32).reshape(-1, 8)
+    t = np.ascontiguousarray(t, np.uint32).reshape(-1, 8)
+    nq, nt = len(q), len(t)
+    bq = DevBuf(max(q.nbytes, 4), device).upload(q)
+    bt = DevBuf(max(t.nbytes, 4), device).upload(t)
+    outs = [DevBuf(max(nq, 1) * 4, device) for _ in range(3)]
+    check(lib().tvl1_k_knn2(bq.ptr, nq, bt.ptr, nt, *[o.ptr for o in outs], None))
+    check(lib().tvl1_dev_sync(device))
+    res = tuple(o.download(nq, np.int32) for o in outs)
+    for x in [bq, bt] + outs:
+        x.free()
+    return res
 
 
 def k_median3(src, device=0):

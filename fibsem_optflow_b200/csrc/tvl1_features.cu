@@ -51,7 +51,8 @@ __constant__ int c_disc_umax[16];            // half-width of row v of the radiu
 __global__ void __launch_bounds__(256) k_gauss7_u8(const uint8_t* __restrict__ src, size_t sp, int w, int h,
                                                    uint8_t* __restrict__ dst, size_t dp)
 {
-    const float k[4] = {0.20236f, 0.17994f, 0.12395f, 0.06493f};   // normalised getGaussianKernel(7, 2): centre, +-1, +-2, +-3
+    // cv::getGaussianKernel(7, 2) rounded to fp32: centre, +-1, +-2, +-3 (they sum to 1)
+    const float k[4] = {0.216105938f, 0.190712824f, 0.131074876f, 0.0701593235f};
     const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
     if (x >= w || y >= h) return;
     auto refl = [](int p, int n) { p = p < 0 ? -p : p; return p >= n ? 2 * n - 2 - p : p; };
@@ -111,8 +112,9 @@ __global__ void __launch_bounds__(256) k_fast_score(const uint8_t* __restrict__ 
 struct Cand { float harris; unsigned short x, y; };
 
 // 3x3 non-maximum suppression of the FAST score, Harris response (7x7 block, Sobel 3x3, k = 0.04) of the
-// survivors, append to the candidate list (atomic counter; entries past the capacity are dropped) and to a
-// 2048-bin histogram of the response's float bits (monotone for positive floats) for the top-N cut
+// survivors, append to the candidate list (atomic counter; entries past the capacity are dropped but still
+// counted, so that the caller can grow the list and run again) and to a 2048-bin histogram of the response's
+// float bits (monotone for positive floats) for the top-N cut
 __global__ void __launch_bounds__(256) k_nms_harris(const float* __restrict__ score, int spitch, const uint8_t* __restrict__ img,
                                                     size_t pitch, int w, int h, int border, Cand* __restrict__ cand,
                                                     int cap, int* __restrict__ count, int* __restrict__ hist)
@@ -165,9 +167,9 @@ __global__ void __launch_bounds__(256) k_select(const Cand* __restrict__ cand, i
 struct KeyPt { float x, y, angle; int level; };   // x, y in level-0 pixels
 
 // one warp per keypoint: intensity-centroid angle on the level image, then the 256 steered tests on the
-// smoothed level; lane l produces byte l of the descriptor
-__global__ void __launch_bounds__(128) k_describe(const uint8_t* __restrict__ img, const uint8_t* __restrict__ blur, size_t pitch,
-                                                  const Cand* __restrict__ kp, int n, float scale, int level,
+// smoothed level; lane l produces byte l of the descriptor.  `pitch` is the level's, `bpitch` the smoothed copy's.
+__global__ void __launch_bounds__(128) k_describe(const uint8_t* __restrict__ img, size_t pitch, const uint8_t* __restrict__ blur,
+                                                  size_t bpitch, const Cand* __restrict__ kp, int n, float scale, int level,
                                                   KeyPt* __restrict__ out_kp, uint32_t* __restrict__ out_desc, int out_base)
 {
     const int wi = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
@@ -188,14 +190,14 @@ __global__ void __launch_bounds__(128) k_describe(const uint8_t* __restrict__ im
     const float ang = atan2f((float)m01, (float)m10);
     float sn, cs;
     sincosf(ang, &sn, &cs);
-    const uint8_t* b = blur + (size_t)cy * pitch + cx;
+    const uint8_t* b = blur + (size_t)cy * bpitch + cx;
     unsigned byte = 0;
 #pragma unroll
     for (int k = 0; k < 8; k++) {
         const signed char* t = c_brief + (lane * 8 + k) * 4;
         const int ax = __float2int_rn(t[0] * cs - t[1] * sn), ay = __float2int_rn(t[0] * sn + t[1] * cs);
         const int bx = __float2int_rn(t[2] * cs - t[3] * sn), by = __float2int_rn(t[2] * sn + t[3] * cs);
-        const int va = b[(ptrdiff_t)ay * (ptrdiff_t)pitch + ax], vb = b[(ptrdiff_t)by * (ptrdiff_t)pitch + bx];
+        const int va = b[(ptrdiff_t)ay * (ptrdiff_t)bpitch + ax], vb = b[(ptrdiff_t)by * (ptrdiff_t)bpitch + bx];
         byte |= (va < vb ? 1u : 0u) << k;
     }
     // four lanes -> one 32-bit word
@@ -452,7 +454,6 @@ struct FeatScratch {
     uint32_t* desc[2] = {nullptr, nullptr};
     int kp_cap = 0;
     int *idx1 = nullptr, *d1 = nullptr, *d2 = nullptr;
-    bool tables = false;
 };
 
 void features_release(void* p)
@@ -465,10 +466,11 @@ void features_release(void* p)
     delete S;
 }
 
-static int upload_tables(FeatScratch& S)
+// the current device's BRIEF pattern and disc table
+static int upload_tables(int device)
 {
     static bool done[64] = {false};          // __constant__ tables live per device, not per handle
-    if (S.tables || done[S.device & 63]) return TVL1_OK;
+    if (done[device & 63]) return TVL1_OK;
     // 256 test pairs: isotropic Gaussian (sigma = patch / 5) clipped to +-13, fixed seed
     signed char pat[256 * 4];
     uint64_t r = 0x2545F4914F6CDD1Dull;
@@ -487,8 +489,7 @@ static int upload_tables(FeatScratch& S)
     int umax[16];
     for (int v = 0; v <= 15; v++) umax[v] = (int)std::floor(std::sqrt(15.0 * 15.0 - (double)v * v) + 1e-9);
     CKF(cudaMemcpyToSymbol(c_disc_umax, umax, sizeof(umax)));
-    S.tables = true;
-    done[S.device & 63] = true;
+    done[device & 63] = true;
     return TVL1_OK;
 }
 
@@ -515,11 +516,11 @@ static int extract(FeatScratch& S, const uint8_t* d_img, size_t pitch, int w, in
         CKF(cudaMalloc(&S.lvl, px)); CKF(cudaMalloc(&S.blur, px)); CKF(cudaMalloc(&S.score, px * sizeof(float)));
         S.img_cap = px;
     }
-    const int cand_cap = 1 << 22, sel_cap = 4 * P.nfeatures + 4096, kp_cap = P.nfeatures + 64;
+    // the candidate list starts at 4M entries and grows when a level has more NMS survivors; the selection
+    // is sized per level from the histogram
+    const int cand_cap = 1 << 22, kp_cap = P.nfeatures + 64;
     if ((rc = grow(&S.cand, (size_t)S.cand_cap, (size_t)cand_cap))) return rc;
     S.cand_cap = std::max(S.cand_cap, cand_cap);
-    if ((rc = grow(&S.sel, (size_t)S.sel_cap, (size_t)sel_cap))) return rc;
-    S.sel_cap = std::max(S.sel_cap, sel_cap);
     if (!S.counters) CKF(cudaMalloc(&S.counters, sizeof(int) * (2 + 2048)));
     if (S.kp_cap < kp_cap) {
         for (int k = 0; k < 2; k++) { cudaFree(S.kp[k]); cudaFree(S.desc[k]); S.kp[k] = nullptr; S.desc[k] = nullptr; }
@@ -561,21 +562,34 @@ static int extract(FeatScratch& S, const uint8_t* d_img, size_t pitch, int w, in
         CKF(cudaGetLastError());
         CKF(cudaMemcpyAsync(h_cnt.data(), S.counters, sizeof(int) * (2 + 2048), cudaMemcpyDeviceToHost, st));
         CKF(cudaStreamSynchronize(st));
-        const int ncand = std::min(h_cnt[0], S.cand_cap), want = std::min(quota[l], P.nfeatures - total);
+        if (h_cnt[0] > S.cand_cap) {
+            // more survivors than the list holds (the atomics decided which were dropped): grow it, list them again
+            if ((rc = grow(&S.cand, (size_t)S.cand_cap, (size_t)h_cnt[0]))) return rc;
+            S.cand_cap = h_cnt[0];
+            CKF(cudaMemsetAsync(S.counters, 0, sizeof(int) * (2 + 2048), st));
+            k_nms_harris<<<g, b, 0, st>>>(S.score, lw, img, lp, lw, lh, border, S.cand, S.cand_cap, S.counters, S.counters + 2);
+            CKF(cudaGetLastError());
+            CKF(cudaMemcpyAsync(h_cnt.data(), S.counters, sizeof(int) * (2 + 2048), cudaMemcpyDeviceToHost, st));
+            CKF(cudaStreamSynchronize(st));
+        }
+        const int ncand = h_cnt[0], want = std::min(quota[l], P.nfeatures - total);
         if (ncand == 0 || want == 0) continue;
-        // highest histogram bin such that the bins from it upwards hold at least `want` candidates
+        // highest histogram bin such that the bins from it upwards hold at least `want` candidates; those bins
+        // hold exactly `nsel`, and the selection has room for all of them
         unsigned cut = 0;
-        for (int bin = 2047, acc = 0; bin >= 0; bin--) { acc += h_cnt[2 + bin]; if (acc >= want) { cut = (unsigned)bin; break; } }
+        int nsel = ncand;
+        for (int bin = 2047, acc = 0; bin >= 0; bin--) {
+            acc += h_cnt[2 + bin];
+            if (acc >= want) { cut = (unsigned)bin; nsel = acc; break; }
+        }
+        if ((rc = grow(&S.sel, (size_t)S.sel_cap, (size_t)nsel))) return rc;
+        S.sel_cap = std::max(S.sel_cap, nsel);
         k_select<<<cdivf(ncand, 256), 256, 0, st>>>(S.cand, ncand, cut, S.sel, S.sel_cap, S.counters + 1);
         CKF(cudaGetLastError());
-        int nsel = 0;
-        CKF(cudaMemcpyAsync(&nsel, S.counters + 1, sizeof(int), cudaMemcpyDeviceToHost, st));
-        CKF(cudaStreamSynchronize(st));
-        nsel = std::min(nsel, S.sel_cap);
         h_sel.resize((size_t)nsel);
         CKF(cudaMemcpyAsync(h_sel.data(), S.sel, sizeof(Cand) * (size_t)nsel, cudaMemcpyDeviceToHost, st));
         CKF(cudaStreamSynchronize(st));
-        // strongest first; position breaks ties so that the order does not depend on the atomics
+        // strongest first; position breaks ties, so that neither the set kept nor its order depends on the atomics
         std::sort(h_sel.begin(), h_sel.end(), [](const Cand& a, const Cand& c) {
             if (a.harris != c.harris) return a.harris > c.harris;
             if (a.y != c.y) return a.y < c.y;
@@ -583,13 +597,36 @@ static int extract(FeatScratch& S, const uint8_t* d_img, size_t pitch, int w, in
         });
         const int keep = std::min(nsel, want);
         CKF(cudaMemcpyAsync(S.sel, h_sel.data(), sizeof(Cand) * (size_t)keep, cudaMemcpyHostToDevice, st));
-        k_describe<<<cdivf(keep * 32, 128), 128, 0, st>>>(img, S.blur, lp, S.sel, keep, (float)sc, l, S.kp[which], S.desc[which], total);
+        k_describe<<<cdivf(keep * 32, 128), 128, 0, st>>>(img, lp, S.blur, (size_t)lw, S.sel, keep, (float)sc, l, S.kp[which],
+                                                          S.desc[which], total);
         CKF(cudaGetLastError());
         CKF(cudaStreamSynchronize(st));   // h_sel is re-used by the next level
         total += keep;
     }
     *n_out = total;
     return TVL1_OK;
+}
+
+static int check_feature_params(const tvl1_feature_params& P)
+{
+    if (P.nfeatures < 16 || P.nfeatures > (1 << 20) || P.nlevels < 1 || P.nlevels > 16 || !(P.scale_factor > 1.f) ||
+        P.fast_threshold < 1 || P.fast_threshold > 254 || !(P.ratio > 0.f) || !(P.ransac > 0.0))
+        return fail(TVL1_ERR_INVALID, "feature parameters out of range");
+    if (P.first_level != 0) return fail(TVL1_ERR_UNSUPPORTED, "firstLevel != 0 is not supported");
+    return TVL1_OK;
+}
+
+// the handle's feature scratch on its device, with the device's tables uploaded
+static int feature_scratch(tvl1_handle* H, FeatScratch** out)
+{
+    const int dev = handle_device(H);
+    CKF(cudaSetDevice(dev));
+    void** slot = handle_feature_slot(H);
+    if (!*slot) *slot = new FeatScratch();
+    FeatScratch* S = (FeatScratch*)*slot;
+    S->device = dev;
+    *out = S;
+    return upload_tables(dev);
 }
 
 }  // namespace tvl1
@@ -615,19 +652,12 @@ int tvl1_find_alignment(tvl1_handle* H, const uint8_t* d_moving, size_t pitch_m,
     if (wm <= 0 || hm <= 0 || wf <= 0 || hf <= 0 || pitch_m < (size_t)wm || pitch_f < (size_t)wf) return fail(TVL1_ERR_INVALID, "bad geometry");
     if (wm > 65535 || hm > 65535 || wf > 65535 || hf > 65535) return fail(TVL1_ERR_INVALID, "frame side > 65535");
     tvl1_feature_params P = *prm;
-    if (P.nfeatures < 16 || P.nfeatures > (1 << 20) || P.nlevels < 1 || P.nlevels > 16 || !(P.scale_factor > 1.f) ||
-        P.fast_threshold < 1 || P.fast_threshold > 254 || !(P.ratio > 0.f) || !(P.ransac > 0.0))
-        return fail(TVL1_ERR_INVALID, "feature parameters out of range");
-    if (P.first_level != 0) return fail(TVL1_ERR_UNSUPPORTED, "firstLevel != 0 is not supported");
-    const int dev = handle_device(H);
-    CKF(cudaSetDevice(dev));
-    void** slot = handle_feature_slot(H);
-    if (!*slot) *slot = new FeatScratch();
-    FeatScratch& S = *(FeatScratch*)*slot;
-    S.device = dev;
-    cudaStream_t st = (cudaStream_t)stream;
-    int rc = upload_tables(S);
+    int rc = check_feature_params(P);
     if (rc) return rc;
+    FeatScratch* Sp = nullptr;
+    if ((rc = feature_scratch(H, &Sp))) return rc;
+    FeatScratch& S = *Sp;
+    cudaStream_t st = (cudaStream_t)stream;
     // identity unless a trustworthy transform is found (src/features.cpp:141-164)
     const float ident[6] = {1.f, 0.f, 0.f, 0.f, 1.f, 0.f};
     memcpy(affine, ident, sizeof(ident));
@@ -720,6 +750,76 @@ int tvl1_warp_affine_f32(const float* d_src, size_t spitch, int sw, int sh, cons
     dim3 b(32, 8), g(cdivf(dw, 32), cdivf(dh, 8));
     k_warp_affine_f32<<<g, b, 0, (cudaStream_t)stream>>>(d_src, spitch / 4, sw, sh, d_dst, dpitch / 4, dw, dh, A);
     CKF(cudaGetLastError());
+    return TVL1_OK;
+}
+
+// ---- stage-level entry points of the feature kernels (launches only; extract() is the production sequence)
+
+int tvl1_k_gauss7_u8(const uint8_t* d_src, size_t spitch, int w, int h, uint8_t* d_dst, size_t dpitch, void* stream)
+{
+    if (!d_src || !d_dst || w <= 0 || h <= 0 || spitch < (size_t)w || dpitch < (size_t)w) return fail(TVL1_ERR_INVALID, "bad argument");
+    dim3 b(32, 8), g(cdivf(w, 32), cdivf(h, 8));
+    k_gauss7_u8<<<g, b, 0, (cudaStream_t)stream>>>(d_src, spitch, w, h, d_dst, dpitch);
+    CKF(cudaGetLastError());
+    return TVL1_OK;
+}
+
+int tvl1_k_fast_corners(const uint8_t* d_img, size_t pitch, int w, int h, int border, int t, float* d_score, int spitch,
+                        void* d_cand, int cap, int* d_count, int* d_hist, void* stream)
+{
+    if (!d_img || !d_score || !d_cand || !d_count || !d_hist || w <= 0 || h <= 0 || w > 65535 || h > 65535 ||
+        pitch < (size_t)w || spitch < w || border < 4 || cap < 0)
+        return fail(TVL1_ERR_INVALID, "bad argument");
+    dim3 b(32, 8), g(cdivf(w, 32), cdivf(h, 8));
+    k_fast_score<<<g, b, 0, (cudaStream_t)stream>>>(d_img, pitch, w, h, border, t, d_score, spitch);
+    k_nms_harris<<<g, b, 0, (cudaStream_t)stream>>>(d_score, spitch, d_img, pitch, w, h, border, (Cand*)d_cand, cap, d_count, d_hist);
+    CKF(cudaGetLastError());
+    return TVL1_OK;
+}
+
+int tvl1_k_describe(const uint8_t* d_img, size_t pitch, const uint8_t* d_blur, size_t bpitch, const void* d_cand, int n,
+                    float scale, int level, void* d_kp, uint32_t* d_desc, void* stream)
+{
+    if (!d_img || !d_blur || !d_cand || !d_kp || !d_desc || n < 0) return fail(TVL1_ERR_INVALID, "bad argument");
+    int dev = 0;
+    CKF(cudaGetDevice(&dev));
+    if (int rc = upload_tables(dev)) return rc;
+    if (n == 0) return TVL1_OK;
+    k_describe<<<cdivf(n * 32, 128), 128, 0, (cudaStream_t)stream>>>(d_img, pitch, d_blur, bpitch, (const Cand*)d_cand, n, scale,
+                                                                     level, (KeyPt*)d_kp, d_desc, 0);
+    CKF(cudaGetLastError());
+    return TVL1_OK;
+}
+
+int tvl1_k_knn2(const uint32_t* d_q, int nq, const uint32_t* d_t, int nt, int* d_idx1, int* d_d1, int* d_d2, void* stream)
+{
+    if (!d_q || !d_t || !d_idx1 || !d_d1 || !d_d2 || nq < 0 || nt < 1) return fail(TVL1_ERR_INVALID, "bad argument");
+    if (nq == 0) return TVL1_OK;
+    k_knn2<<<cdivf(nq, 128), 128, 0, (cudaStream_t)stream>>>(d_q, nq, d_t, nt, d_idx1, d_d1, d_d2);
+    CKF(cudaGetLastError());
+    return TVL1_OK;
+}
+
+int tvl1_features_extract(tvl1_handle* H, const uint8_t* d_img, size_t pitch, int w, int h, const tvl1_feature_params* prm,
+                          void* d_kp, uint32_t* d_desc, int cap, int* n_out, void* stream)
+{
+    if (!H || !d_img || !prm || !d_kp || !d_desc || !n_out) return fail(TVL1_ERR_INVALID, "null argument");
+    if (w <= 0 || h <= 0 || pitch < (size_t)w || w > 65535 || h > 65535) return fail(TVL1_ERR_INVALID, "bad geometry");
+    const tvl1_feature_params P = *prm;
+    int rc = check_feature_params(P);
+    if (rc) return rc;
+    if (cap < P.nfeatures) return fail(TVL1_ERR_INVALID, "cap %d < nfeatures %d", cap, P.nfeatures);
+    FeatScratch* S = nullptr;
+    if ((rc = feature_scratch(H, &S))) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    int n = 0;
+    if ((rc = extract(*S, d_img, pitch, w, h, P, 0, st, &n))) return rc;
+    if (n > 0) {
+        CKF(cudaMemcpyAsync(d_kp, S->kp[0], sizeof(KeyPt) * (size_t)n, cudaMemcpyDeviceToDevice, st));
+        CKF(cudaMemcpyAsync(d_desc, S->desc[0], 32 * (size_t)n, cudaMemcpyDeviceToDevice, st));
+    }
+    CKF(cudaStreamSynchronize(st));
+    *n_out = n;
     return TVL1_OK;
 }
 

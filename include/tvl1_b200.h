@@ -303,6 +303,28 @@ int tvl1_k_outer(const float* d_I1wx, const float* d_I1wy, const float* d_grad,
 int tvl1_k_median5(const float* d_src, int w, int h, int pitch, float* d_dst, void* stream);
 /* medianBlur(src, 3): the other fp32 aperture (medianFiltering = 3) */
 int tvl1_k_median3(const float* d_src, int w, int h, int pitch, float* d_dst, void* stream);
+/* The feature pre-alignment's kernels (8-bit images, pitches in BYTES; the score plane's in elements).
+ * Candidates are {float harris; uint16_t x, y} (8 bytes), keypoints {float x, y, angle; int level}
+ * (16 bytes, x and y in level-0 pixels), descriptors 8 uint32 words (byte l = tests 8l .. 8l+7, bit k = test 8l+k).
+ * tvl1_k_gauss7_u8: 7x7 Gaussian (sigma 2), reflect-101 border, rounded to 8 bits. */
+int tvl1_k_gauss7_u8(const uint8_t* d_src, size_t spitch, int w, int h, uint8_t* d_dst, size_t dpitch, void* stream);
+/* FAST-9 score plane (0 within `border` of the frame), then 3x3 non-maximum suppression and the Harris response
+ * of the survivors: up to `cap` candidates in d_cand, in any order.  *d_count and the 2048-bin histogram of the
+ * responses' float bits >> 20 are ADDED to (the caller zeroes them) and count every survivor, listed or not. */
+int tvl1_k_fast_corners(const uint8_t* d_img, size_t pitch, int w, int h, int border, int t, float* d_score, int spitch,
+                        void* d_cand, int cap, int* d_count, int* d_hist, void* stream);
+/* intensity-centroid angle on d_img and the 256 steered tests on d_blur (its own pitch) for n candidates;
+ * keypoint x, y = candidate position * scale */
+int tvl1_k_describe(const uint8_t* d_img, size_t pitch, const uint8_t* d_blur, size_t bpitch, const void* d_cand, int n,
+                    float scale, int level, void* d_kp, uint32_t* d_desc, void* stream);
+/* Hamming 2-NN of nq query descriptors among nt >= 1 train descriptors: nearest index (first on ties), its
+ * distance and the second smallest distance (1 << 30 when nt == 1) */
+int tvl1_k_knn2(const uint32_t* d_q, int nq, const uint32_t* d_t, int nt, int* d_idx1, int* d_d1, int* d_d2, void* stream);
+/* one frame through the keypoint + descriptor stage of tvl1_find_alignment: *n_out <= nfeatures keypoints and
+ * descriptors, level by level, each level's strongest first; cap (entries of d_kp / d_desc) >= nfeatures */
+int tvl1_features_extract(tvl1_handle* h, const uint8_t* d_img, size_t pitch, int width, int height,
+                          const tvl1_feature_params* prm, void* d_kp, uint32_t* d_desc, int cap, int* n_out,
+                          void* stream);
 /* CUDA-event time of the kernel launches of the calling thread's most recent tvl1_k_warp /
  * tvl1_k_iterate / tvl1_k_median5 call (waits for them). */
 int tvl1_k_last_ms(float* ms);

@@ -67,10 +67,15 @@ def test_warp_affine_matches_cv2(gpu, aff):
     want = cv2.warpAffine(img, A.astype(np.float64), (390, 280), flags=cv2.INTER_LINEAR, borderMode=cv2.BORDER_CONSTANT, borderValue=0)
     got = gpu.warp_affine(img, A, (390, 280))
     assert np.array_equal(got, want), int(np.abs(got.astype(int) - want).max())
+    # pitched source and destination (GpuMat rows are padded): the same pixels, the padding neither read nor written
+    for sp, dp in [(512, 390), (407, 391), (408, 512)]:
+        assert np.array_equal(gpu.warp_affine(img, A, (390, 280), spitch=sp, dpitch=dp), want), (sp, dp)
     plane = (rng.standard_normal((301, 407)) * 100).astype(np.float32)
     want = cv2.warpAffine(plane, A.astype(np.float64), (390, 280), flags=cv2.INTER_LINEAR, borderMode=cv2.BORDER_CONSTANT, borderValue=0)
     got = gpu.warp_affine(plane, A, (390, 280))
     np.testing.assert_allclose(got, want, rtol=0, atol=2e-4)
+    for sp, dp in [(416, 390), (407, 393)]:
+        assert np.array_equal(gpu.warp_affine(plane, A, (390, 280), spitch=sp, dpitch=dp), got), (sp, dp)
 
 
 def _composition(orc, f0, f1, aff, output_type, tv):
