@@ -13,6 +13,8 @@ SO_PATH = os.environ.get("TVL1_SO") or os.path.join(_HERE, "csrc", "libtvl1_b200
 
 MAX_LEVELS = 32
 MAX_WARPS = 64
+SEMANTICS_CPU = 0    # TVL1_SEMANTICS_CPU: cv::DualTVL1OpticalFlow (default)
+SEMANTICS_CUDA = 1   # TVL1_SEMANTICS_CUDA: cv::cuda::OpticalFlowDual_TVL1's algorithm
 
 
 class Tvl1Error(RuntimeError):
@@ -26,7 +28,7 @@ class Params(C.Structure):
         ("nscales", C.c_int), ("warps", C.c_int), ("iterations", C.c_int),
         ("inner_iterations", C.c_int), ("outer_iterations", C.c_int),
         ("median_filtering", C.c_int), ("use_initial_flow", C.c_int),
-        ("reserved", C.c_int * 3),
+        ("semantics", C.c_int), ("reserved", C.c_int * 2),
     ]
 
 
@@ -83,7 +85,7 @@ EXPORTS = [
     "tvl1_prescaled_size", "tvl1_prescale_u8", "tvl1_prescale_u8_host",
     "tvl1_mask_flow_u8", "tvl1_finish_flow_u8", "tvl1_sample_matches", "tvl1_sample_matches_skip", "tvl1_sample_matches_ex",
     "tvl1_default_feature_params", "tvl1_find_alignment", "tvl1_warp_affine_u8", "tvl1_warp_affine_f32", "tvl1_stack_run", "tvl1_k_convert_u8", "tvl1_k_resize",
-    "tvl1_k_centered_gradient", "tvl1_k_warp", "tvl1_k_iterate", "tvl1_k_iterate_fused2", "tvl1_k_outer", "tvl1_k_iterate_gamma", "tvl1_k_median5", "tvl1_k_median3", "tvl1_k_last_ms",
+    "tvl1_k_centered_gradient", "tvl1_k_warp", "tvl1_k_resize_cuda", "tvl1_k_warp_cuda", "tvl1_k_iterate", "tvl1_k_iterate_fused2", "tvl1_k_outer", "tvl1_k_iterate_gamma", "tvl1_k_median5", "tvl1_k_median3", "tvl1_k_last_ms",
     "tvl1_k_gauss7_u8", "tvl1_k_fast_corners", "tvl1_k_describe", "tvl1_k_knn2", "tvl1_features_extract",
     "tvl1_pyramid_sizes", "tvl1_glibc_rand", "tvl1_selftest_arith", "tvl1_dev_count", "tvl1_dev_alloc", "tvl1_dev_free",
     "tvl1_dev_memset", "tvl1_dev_h2d", "tvl1_dev_d2h", "tvl1_dev_sync", "tvl1_set_device", "tvl1_stream_create",
@@ -149,6 +151,8 @@ def lib():
                                 C.c_double, C.c_float, _vp]
     L.tvl1_k_centered_gradient.argtypes = [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp]
     L.tvl1_k_warp.argtypes = [_vp] * 4 + [C.c_int, C.c_int, C.c_int] + [_vp] * 6
+    L.tvl1_k_resize_cuda.argtypes = L.tvl1_k_resize.argtypes
+    L.tvl1_k_warp_cuda.argtypes = L.tvl1_k_warp.argtypes
     L.tvl1_k_iterate.argtypes = [_vp] * 10 + [C.c_int, C.c_int, C.c_int, C.c_float, C.c_float,
                                               C.c_float, C.c_int, _vp, _vp]
     L.tvl1_k_iterate_fused2.argtypes = L.tvl1_k_iterate.argtypes
@@ -207,9 +211,13 @@ def require_device():
 
 
 def default_params(**kw):
+    """tvl1_default_params with the given fields replaced (the reference's key names accepted).
+    semantics: SEMANTICS_CPU / SEMANTICS_CUDA, or "cpu" / "cuda"."""
     p = Params()
     lib().tvl1_default_params(C.byref(p))
     for k, v in kw.items():
+        if k == "semantics" and isinstance(v, str):
+            v = semantics_code(v)
         k = {"lambda": "lambda_", "scaleStep": "scale_step", "useInitialFlow": "use_initial_flow",
              "innerIterations": "inner_iterations", "outerIterations": "outer_iterations",
              "medianFiltering": "median_filtering"}.get(k, k)
@@ -217,6 +225,14 @@ def default_params(**kw):
             raise KeyError(k)
         setattr(p, k, v)
     return p
+
+
+def semantics_code(name):
+    """"cpu" -> SEMANTICS_CPU, "cuda" -> SEMANTICS_CUDA; anything else raises ValueError"""
+    codes = {"cpu": SEMANTICS_CPU, "cuda": SEMANTICS_CUDA}
+    if name not in codes:
+        raise ValueError("semantics must be 'cpu' or 'cuda', not %r" % (name,))
+    return codes[name]
 
 
 def pyramid_sizes(w, h, nscales, scale_step):
@@ -556,6 +572,45 @@ def k_warp(I0, I1, u1, u2, device=0):
     check(lib().tvl1_k_warp(*[p.ptr for p in ins], w, h, ins[0].pitch, *[p.ptr for p in outs], None))
     check(lib().tvl1_dev_sync(device))
     return tuple(p.get() for p in outs)
+
+
+def k_resize_cuda(src, dw=None, dh=None, inv_scale=0.0, mul=1.0, device=0, spitch=None, dpitch=None):
+    """cuda::resize(INTER_LINEAR) of TVL1_SEMANTICS_CUDA (tvl1_k_resize_cuda).  spitch / dpitch: pitches in
+    elements of the device planes (default: the width rounded up to 32)."""
+    src = np.asarray(src, np.float32)
+    sh, sw = src.shape
+    if inv_scale > 0:
+        dw, dh = int(np.rint(sw * inv_scale)), int(np.rint(sh * inv_scale))
+    sp, dp = int(spitch or pitch_of(sw)), int(dpitch or pitch_of(dw))
+    a = np.zeros((sh, sp), np.float32)
+    a[:, :sw] = src
+    s = DevBuf(a.nbytes, device).upload(a)
+    d = DevBuf(dh * dp * 4, device).zero()
+    check(lib().tvl1_k_resize_cuda(s.ptr, sw, sh, sp, d.ptr, dw, dh, dp, inv_scale, mul, None))
+    check(lib().tvl1_dev_sync(device))
+    out = d.download((dh, dp), np.float32)[:, :dw].copy()
+    s.free()
+    d.free()
+    return out
+
+
+def k_warp_cuda(I0, I1, u1, u2, device=0, pitch=None):
+    """warpBackward of TVL1_SEMANTICS_CUDA (tvl1_k_warp_cuda): returns I1w, I1wx, I1wy, grad, rho_c.  pitch: of
+    all device planes, in elements (default: the width rounded up to 32)."""
+    h, w = np.asarray(I0).shape
+    p = int(pitch or pitch_of(w))
+    bufs = []
+    for a in (I0, I1, u1, u2):
+        x = np.zeros((h, p), np.float32)
+        x[:, :w] = a
+        bufs.append(DevBuf(x.nbytes, device).upload(x))
+    outs = [DevBuf(h * p * 4, device).zero() for _ in range(5)]
+    check(lib().tvl1_k_warp_cuda(*[b.ptr for b in bufs], w, h, p, *[o.ptr for o in outs], None))
+    check(lib().tvl1_dev_sync(device))
+    res = tuple(o.download((h, p), np.float32)[:, :w].copy() for o in outs)
+    for b in bufs + outs:
+        b.free()
+    return res
 
 
 def k_iterate(I1wx, I1wy, grad, rho_c, u1, u2, p11, p12, p21, p22, l_t, theta, taut, n=1, device=0,

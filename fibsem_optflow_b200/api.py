@@ -27,6 +27,9 @@ TV_DEFAULTS = {"tau": 0.25, "lambda": 0.05, "theta": 0.3, "nscales": 10, "warps"
                "useInitialFlow": False}
 # optional extra keys (SURVEY.md T3/T4): the CPU-class parameters the cv::cuda API lacks
 EXTRA_KEYS = ("innerIterations", "outerIterations", "medianFiltering")
+# "semantics": "cpu" (default) computes cv::DualTVL1OpticalFlow, "cuda" cv::cuda::OpticalFlowDual_TVL1's algorithm,
+# which has none of EXTRA_KEYS
+SEMANTICS = ("cpu", "cuda")
 
 
 def _get(im_args, args, key, default):
@@ -49,6 +52,16 @@ def generate_TV_args(im_args, args):
         v = _get(im_args, args, k, None)
         if v is not None:
             tv[k] = int(v)
+    sem = _get(im_args, args, "semantics", None)
+    if sem is None:   # the default, "cpu": the dict stays exactly generate_TV_args's
+        return tv
+    if sem not in SEMANTICS:
+        raise ValueError("\"semantics\" must be \"cpu\" or \"cuda\", not %r" % (sem,))
+    if sem == "cuda":
+        bad = [k for k in EXTRA_KEYS if k in tv]
+        if bad:
+            raise ValueError("%s has no meaning with \"semantics\": \"cuda\"" % ", ".join('"%s"' % k for k in bad))
+    tv["semantics"] = sem
     return tv
 
 
@@ -69,6 +82,13 @@ def params_from_TV_args(tv):
     p.inner_iterations = int(tv.get("innerIterations", 0))
     p.outer_iterations = int(tv.get("outerIterations", 0))
     p.median_filtering = int(tv.get("medianFiltering", 5))
+    sem = tv.get("semantics", "cpu")
+    p.semantics = N.semantics_code(sem)
+    if sem == "cuda":
+        bad = [k for k in EXTRA_KEYS if k in tv]
+        if bad:
+            raise ValueError("%s has no meaning with \"semantics\": \"cuda\"" % ", ".join('"%s"' % k for k in bad))
+        p.median_filtering = 1
     return p
 
 

@@ -208,6 +208,21 @@ int launch_resize(const float* src, int sw, int sh, int sp, float* dst, int dw, 
     return launch_resize2(src, nullptr, sw, sh, sp, dst, nullptr, dw, dh, dp, inv_scale, mul, apply_mul, st);
 }
 
+// cv::cuda semantics: cuda::resize(INTER_LINEAR) of one or two planes (srcB / dstB may be null).  inv_scale > 0:
+// resize(src, Size(), inv_scale, inv_scale); otherwise the explicit size dw x dh (factor dw / sw in fp64).
+int launch_resize_cuda2(const float* srcA, const float* srcB, int sw, int sh, int sp, float* dstA, float* dstB, int dw,
+                        int dh, int dp, double inv_scale, float mul, int apply_mul, cudaStream_t st)
+{
+    const double f_x = inv_scale > 0 ? inv_scale : (double)dw / sw;
+    const double f_y = inv_scale > 0 ? inv_scale : (double)dh / sh;
+    const float fx = (float)(1.0 / f_x), fy = (float)(1.0 / f_y);
+    dim3 b(32, 8);
+    dim3 g(cdiv(dw, 32), cdiv(dh, 8), srcB ? 2 : 1);
+    k_resize_cuda<<<g, b, 0, st>>>(srcA, srcB, sw, sh, sp, dstA, dstB, dw, dh, dp, fx, fy, mul, apply_mul);
+    CK(cudaGetLastError());
+    return TVL1_OK;
+}
+
 int launch_gradient(const float* src, int w, int h, int pitch, float* dx, float* dy, cudaStream_t st)
 {
     dim3 b(32, 8);
@@ -236,6 +251,25 @@ int launch_warp(const WarpArgs& a, cudaStream_t st)
     return TVL1_OK;
 }
 
+// cv::cuda semantics: warpBackward (persistent blocks over the 32 x 16 tiles)
+int launch_warp_cuda(const WarpArgs& a, cudaStream_t st)
+{
+    static int cached[64] = {};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    int& resident = cached[dev & 63];
+    if (!resident) {
+        int sms = 148, occ = 0;
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_warp_cuda, 256, 0) != cudaSuccess || occ < 1) occ = 2;
+        resident = sms * occ;
+    }
+    const long long ntiles = (long long)cdiv(a.w, TVL1_WC_TW) * cdiv(a.h, TVL1_WC_TH);
+    k_warp_cuda<<<(unsigned)(ntiles < resident ? ntiles : resident), dim3(32, 8), 0, st>>>(a);
+    CK(cudaGetLastError());
+    return TVL1_OK;
+}
+
 #ifndef TVL1_ITER_NW
 #define TVL1_ITER_NW 4
 #endif
@@ -246,6 +280,8 @@ static const int ITER_NW = TVL1_ITER_NW;
 enum { KI_SMALL = 0, KI_LARGE = 1, KI_FUSED = 2, KI_MULTI = 3, KI_OUTER = 4 };   // k_iterate<.,5>, k_iterate<.,4>, k_iterate2, k_iterate_multi
 static const long long ITER_LARGE_PX = 16000000;     // levels at least this large: 4 blocks per SM
 
+// CS: the instantiation with the cv::cuda stop schedule (TVL1_SEMANTICS_CUDA)
+template <bool CS>
 static int resident_blocks(int which)
 {
     static int cached[5][64] = {};
@@ -257,22 +293,24 @@ static int resident_blocks(int which)
     cudaError_t e;
     if (which == KI_FUSED) {
         // the shared-memory ring needs the opt-in limit raised first
-        cudaFuncSetAttribute(k_iterate2<ITER_NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, TVL1_RING_BYTES(ITER_NW));
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_iterate2<ITER_NW>, 32 * ITER_NW, TVL1_RING_BYTES(ITER_NW));
+        cudaFuncSetAttribute(k_iterate2<ITER_NW, CS>, cudaFuncAttributeMaxDynamicSharedMemorySize, TVL1_RING_BYTES(ITER_NW));
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_iterate2<ITER_NW, CS>, 32 * ITER_NW, TVL1_RING_BYTES(ITER_NW));
     } else if (which == KI_OUTER) {
-        cudaFuncSetAttribute(k_outer<ITER_NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, TVL1_RING_BYTES(ITER_NW));
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_outer<ITER_NW>, 32 * ITER_NW, TVL1_RING_BYTES(ITER_NW));
+        cudaFuncSetAttribute(k_outer<ITER_NW, CS>, cudaFuncAttributeMaxDynamicSharedMemorySize, TVL1_RING_BYTES(ITER_NW));
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_outer<ITER_NW, CS>, 32 * ITER_NW, TVL1_RING_BYTES(ITER_NW));
     } else if (which == KI_MULTI) {
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_iterate_multi<ITER_NW, 4>, 32 * ITER_NW, 0);
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_iterate_multi<ITER_NW, 4, CS>, 32 * ITER_NW, 0);
     } else if (which == KI_LARGE) {
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_iterate<ITER_NW, 4>, 32 * ITER_NW, 0);
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_iterate<ITER_NW, 4, CS>, 32 * ITER_NW, 0);
     } else {
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_iterate<ITER_NW, 5>, 32 * ITER_NW, 0);
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_iterate<ITER_NW, 5, CS>, 32 * ITER_NW, 0);
     }
     if (e != cudaSuccess || occ < 1) occ = (which == KI_FUSED || which == KI_OUTER) ? 3 : 4;
     c = sms * occ;
     return c;
 }
+
+static int resident_blocks(int which, bool cs) { return cs ? resident_blocks<true>(which) : resident_blocks<false>(which); }
 
 // upper bound of the grid of any iteration kernel (blocks resident on the device), for the
 // per-block partial sums: SMs x the 32-blocks-per-SM hardware limit, two slabs
@@ -335,24 +373,27 @@ static int tile_rows(int w, int h, int strip, int halo, int rmin, int resident_b
     return e.rows;
 }
 
-int launch_iterate(IterArgs& a, cudaStream_t st)
+int launch_iterate(IterArgs& a, cudaStream_t st, bool cs = false)
 {
     int grid = 1;
     const bool large = (long long)a.w * a.h >= ITER_LARGE_PX;
-    a.rows = tile_rows(a.w, a.h, TVL1_STRIP, 1, 4, resident_blocks(large ? KI_LARGE : KI_SMALL), &grid);
+    a.rows = tile_rows(a.w, a.h, TVL1_STRIP, 1, 4, resident_blocks(large ? KI_LARGE : KI_SMALL, cs), &grid);
     dim3 b(32, ITER_NW);
-    if (large) k_iterate<ITER_NW, 4><<<grid, b, 0, st>>>(a);
+    if (cs) {
+        if (large) k_iterate<ITER_NW, 4, true><<<grid, b, 0, st>>>(a);
+        else k_iterate<ITER_NW, 5, true><<<grid, b, 0, st>>>(a);
+    } else if (large) k_iterate<ITER_NW, 4><<<grid, b, 0, st>>>(a);
     else k_iterate<ITER_NW, 5><<<grid, b, 0, st>>>(a);
     CK(cudaGetLastError());
     return TVL1_OK;
 }
 
 // several iterations in one cooperative launch (small levels); the grid must be co-resident
-int launch_iterate_multi(IterArgs& a, cudaStream_t st)
+int launch_iterate_multi(IterArgs& a, cudaStream_t st, bool cs = false)
 {
     // these levels are bound by latency, not by throughput: the shortest tiles that still give every
     // tile its own warp (one round) make an iteration a chain of R + 1 dependent row steps only
-    const int resident = resident_blocks(KI_MULTI);
+    const int resident = resident_blocks(KI_MULTI, cs);
     const long long slots = (long long)resident * ITER_NW, ns = cdiv(a.w, TVL1_STRIP);
     int grid = 1, R = 0;
     for (int r = 1; r <= 8 && !R; ++r)
@@ -365,16 +406,17 @@ int launch_iterate_multi(IterArgs& a, cudaStream_t st)
     }
     dim3 b(32, ITER_NW), g(grid);
     void* args[] = {(void*)&a};
-    cudaError_t e = cudaLaunchCooperativeKernel((const void*)k_iterate_multi<ITER_NW, 4>, g, b, args, 0, st);
+    const void* fn = cs ? (const void*)k_iterate_multi<ITER_NW, 4, true> : (const void*)k_iterate_multi<ITER_NW, 4>;
+    cudaError_t e = cudaLaunchCooperativeKernel(fn, g, b, args, 0, st);
     if (e != cudaSuccess) return fail(TVL1_ERR_CUDA, "cooperative launch of k_iterate_multi failed: %s", cudaGetErrorString(e));
     return TVL1_OK;
 }
 
 // the inner loop of one outer iteration (fused + single passes) in one cooperative launch
-int launch_outer(IterArgs& a, cudaStream_t st)
+int launch_outer(IterArgs& a, cudaStream_t st, bool cs = false)
 {
     int grid = 1, g1 = 1;
-    const int resident = resident_blocks(KI_OUTER);
+    const int resident = resident_blocks(KI_OUTER, cs);
     const long long slots = (long long)resident * ITER_NW;
     const long long ns2 = cdiv(a.w, TVL1_STRIP2), ns1 = cdiv(a.w, TVL1_STRIP);
     int R2 = 0, R1 = 0;
@@ -392,17 +434,19 @@ int launch_outer(IterArgs& a, cudaStream_t st)
     a.rows1 = R1 ? R1 : tile_rows(a.w, a.h, TVL1_STRIP, 1, 4, resident, &g1);   // single passes stride over the same grid
     dim3 b(32, ITER_NW), g(grid);
     void* args[] = {(void*)&a};
-    cudaError_t e = cudaLaunchCooperativeKernel((const void*)k_outer<ITER_NW>, g, b, args, TVL1_RING_BYTES(ITER_NW), st);
+    const void* fn = cs ? (const void*)k_outer<ITER_NW, true> : (const void*)k_outer<ITER_NW>;
+    cudaError_t e = cudaLaunchCooperativeKernel(fn, g, b, args, TVL1_RING_BYTES(ITER_NW), st);
     if (e != cudaSuccess) return fail(TVL1_ERR_CUDA, "cooperative launch of k_outer failed: %s", cudaGetErrorString(e));
     return TVL1_OK;
 }
 
-int launch_iterate2(IterArgs& a, cudaStream_t st)
+int launch_iterate2(IterArgs& a, cudaStream_t st, bool cs = false)
 {
     int grid = 1;
-    a.rows = tile_rows(a.w, a.h, TVL1_STRIP2, 3, 8, resident_blocks(KI_FUSED), &grid);   // 3 halo rows per tile
+    a.rows = tile_rows(a.w, a.h, TVL1_STRIP2, 3, 8, resident_blocks(KI_FUSED, cs), &grid);   // 3 halo rows per tile
     dim3 b(32, ITER_NW);
-    k_iterate2<ITER_NW><<<grid, b, TVL1_RING_BYTES(ITER_NW), st>>>(a);
+    if (cs) k_iterate2<ITER_NW, true><<<grid, b, TVL1_RING_BYTES(ITER_NW), st>>>(a);
+    else k_iterate2<ITER_NW><<<grid, b, TVL1_RING_BYTES(ITER_NW), st>>>(a);
     CK(cudaGetLastError());
     return TVL1_OK;
 }
@@ -651,6 +695,12 @@ static int ensure_gamma(tvl1_handle* H, cudaStream_t st)
 static int resolve_iterations(tvl1_handle* H)
 {
     const tvl1_params& p = H->prm;
+    if (p.semantics == TVL1_SEMANTICS_CUDA) {
+        // cv::cuda's flat loop: `iterations` iterations per (level, warp), no outer iterations
+        H->inner = p.iterations > 0 ? p.iterations : 300;
+        H->outer = 1;
+        return TVL1_OK;
+    }
     if (p.inner_iterations > 0 && p.outer_iterations > 0) {
         H->inner = p.inner_iterations;
         H->outer = p.outer_iterations;
@@ -672,6 +722,16 @@ static int check_params(const tvl1_params* p)
     if (!(p->scale_step > 0.0 && p->scale_step < 1.0)) return fail(TVL1_ERR_INVALID, "scaleStep must be in (0,1)");
     if (!(p->gamma == p->gamma)) return fail(TVL1_ERR_INVALID, "gamma is not a number");
     if (p->use_initial_flow) return fail(TVL1_ERR_UNSUPPORTED, "useInitialFlow is not supported (the reference never forwards it)");
+    if (p->semantics != TVL1_SEMANTICS_CPU && p->semantics != TVL1_SEMANTICS_CUDA)
+        return fail(TVL1_ERR_INVALID, "semantics must be TVL1_SEMANTICS_CPU (0) or TVL1_SEMANTICS_CUDA (1)");
+    if (p->semantics == TVL1_SEMANTICS_CUDA) {   // medianFiltering is not read in this mode
+        if (p->inner_iterations > 0 || p->outer_iterations > 0)
+            return fail(TVL1_ERR_INVALID, "cuda semantics has one flat loop of `iterations`: inner/outer iterations must be <= 0");
+        if (p->gamma != 0.0) return fail(TVL1_ERR_UNSUPPORTED, "gamma != 0 is not supported with cuda semantics");
+        if (!(p->theta > 0.0)) return fail(TVL1_ERR_INVALID, "theta must be > 0");
+        if (!(p->lambda >= 0.0)) return fail(TVL1_ERR_INVALID, "lambda must be >= 0");
+        return TVL1_OK;
+    }
     if (p->median_filtering != 1 && p->median_filtering != 3 && p->median_filtering != 5)   // cv::medianBlur's fp32 apertures
         return fail(TVL1_ERR_UNSUPPORTED, "medianFiltering must be 1 (off), 3 or 5");
     if (!(p->theta > 0.0)) return fail(TVL1_ERR_INVALID, "theta must be > 0");
@@ -699,6 +759,8 @@ static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const u
     const float l_t = (float)(P.lambda * P.theta);
     const float taut = (float)(P.tau / P.theta);
     const float theta = (float)P.theta;
+    // TVL1_SEMANTICS_CUDA: cv::cuda's resize, warp and flat loop with its sparse stop test, no median
+    const bool cs = P.semantics == TVL1_SEMANTICS_CUDA;
     long long launches = 0;
     H->ev_used = 0;
 
@@ -728,7 +790,8 @@ static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const u
     launches += 2;
     for (int s = 1; s < L; s++) {
         const Level &a = H->lv[s - 1], &b = H->lv[s];
-        if ((rc = launch_resize2(a.I0, a.I1, a.w, a.h, a.pitch, b.I0, b.I1, b.w, b.h, b.pitch, P.scale_step, 1.f, 0, st))) return rc;
+        if ((rc = (cs ? launch_resize_cuda2 : launch_resize2)(a.I0, a.I1, a.w, a.h, a.pitch, b.I0, b.I1, b.w, b.h, b.pitch,
+                                                              P.scale_step, 1.f, 0, st))) return rc;
         launches += 1;
     }
     {
@@ -763,6 +826,8 @@ static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const u
         ia.level = s; ia.ctrl = H->d_ctrl; ia.partials = H->d_partials; ia.errlog = nullptr;
         ia.mode = 0; ia.inner_max = H->inner;
         ia.tm = lv.tm_iter;
+        ia.eps_d = P.epsilon * P.epsilon * (double)(lv.w * lv.h);
+        ia.err_on = P.epsilon > 0.0;
         const bool with_gamma = P.gamma != 0.0;
         GammaArgs ga;
         if (with_gamma) {
@@ -798,7 +863,7 @@ static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const u
             // (2) warp I1 by the current flow; also re-arms the stop test (error = FLT_MAX)
             if ((rc = span_begin(1, s))) return rc;
             for (int k = 0; k < 4; k++) wa.pz[k] = wi == 0 ? H->p[k][0] : nullptr;
-            if ((rc = launch_warp(wa, st))) return rc;
+            if ((rc = cs ? launch_warp_cuda(wa, st) : launch_warp(wa, st))) return rc;
             launches++;
             span_end();
             // (3) outer iterations: median + up to `inner` primal-dual iterations.  Every kernel is a
@@ -810,7 +875,7 @@ static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const u
             const int pred_total = wi > 0 ? counts[slot - 1] : (s < L - 1 ? counts[(s + 1) * W] : H->inner);
             int done_total = 0;
             for (int no = 0; no < H->outer; ++no) {
-                if (P.median_filtering > 1) {
+                if (P.median_filtering > 1 && !cs) {
                     if ((rc = span_begin(2, s))) return rc;
                     if ((rc = P.median_filtering == 3 ? launch_median3(ma, 2, st) : launch_median(ma, 2, st))) return rc;
                     launches++;
@@ -835,7 +900,7 @@ static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const u
                         // the whole inner loop of this outer iteration in one cooperative launch
                         IterArgs io = ia;
                         io.mode = 2;
-                        if ((rc = launch_outer(io, st))) return rc;
+                        if ((rc = launch_outer(io, st, cs))) return rc;
                         launches += 1;
                     } else if (fused) {
                         // temporally blocked schedule: [fused pair | single] slot pairs.  Which slot
@@ -846,21 +911,21 @@ static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const u
                         i2.mode = 2; i1.mode = 1;
                         const int groups = (want + 1) / 2;
                         for (int k = 0; k < groups; ++k) {
-                            if ((rc = launch_iterate2(i2, st))) return rc;
-                            if ((rc = launch_iterate(i1, st))) return rc;
+                            if ((rc = launch_iterate2(i2, st, cs))) return rc;
+                            if ((rc = launch_iterate(i1, st, cs))) return rc;
                         }
                         launches += 2 * groups;
                     } else if (multi) {
                         // small level: one cooperative launch runs the rest of this outer iteration
                         IterArgs im = ia;
                         im.mode = 3;
-                        if ((rc = launch_iterate_multi(im, st))) return rc;
+                        if ((rc = launch_iterate_multi(im, st, cs))) return rc;
                         launches += 1;
                     } else {
                         IterArgs i3 = ia;
                         i3.mode = 3;
                         for (int k = 0; k < want; ++k)
-                            if ((rc = launch_iterate(i3, st))) return rc;
+                            if ((rc = launch_iterate(i3, st, cs))) return rc;
                         launches += want;
                     }
                     if ((rc = copy_words(H->d_ctrl, H->h_ctrl, (int)(hdr / 4), st))) return rc;   // no copy engine: see copy_words
@@ -887,8 +952,8 @@ static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const u
         const int uc = H->h_ctrl->ucur[s];
         const float mul = (float)(1 / P.scale_step);
         if ((rc = span_begin(3, s))) return rc;
-        if ((rc = launch_resize2(uc ? H->u1x : lv.u1, uc ? H->u2x : lv.u2, lv.w, lv.h, lv.pitch, up.u1, up.u2, up.w, up.h,
-                                 up.pitch, 0.0, mul, 1, st))) return rc;
+        if ((rc = (cs ? launch_resize_cuda2 : launch_resize2)(uc ? H->u1x : lv.u1, uc ? H->u2x : lv.u2, lv.w, lv.h, lv.pitch,
+                                                              up.u1, up.u2, up.w, up.h, up.pitch, 0.0, mul, 1, st))) return rc;
         launches += 1;
         if (with_gamma) {   // u3 is zoomed like the flow but not scaled
             if ((rc = launch_resize(H->u3[s], lv.w, lv.h, lv.pitch, H->u3[s - 1], up.w, up.h, up.pitch, 0.0, 1.f, 0, st))) return rc;
@@ -1306,6 +1371,15 @@ int tvl1_k_resize(const float* d_src, int sw, int sh, int spitch, float* d_dst, 
     return launch_resize(d_src, sw, sh, spitch, d_dst, dw, dh, dpitch, inv_scale, mul, mul != 1.f, (cudaStream_t)stream);
 }
 
+int tvl1_k_resize_cuda(const float* d_src, int sw, int sh, int spitch, float* d_dst, int dw, int dh, int dpitch,
+                       double inv_scale, float mul, void* stream)
+{
+    if (!d_src || !d_dst || sw <= 0 || sh <= 0 || dw <= 0 || dh <= 0 || spitch < sw || dpitch < dw)
+        return fail(TVL1_ERR_INVALID, "bad argument");
+    return launch_resize_cuda2(d_src, nullptr, sw, sh, spitch, d_dst, nullptr, dw, dh, dpitch, inv_scale, mul, mul != 1.f,
+                               (cudaStream_t)stream);
+}
+
 int tvl1_k_centered_gradient(const float* d_src, int w, int h, int pitch, float* d_dx, float* d_dy, void* stream)
 {
     if (!d_src || !d_dx || !d_dy || w <= 0 || h <= 0) return fail(TVL1_ERR_INVALID, "bad argument");
@@ -1331,6 +1405,24 @@ int tvl1_k_warp(const float* d_I0, const float* d_I1, const float* d_u1, const f
         if ((rc = make_plane_map(&a.tmI1[k], d_I1, pitch, h, TVL1_WP_RW, k == 0 ? 16 : TVL1_WP_RH))) return rc;
     stage_begin((cudaStream_t)stream);
     rc = launch_warp(a, (cudaStream_t)stream);
+    stage_end((cudaStream_t)stream);
+    return rc;
+}
+
+int tvl1_k_warp_cuda(const float* d_I0, const float* d_I1, const float* d_u1, const float* d_u2, int w, int h,
+                     int pitch, float* d_I1w, float* d_I1wx, float* d_I1wy, float* d_grad, float* d_rho_c, void* stream)
+{
+    if (!d_I0 || !d_I1 || !d_u1 || !d_u2 || !d_I1wx || !d_I1wy || !d_rho_c || w <= 0 || h <= 0 || pitch < w)
+        return fail(TVL1_ERR_INVALID, "bad argument");
+    WarpArgs a;
+    memset(a.tmI1, 0, sizeof(a.tmI1));   // k_warp_cuda stages its windows with plain loads
+    a.I0 = d_I0; a.I1 = d_I1;
+    a.u1[0] = a.u1[1] = d_u1; a.u2[0] = a.u2[1] = d_u2;
+    a.I1w = d_I1w; a.I1wx = d_I1wx; a.I1wy = d_I1wy; a.grad = d_grad; a.rho_c = d_rho_c;
+    a.w = w; a.h = h; a.pitch = pitch; a.level = -1; a.ctrl = nullptr; a.one = 1.0f;
+    for (int k = 0; k < 4; k++) a.pz[k] = nullptr;
+    stage_begin((cudaStream_t)stream);
+    const int rc = launch_warp_cuda(a, (cudaStream_t)stream);
     stage_end((cudaStream_t)stream);
     return rc;
 }

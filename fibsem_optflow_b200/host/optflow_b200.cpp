@@ -196,6 +196,18 @@ tvl1_params tv_params(const Value& im, const Value& args)
     p.inner_iterations = (int)pick(im, args, "innerIterations", Value(0)).asInt();
     p.outer_iterations = (int)pick(im, args, "outerIterations", Value(0)).asInt();
     p.median_filtering = (int)pick(im, args, "medianFiltering", Value(5)).asInt();
+    // "cpu" (default): cv::DualTVL1OpticalFlow; "cuda": cv::cuda::OpticalFlowDual_TVL1's algorithm, whose flat
+    // loop has no inner / outer iterations and no median -- those keys are refused rather than ignored
+    const std::string sem = pick(im, args, "semantics", Value("cpu")).asString();
+    if (sem == "cuda") {
+        p.semantics = TVL1_SEMANTICS_CUDA;
+        for (const char* k : {"innerIterations", "outerIterations", "medianFiltering"})
+            if (im.isMember(k) || args.isMember(k))
+                pair_fail(std::string("\"") + k + "\" has no meaning with \"semantics\": \"cuda\"");
+        p.median_filtering = 1;
+    } else if (sem != "cpu") {
+        pair_fail("\"semantics\" must be \"cpu\" or \"cuda\", not \"" + sem + "\"");
+    }
     return p;
 }
 

@@ -22,11 +22,20 @@
  *   tvl1_prescale_u8                    <- the loader's cv::resize   src/optflow.cpp:111,124
  *   tvl1_stack_run                      <- the pair loop of from_file   src/optflow.cpp:75-178
  *
- * NUMERICS: the solver computes what OpenCV's CPU class cv::DualTVL1OpticalFlow computes (cubic
- * 1/32-px remap, 5x5 median per outer iteration, stop test every iteration), bit for bit against
- * the CPU restatement in oracle/.  The reference BINARY calls cv::cuda::OpticalFlowDual_TVL1
- * (src/optflow.cpp:518: flat loop, no median, another bicubic, fast-math), so outputs are not
- * bit-comparable with that binary's for the same job; see DESIGN.md section 1.
+ * NUMERICS: by default (semantics = TVL1_SEMANTICS_CPU) the solver computes what OpenCV's CPU class
+ * cv::DualTVL1OpticalFlow computes (cubic 1/32-px remap, 5x5 median per outer iteration, stop test
+ * every iteration), bit for bit against the CPU restatement in oracle/.  The reference BINARY calls
+ * cv::cuda::OpticalFlowDual_TVL1 (src/optflow.cpp:518).  semantics = TVL1_SEMANTICS_CUDA computes that
+ * class's ALGORITHM: cuda::resize's linear mapping without the half-pixel offset, warpBackward's
+ * normalised A = -0.5 cubic with clamped reads, one flat loop of `iterations` per (level, warp) with no
+ * median and the error evaluated only on odd iterations while its budget lasts, the sum in fp64 --
+ * in IEEE fp32 arithmetic, bit for bit against its CPU restatement in oracle/.  It does NOT reproduce
+ * the binary's bits: not its --use_fast_math rounding (approximate division and square root,
+ * flush-to-zero, FMA contraction), not CUDA's hypotf (up to 3 ulp; here the canonical double-rounded
+ * hypot), not the order of cuda::sum's reduction, not a 9-bit-weight texture path OpenCV may take for the
+ * upsampling.  Those differ from this mode by rounding, not by algorithm.  The restatement comes from
+ * OpenCV 3.4.1 as recalled (SURVEY.md Appendix B); OpenCV's CUDA sources were not at hand to check it
+ * against.  See DESIGN.md section 1.
  *
  * Conventions: plain pointers and sizes, no C++ or torch types.  "d_" pointers are
  * device memory on the handle's device, "h_" pointers are host memory.  8-bit images
@@ -53,6 +62,9 @@ extern "C" {
 #define TVL1_ERR_UNSUPPORTED (-3)
 #define TVL1_ERR_NOMEM (-4)
 
+#define TVL1_SEMANTICS_CPU 0    /* tvl1_params.semantics: cv::DualTVL1OpticalFlow (default) */
+#define TVL1_SEMANTICS_CUDA 1   /* cv::cuda::OpticalFlowDual_TVL1's algorithm, see NUMERICS above */
+
 #define TVL1_MAX_LEVELS 32
 #define TVL1_MAX_WARPS 64
 
@@ -76,7 +88,11 @@ typedef struct tvl1_params {
     int median_filtering;   /* 5 (CPU class); 3; 1 = off */
     int use_initial_flow;   /* read by the reference but never forwarded
                                (src/optflow.cpp:512,518); must be 0 */
-    int reserved[3];
+    int semantics;          /* TVL1_SEMANTICS_CPU (0, default) or TVL1_SEMANTICS_CUDA (1).  CUDA: `iterations`
+                               is the flat count per (level, warp); inner/outer iterations must be <= 0
+                               (TVL1_ERR_INVALID), gamma must be 0 (TVL1_ERR_UNSUPPORTED), median_filtering
+                               is not read.  stats.outer[] and ms_median are 0 */
+    int reserved[2];
 } tvl1_params;
 
 /* Iteration counts and stage times of the last calc. */
@@ -276,6 +292,14 @@ int tvl1_k_centered_gradient(const float* d_src, int w, int h, int pitch, float*
 int tvl1_k_warp(const float* d_I0, const float* d_I1, const float* d_u1, const float* d_u2,
                 int w, int h, int pitch, float* d_I1w, float* d_I1wx, float* d_I1wy,
                 float* d_grad, float* d_rho_c, void* stream);
+/* TVL1_SEMANTICS_CUDA's stages: cuda::resize(INTER_LINEAR) (inv_scale > 0: by that factor, else to dw x dh;
+ * then times mul) and warpBackward + calcGradRho (I1's centred gradients formed inside, clamped reads).  Same
+ * arguments as tvl1_k_resize / tvl1_k_warp. */
+int tvl1_k_resize_cuda(const float* d_src, int sw, int sh, int spitch, float* d_dst, int dw, int dh,
+                       int dpitch, double inv_scale, float mul, void* stream);
+int tvl1_k_warp_cuda(const float* d_I0, const float* d_I1, const float* d_u1, const float* d_u2,
+                     int w, int h, int pitch, float* d_I1w, float* d_I1wx, float* d_I1wy,
+                     float* d_grad, float* d_rho_c, void* stream);
 /* n inner iterations with no stop test; state planes are updated in place (the result
  * is copied back if it ends in the internal twin buffers).  errors (host, may be NULL)
  * receives the n per-iteration error sums. */
@@ -326,7 +350,7 @@ int tvl1_features_extract(tvl1_handle* h, const uint8_t* d_img, size_t pitch, in
                           const tvl1_feature_params* prm, void* d_kp, uint32_t* d_desc, int cap, int* n_out,
                           void* stream);
 /* CUDA-event time of the kernel launches of the calling thread's most recent tvl1_k_warp /
- * tvl1_k_iterate / tvl1_k_median5 call (waits for them). */
+ * tvl1_k_warp_cuda / tvl1_k_iterate / tvl1_k_median5 call (waits for them). */
 int tvl1_k_last_ms(float* ms);
 
 /* Self-test of the kernels' exact fast paths (reciprocal-sharing division, fused hypot) against
