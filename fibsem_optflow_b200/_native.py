@@ -15,6 +15,8 @@ MAX_LEVELS = 32
 MAX_WARPS = 64
 SEMANTICS_CPU = 0    # TVL1_SEMANTICS_CPU: cv::DualTVL1OpticalFlow (default)
 SEMANTICS_CUDA = 1   # TVL1_SEMANTICS_CUDA: cv::cuda::OpticalFlowDual_TVL1's algorithm
+FRAME_U8 = 0         # TVL1_FRAME_U8: tvl1_calc_ex frame type, 8-bit rows
+FRAME_F32 = 1        # TVL1_FRAME_F32: fp32 rows, scaled by 255 like convertTo
 
 
 class Tvl1Error(RuntimeError):
@@ -82,9 +84,10 @@ class StackIO(C.Structure):
 EXPORTS = [
     "tvl1_version", "tvl1_last_error", "tvl1_default_params", "tvl1_create", "tvl1_destroy",
     "tvl1_set_params", "tvl1_set_option", "tvl1_set_timing", "tvl1_calc_u8", "tvl1_calc_u8_host",
+    "tvl1_calc_ex", "tvl1_calc_ex_host",
     "tvl1_prescaled_size", "tvl1_prescale_u8", "tvl1_prescale_u8_host",
     "tvl1_mask_flow_u8", "tvl1_finish_flow_u8", "tvl1_sample_matches", "tvl1_sample_matches_skip", "tvl1_sample_matches_ex",
-    "tvl1_default_feature_params", "tvl1_find_alignment", "tvl1_warp_affine_u8", "tvl1_warp_affine_f32", "tvl1_stack_run", "tvl1_k_convert_u8", "tvl1_k_resize",
+    "tvl1_default_feature_params", "tvl1_find_alignment", "tvl1_warp_affine_u8", "tvl1_warp_affine_f32", "tvl1_stack_run", "tvl1_k_convert_u8", "tvl1_k_convert_f32", "tvl1_k_resize",
     "tvl1_k_centered_gradient", "tvl1_k_warp", "tvl1_k_resize_cuda", "tvl1_k_warp_cuda", "tvl1_k_iterate", "tvl1_k_iterate_fused2", "tvl1_k_outer", "tvl1_k_iterate_gamma", "tvl1_k_median5", "tvl1_k_median3", "tvl1_k_last_ms",
     "tvl1_k_gauss7_u8", "tvl1_k_fast_corners", "tvl1_k_describe", "tvl1_k_knn2", "tvl1_features_extract",
     "tvl1_pyramid_sizes", "tvl1_glibc_rand", "tvl1_selftest_arith", "tvl1_dev_count", "tvl1_dev_alloc", "tvl1_dev_free",
@@ -129,6 +132,10 @@ def lib():
                                C.POINTER(Stats)]
     L.tvl1_calc_u8_host.argtypes = [_vp, _vp, _sz, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz,
                                     C.POINTER(Stats)]
+    L.tvl1_calc_ex.argtypes = [_vp, C.c_int, _vp, _sz, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, _vp, _vp, _sz, _vp,
+                               C.POINTER(Stats)]
+    L.tvl1_calc_ex_host.argtypes = [_vp, C.c_int, _vp, _sz, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, _vp, _vp, _sz,
+                                    C.POINTER(Stats)]
     L.tvl1_mask_flow_u8.argtypes = [_vp, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, _vp]
     L.tvl1_finish_flow_u8.argtypes = [_vp, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, C.c_int, _vp]
     L.tvl1_sample_matches.argtypes = [_vp, _vp, _sz, _vp, _sz, _vp, _vp, _sz, C.c_int, C.c_int,
@@ -147,6 +154,7 @@ def lib():
     L.tvl1_warp_affine_f32.argtypes = [_vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, C.c_int, C.c_int, _vp]
     L.tvl1_stack_run.argtypes = [_vp, C.POINTER(StackIO), C.POINTER(C.c_float)]
     L.tvl1_k_convert_u8.argtypes = [_vp, _sz, C.c_int, C.c_int, _vp, C.c_int, _vp]
+    L.tvl1_k_convert_f32.argtypes = L.tvl1_k_convert_u8.argtypes
     L.tvl1_k_resize.argtypes = [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, C.c_int, C.c_int,
                                 C.c_double, C.c_float, _vp]
     L.tvl1_k_centered_gradient.argtypes = [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp]
@@ -384,9 +392,40 @@ class Solver:
                                       u.ctypes.data, v.ctypes.data, w * 4, C.byref(self.stats)))
         return u, v
 
+    def calc_ex(self, I0, I1, init=None):
+        """calc(I0, I1, flow) of the OpenCV classes (tvl1_calc_ex_host): host frames, both uint8 or both float32
+        (scaled by 255 like convertTo), and init = (u0, v0) float32 planes the solve starts from (useInitialFlow),
+        or None for a zero start.  Returns (u, v) host float32."""
+        I0, I1 = np.asarray(I0), np.asarray(I1)
+        if I0.dtype != I1.dtype or I0.dtype not in (np.uint8, np.float32):
+            raise Tvl1Error("frames must both be uint8 or both float32, not %s and %s" % (I0.dtype, I1.dtype))
+        if I0.ndim != 2 or I0.shape != I1.shape:
+            raise Tvl1Error("frames must be 2-D arrays of equal size")
+        I0, I1 = np.ascontiguousarray(I0), np.ascontiguousarray(I1)
+        ft = FRAME_U8 if I0.dtype == np.uint8 else FRAME_F32
+        h, w = I0.shape
+        u0 = v0 = None
+        if init is not None:
+            u0, v0 = (np.ascontiguousarray(a, np.float32) for a in init)
+            if u0.shape != (h, w) or v0.shape != (h, w):
+                raise Tvl1Error("the initial flow planes must have the frames' size")
+        u = np.empty((h, w), np.float32)
+        v = np.empty((h, w), np.float32)
+        e = I0.itemsize
+        check(lib().tvl1_calc_ex_host(self.handle, ft, I0.ctypes.data, w * e, I1.ctypes.data, w * e, w, h,
+                                      None if u0 is None else u0.ctypes.data, None if v0 is None else v0.ctypes.data,
+                                      w * 4, u.ctypes.data, v.ctypes.data, w * 4, C.byref(self.stats)))
+        return u, v
+
     def calc_device(self, d_f0, pitch0, d_f1, pitch1, w, h, d_u, d_v, pitch_out, stream=None):
         check(lib().tvl1_calc_u8(self.handle, d_f0, pitch0, d_f1, pitch1, w, h, d_u, d_v,
                                  pitch_out, stream, C.byref(self.stats)))
+
+    def calc_ex_device(self, frame_type, d_f0, pitch0, d_f1, pitch1, w, h, d_u0, d_v0, pitch_init, d_u, d_v,
+                       pitch_out, stream=None):
+        """tvl1_calc_ex on device pointers (d_u0 / d_v0 None: zero start); returns the status, raises on error"""
+        return check(lib().tvl1_calc_ex(self.handle, frame_type, d_f0, pitch0, d_f1, pitch1, w, h, d_u0, d_v0,
+                                        pitch_init, d_u, d_v, pitch_out, stream, C.byref(self.stats)))
 
     def mask_flow_device(self, d_f1, pitch1, w, h, d_u, d_v, pitch_out, stream=None):
         check(lib().tvl1_mask_flow_u8(self.handle, d_f1, pitch1, w, h, d_u, d_v, pitch_out, stream))
@@ -540,6 +579,24 @@ def k_convert_u8(img, device=0):
     check(lib().tvl1_k_convert_u8(src.ptr, w, w, h, dst.ptr, dst.pitch, None))
     check(lib().tvl1_dev_sync(device))
     return dst.get()
+
+
+def k_convert_f32(img, spitch=None, device=0):
+    """fp32 frame -> level 0 (x 255).  spitch: row pitch of the device copy in elements (default: the width); the
+    padding holds NaN, which must not be read."""
+    img = np.ascontiguousarray(img, np.float32)
+    h, w = img.shape
+    sp = int(spitch or w)
+    a = np.full((h, sp), np.nan, np.float32)
+    a[:, :w] = img
+    src = DevBuf(a.nbytes, device).upload(a)
+    dst = DevBuf(h * pitch_of(w) * 4, device).upload(np.full((h, pitch_of(w)), 7.0, np.float32))
+    check(lib().tvl1_k_convert_f32(src.ptr, sp * 4, w, h, dst.ptr, pitch_of(w), None))
+    check(lib().tvl1_dev_sync(device))
+    out = dst.download((h, pitch_of(w)), np.float32)
+    src.free()
+    dst.free()
+    return out   # with the pad columns
 
 
 def k_resize(src, dw=None, dh=None, inv_scale=0.0, mul=1.0, device=0):

@@ -112,11 +112,14 @@ def release_solvers():
     _solvers.clear()
 
 
-def TVL1_solve(frame0, frame1, TV_args, device=0):
-    """Flow from frame0 to frame1 (uint8, equal size) -> (flow_x, flow_y) float32 planes."""
+def TVL1_solve(frame0, frame1, TV_args, device=0, init_flow=None):
+    """Flow from frame0 to frame1 (uint8, equal size) -> (flow_x, flow_y) float32 planes.  init_flow: (flow_x,
+    flow_y) float32 planes the solve starts from (OpenCV's useInitialFlow + calc(I0, I1, flow)); with it, the frames
+    may also both be float32 (scaled by 255, as the OpenCV classes' convertTo does)."""
     s = _solver_for(TV_args, device)
-    u, v = s.calc(frame0, frame1)
-    return u, v
+    if init_flow is None:
+        return s.calc(frame0, frame1)
+    return s.calc_ex(frame0, frame1, init=init_flow)
 
 
 # orb_defaults (src/features.cpp:19-32) and the matcher / RANSAC keys (:107, :133)

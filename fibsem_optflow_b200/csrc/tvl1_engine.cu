@@ -181,18 +181,31 @@ int launch_convert(const uint8_t* src, size_t pitch, int w, int h, float* dst, i
     return TVL1_OK;
 }
 
-// one or two planes (srcB / dstB may be null) resized alike in one launch
+// fp32 frame (byte pitch, a multiple of 4) -> level 0, x 255
+int launch_convert_f32(const float* src, size_t pitch_bytes, int w, int h, float* dst, int dpitch, cudaStream_t st)
+{
+    dim3 b(32, 8);
+    dim3 g(cdiv(cdiv(w, 4), 32), cdiv(h, 8));
+    k_convert_f32<<<g, b, 0, st>>>(src, pitch_bytes / 4, w, h, dst, dpitch);
+    CK(cudaGetLastError());
+    return TVL1_OK;
+}
+
+// one or two planes (srcB / dstB may be null) resized alike in one launch; apply_mul: see scale_px
 int launch_resize2(const float* srcA, const float* srcB, int sw, int sh, int sp, float* dstA, float* dstB, int dw, int dh,
-                   int dp, double inv_scale, float mul, int apply_mul, cudaStream_t st)
+                   int dp, double inv_scale, double mul, int apply_mul, cudaStream_t st)
 {
     double inv_x, inv_y;
     if (inv_scale > 0) { inv_x = inv_scale; inv_y = inv_scale; }
     else { inv_x = (double)dw / sw; inv_y = (double)dh / sh; }
     const double scale_x = 1. / inv_x, scale_y = 1. / inv_y;
     dim3 b(32, 8);
-    if (inv_scale == 0.5 && !apply_mul) {   // resize(src, Size(), 0.5, 0.5): OpenCV's INTER_AREA fast path
+    // resize(src, Size(), 0.5, 0.5): OpenCV's INTER_AREA fast path.  The fp32 multiply (tvl1_k_resize with mul != 1)
+    // has always taken the bilinear kernel at 0.5 and keeps doing so; the fp64 one (an initial flow's downscale) is
+    // cv::resize followed by cv::multiply and so takes the area path like the image pyramid
+    if (inv_scale == 0.5 && apply_mul != 1) {
         dim3 gh(cdiv(dw, 32), cdiv(dh, 8), srcB ? 2 : 1);
-        k_resize_half<<<gh, b, 0, st>>>(srcA, srcB, sw, sh, sp, dstA, dstB, dw, dh, dp);
+        k_resize_half<<<gh, b, 0, st>>>(srcA, srcB, sw, sh, sp, dstA, dstB, dw, dh, dp, mul, apply_mul);
         CK(cudaGetLastError());
         return TVL1_OK;
     }
@@ -203,7 +216,7 @@ int launch_resize2(const float* srcA, const float* srcB, int sw, int sh, int sp,
 }
 
 int launch_resize(const float* src, int sw, int sh, int sp, float* dst, int dw, int dh, int dp,
-                  double inv_scale, float mul, int apply_mul, cudaStream_t st)
+                  double inv_scale, double mul, int apply_mul, cudaStream_t st)
 {
     return launch_resize2(src, nullptr, sw, sh, sp, dst, nullptr, dw, dh, dp, inv_scale, mul, apply_mul, st);
 }
@@ -211,14 +224,14 @@ int launch_resize(const float* src, int sw, int sh, int sp, float* dst, int dw, 
 // cv::cuda semantics: cuda::resize(INTER_LINEAR) of one or two planes (srcB / dstB may be null).  inv_scale > 0:
 // resize(src, Size(), inv_scale, inv_scale); otherwise the explicit size dw x dh (factor dw / sw in fp64).
 int launch_resize_cuda2(const float* srcA, const float* srcB, int sw, int sh, int sp, float* dstA, float* dstB, int dw,
-                        int dh, int dp, double inv_scale, float mul, int apply_mul, cudaStream_t st)
+                        int dh, int dp, double inv_scale, double mul, int apply_mul, cudaStream_t st)
 {
     const double f_x = inv_scale > 0 ? inv_scale : (double)dw / sw;
     const double f_y = inv_scale > 0 ? inv_scale : (double)dh / sh;
     const float fx = (float)(1.0 / f_x), fy = (float)(1.0 / f_y);
     dim3 b(32, 8);
     dim3 g(cdiv(dw, 32), cdiv(dh, 8), srcB ? 2 : 1);
-    k_resize_cuda<<<g, b, 0, st>>>(srcA, srcB, sw, sh, sp, dstA, dstB, dw, dh, dp, fx, fy, mul, apply_mul);
+    k_resize_cuda<<<g, b, 0, st>>>(srcA, srcB, sw, sh, sp, dstA, dstB, dw, dh, dp, fx, fy, (float)mul, apply_mul);
     CK(cudaGetLastError());
     return TVL1_OK;
 }
@@ -547,10 +560,11 @@ struct tvl1_handle {
     Ctrl* h_ctrl = nullptr;                 // pinned
     double* d_partials = nullptr;
     size_t partials_cap = 0;
-    // staging for the host-buffer entry point
-    uint8_t *d_f0 = nullptr, *d_f1 = nullptr;
-    float *d_uo = nullptr, *d_vo = nullptr;
-    size_t stage_pitch8 = 0;
+    // staging for the host-buffer entry points: frames (rows of stage_pitch bytes, u8 or fp32), flow out, and the
+    // initial flow (allocated on first use); reallocated when the size changes or fp32 rows need more room
+    void *d_f0 = nullptr, *d_f1 = nullptr;
+    float *d_uo = nullptr, *d_vo = nullptr, *d_ui = nullptr, *d_vi = nullptr;
+    size_t stage_pitch = 0;
     int stage_w = 0, stage_h = 0;
     cudaStream_t own_stream = nullptr;
     std::vector<cudaEvent_t> events;
@@ -739,18 +753,34 @@ static int check_params(const tvl1_params* p)
     return TVL1_OK;
 }
 
-// the solve proper; everything is enqueued on `st`
-static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const uint8_t* f1, size_t pitch1,
-                       int w, int h, float* d_u, float* d_v, size_t pitch_out, cudaStream_t st,
-                       tvl1_stats* stats)
+// frame type, row pitches and initial-flow planes of tvl1_calc_ex[_host]
+static int check_frames(int frame_type, size_t pitch0, size_t pitch1, int w, int h, const float* u0, const float* v0,
+                        size_t pitch_init, size_t pitch_out)
+{
+    if (w <= 0 || h <= 0) return fail(TVL1_ERR_INVALID, "empty image (%dx%d)", w, h);
+    if (frame_type != TVL1_FRAME_U8 && frame_type != TVL1_FRAME_F32)
+        return fail(TVL1_ERR_INVALID, "frame_type must be TVL1_FRAME_U8 (0) or TVL1_FRAME_F32 (1)");
+    const size_t row = (size_t)w * (frame_type == TVL1_FRAME_F32 ? 4 : 1);
+    if (pitch0 < row || pitch1 < row || pitch_out < (size_t)w * 4) return fail(TVL1_ERR_INVALID, "pitch smaller than a row");
+    if (frame_type == TVL1_FRAME_F32 && (pitch0 % 4 || pitch1 % 4))
+        return fail(TVL1_ERR_INVALID, "fp32 frame pitches must be multiples of 4 bytes");
+    if ((u0 == nullptr) != (v0 == nullptr)) return fail(TVL1_ERR_INVALID, "the initial flow needs both planes (or neither)");
+    if (u0 && (pitch_init % 4 || pitch_init < (size_t)w * 4))
+        return fail(TVL1_ERR_INVALID, "initial-flow pitch must be a multiple of 4 bytes and at least a row");
+    return TVL1_OK;
+}
+
+// the solve proper; everything is enqueued on `st`.  u0 / v0 (both or neither): the initial flow (useInitialFlow),
+// which may be d_u / d_v themselves
+static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pitch0, const void* f1, size_t pitch1,
+                       int w, int h, const float* u0, const float* v0, size_t pitch_init,
+                       float* d_u, float* d_v, size_t pitch_out, cudaStream_t st, tvl1_stats* stats)
 {
     if (!f0 || !f1 || !d_u || !d_v) return fail(TVL1_ERR_INVALID, "null image or flow pointer");
-    if (w <= 0 || h <= 0) return fail(TVL1_ERR_INVALID, "empty image (%dx%d)", w, h);
+    int rc = check_frames(frame_type, pitch0, pitch1, w, h, u0, v0, pitch_init, pitch_out);
+    if (rc) return rc;
     if (w > 32767 || h > 32767) return fail(TVL1_ERR_INVALID, "image side > 32767 (remap uses int16 coordinates)");
-    if (pitch0 < (size_t)w || pitch1 < (size_t)w || pitch_out < (size_t)w * 4)
-        return fail(TVL1_ERR_INVALID, "pitch smaller than a row");
     CK(cudaSetDevice(H->device));
-    int rc;
     if ((rc = ensure_capacity(H, w, h, st))) return rc;
     if ((rc = ensure_gamma(H, st))) return rc;
     if ((rc = upload_cubic_table(H->device))) return rc;
@@ -785,8 +815,13 @@ static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const u
     CK(cudaEventRecord(ev_begin, st));
     CK(cudaMemsetAsync(H->d_ctrl, 0, sizeof(Ctrl), st));
     // (1) pyramid: convert, then resize level by level
-    if ((rc = launch_convert(f0, pitch0, w, h, H->lv[0].I0, H->lv[0].pitch, st))) return rc;
-    if ((rc = launch_convert(f1, pitch1, w, h, H->lv[0].I1, H->lv[0].pitch, st))) return rc;
+    if (frame_type == TVL1_FRAME_F32) {
+        if ((rc = launch_convert_f32((const float*)f0, pitch0, w, h, H->lv[0].I0, H->lv[0].pitch, st))) return rc;
+        if ((rc = launch_convert_f32((const float*)f1, pitch1, w, h, H->lv[0].I1, H->lv[0].pitch, st))) return rc;
+    } else {
+        if ((rc = launch_convert((const uint8_t*)f0, pitch0, w, h, H->lv[0].I0, H->lv[0].pitch, st))) return rc;
+        if ((rc = launch_convert((const uint8_t*)f1, pitch1, w, h, H->lv[0].I1, H->lv[0].pitch, st))) return rc;
+    }
     launches += 2;
     for (int s = 1; s < L; s++) {
         const Level &a = H->lv[s - 1], &b = H->lv[s];
@@ -794,11 +829,31 @@ static int calc_device(tvl1_handle* H, const uint8_t* f0, size_t pitch0, const u
                                                               P.scale_step, 1.f, 0, st))) return rc;
         launches += 1;
     }
+    if (u0) {
+        // useInitialFlow: level 0 is the caller's flow, each coarser level the image pyramid's resize of the finer
+        // one, then times scaleStep as a rounding of its own -- cv::multiply by a double Scalar in the CPU class,
+        // an fp32 product in cv::cuda (SURVEY.md A.2a, Appendix B).  Into twin 0, which ucur names after the Ctrl
+        // memset; the coarsest level is not zeroed, the finer ones are overwritten by the upsample as usual.
+        const Level& l0 = H->lv[0];
+        CK(cudaMemcpy2DAsync(l0.u1, (size_t)l0.pitch * 4, u0, pitch_init, (size_t)w * 4, h, cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpy2DAsync(l0.u2, (size_t)l0.pitch * 4, v0, pitch_init, (size_t)w * 4, h, cudaMemcpyDeviceToDevice, st));
+        for (int s = 1; s < L; s++) {
+            const Level &a = H->lv[s - 1], &b = H->lv[s];
+            rc = cs ? launch_resize_cuda2(a.u1, a.u2, a.w, a.h, a.pitch, b.u1, b.u2, b.w, b.h, b.pitch, P.scale_step,
+                                          (float)P.scale_step, 1, st)
+                    : launch_resize2(a.u1, a.u2, a.w, a.h, a.pitch, b.u1, b.u2, b.w, b.h, b.pitch, P.scale_step,
+                                     P.scale_step, 2, st);
+            if (rc) return rc;
+            launches += 1;
+        }
+    }
     {
         const Level& c = H->lv[L - 1];
         const size_t b = (size_t)c.pitch * c.h * sizeof(float);
-        CK(cudaMemsetAsync(c.u1, 0, b, st));
-        CK(cudaMemsetAsync(c.u2, 0, b, st));
+        if (!u0) {
+            CK(cudaMemsetAsync(c.u1, 0, b, st));
+            CK(cudaMemsetAsync(c.u2, 0, b, st));
+        }
         if (P.gamma != 0.0) CK(cudaMemsetAsync(H->u3[L - 1], 0, b, st));
     }
     CK(cudaEventRecord(ev_pyr, st));
@@ -1071,6 +1126,8 @@ void tvl1_destroy(tvl1_handle* H)
     if (H->d_f1) cudaFree(H->d_f1);
     if (H->d_uo) cudaFree(H->d_uo);
     if (H->d_vo) cudaFree(H->d_vo);
+    if (H->d_ui) cudaFree(H->d_ui);
+    if (H->d_vi) cudaFree(H->d_vi);
     tvl1::sampler_release(H->samp);
     tvl1::features_release(H->feat);
     for (int i = 0; i < TVL1_STACK_SLOTS; i++) { if (H->st_slice[i]) cudaFree(H->st_slice[i]); if (H->st_up[i]) cudaEventDestroy(H->st_up[i]); }
@@ -1112,46 +1169,70 @@ int tvl1_set_timing(tvl1_handle* H, int enabled)
     return TVL1_OK;
 }
 
+int tvl1_calc_ex(tvl1_handle* H, int frame_type, const void* d_frame0, size_t pitch0, const void* d_frame1,
+                 size_t pitch1, int width, int height, const float* d_u0, const float* d_v0, size_t pitch_init,
+                 float* d_u, float* d_v, size_t pitch_out, void* stream, tvl1_stats* stats)
+{
+    if (!H) return fail(TVL1_ERR_INVALID, "handle is null");
+    return calc_device(H, frame_type, d_frame0, pitch0, d_frame1, pitch1, width, height, d_u0, d_v0, pitch_init, d_u, d_v,
+                       pitch_out, (cudaStream_t)stream, stats);
+}
+
 int tvl1_calc_u8(tvl1_handle* H, const uint8_t* d_frame0, size_t pitch0, const uint8_t* d_frame1, size_t pitch1,
                  int width, int height, float* d_u, float* d_v, size_t pitch_out, void* stream, tvl1_stats* stats)
 {
-    if (!H) return fail(TVL1_ERR_INVALID, "handle is null");
-    return calc_device(H, d_frame0, pitch0, d_frame1, pitch1, width, height, d_u, d_v, pitch_out,
-                       (cudaStream_t)stream, stats);
+    return tvl1_calc_ex(H, TVL1_FRAME_U8, d_frame0, pitch0, d_frame1, pitch1, width, height, nullptr, nullptr, 0, d_u, d_v,
+                        pitch_out, stream, stats);
 }
 
-int tvl1_calc_u8_host(tvl1_handle* H, const uint8_t* h_frame0, size_t pitch0, const uint8_t* h_frame1, size_t pitch1,
-                      int width, int height, float* h_u, float* h_v, size_t pitch_out, tvl1_stats* stats)
+int tvl1_calc_ex_host(tvl1_handle* H, int frame_type, const void* h_frame0, size_t pitch0, const void* h_frame1,
+                      size_t pitch1, int width, int height, const float* h_u0, const float* h_v0, size_t pitch_init,
+                      float* h_u, float* h_v, size_t pitch_out, tvl1_stats* stats)
 {
     if (!H) return fail(TVL1_ERR_INVALID, "handle is null");
     if (!h_frame0 || !h_frame1 || !h_u || !h_v) return fail(TVL1_ERR_INVALID, "null image or flow pointer");
-    if (width <= 0 || height <= 0) return fail(TVL1_ERR_INVALID, "empty image (%dx%d)", width, height);
-    if (pitch0 < (size_t)width || pitch1 < (size_t)width || pitch_out < (size_t)width * 4)
-        return fail(TVL1_ERR_INVALID, "pitch smaller than a row");
+    int rc = check_frames(frame_type, pitch0, pitch1, width, height, h_u0, h_v0, pitch_init, pitch_out);
+    if (rc) return rc;
     CK(cudaSetDevice(H->device));
-    if (H->stage_w != width || H->stage_h != height) {
-        if (H->d_f0) cudaFree(H->d_f0);
-        if (H->d_f1) cudaFree(H->d_f1);
-        if (H->d_uo) cudaFree(H->d_uo);
-        if (H->d_vo) cudaFree(H->d_vo);
-        H->d_f0 = H->d_f1 = nullptr; H->d_uo = H->d_vo = nullptr; H->stage_w = H->stage_h = 0;
-        H->stage_pitch8 = (size_t)round_up(width, 128);
-        CK(cudaMalloc(&H->d_f0, H->stage_pitch8 * height));
-        CK(cudaMalloc(&H->d_f1, H->stage_pitch8 * height));
-        CK(cudaMalloc(&H->d_uo, (size_t)width * height * 4));
-        CK(cudaMalloc(&H->d_vo, (size_t)width * height * 4));
+    const size_t row = (size_t)width * (frame_type == TVL1_FRAME_F32 ? 4 : 1);
+    const size_t plane = (size_t)width * height * 4;
+    if (H->stage_w != width || H->stage_h != height || H->stage_pitch < row) {
+        void** bufs[6] = {&H->d_f0, &H->d_f1, (void**)&H->d_uo, (void**)&H->d_vo, (void**)&H->d_ui, (void**)&H->d_vi};
+        for (void** b : bufs) { if (*b) cudaFree(*b); *b = nullptr; }
+        H->stage_w = H->stage_h = 0;
+        H->stage_pitch = (size_t)round_up((int)row, 128);
+        CK(cudaMalloc(&H->d_f0, H->stage_pitch * height));
+        CK(cudaMalloc(&H->d_f1, H->stage_pitch * height));
+        CK(cudaMalloc(&H->d_uo, plane));
+        CK(cudaMalloc(&H->d_vo, plane));
         H->stage_w = width; H->stage_h = height;
     }
+    if (h_u0 && !H->d_ui) {
+        CK(cudaMalloc(&H->d_ui, plane));
+        CK(cudaMalloc(&H->d_vi, plane));
+    }
     cudaStream_t st = H->own_stream;
-    CK(cudaMemcpy2DAsync(H->d_f0, H->stage_pitch8, h_frame0, pitch0, width, height, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpy2DAsync(H->d_f1, H->stage_pitch8, h_frame1, pitch1, width, height, cudaMemcpyHostToDevice, st));
-    int rc = calc_device(H, H->d_f0, H->stage_pitch8, H->d_f1, H->stage_pitch8, width, height, H->d_uo, H->d_vo,
-                         (size_t)width * 4, st, stats);
+    CK(cudaMemcpy2DAsync(H->d_f0, H->stage_pitch, h_frame0, pitch0, row, height, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpy2DAsync(H->d_f1, H->stage_pitch, h_frame1, pitch1, row, height, cudaMemcpyHostToDevice, st));
+    if (h_u0) {
+        CK(cudaMemcpy2DAsync(H->d_ui, (size_t)width * 4, h_u0, pitch_init, (size_t)width * 4, height, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpy2DAsync(H->d_vi, (size_t)width * 4, h_v0, pitch_init, (size_t)width * 4, height, cudaMemcpyHostToDevice, st));
+    }
+    rc = calc_device(H, frame_type, H->d_f0, H->stage_pitch, H->d_f1, H->stage_pitch, width, height,
+                     h_u0 ? H->d_ui : nullptr, h_u0 ? H->d_vi : nullptr, (size_t)width * 4, H->d_uo, H->d_vo,
+                     (size_t)width * 4, st, stats);
     if (rc) return rc;
     CK(cudaMemcpy2DAsync(h_u, pitch_out, H->d_uo, (size_t)width * 4, (size_t)width * 4, height, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpy2DAsync(h_v, pitch_out, H->d_vo, (size_t)width * 4, (size_t)width * 4, height, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return TVL1_OK;
+}
+
+int tvl1_calc_u8_host(tvl1_handle* H, const uint8_t* h_frame0, size_t pitch0, const uint8_t* h_frame1, size_t pitch1,
+                      int width, int height, float* h_u, float* h_v, size_t pitch_out, tvl1_stats* stats)
+{
+    return tvl1_calc_ex_host(H, TVL1_FRAME_U8, h_frame0, pitch0, h_frame1, pitch1, width, height, nullptr, nullptr, 0,
+                             h_u, h_v, pitch_out, stats);
 }
 
 static int launch_mask_flow(const uint8_t* f1, size_t pitch1, int w, int h, float* u, float* v, size_t pitch_f, int add_grid,
@@ -1304,8 +1385,8 @@ int tvl1_stack_run(tvl1_handle* H, const tvl1_stack_io* io, float* ms_total)
         if (k >= 2 && io->h_u) CK(cudaStreamWaitEvent(cs, H->st_down[fb], 0));   // flow buffer still draining
         float* du = H->st_flow[fb][0];
         float* dv = H->st_flow[fb][1];
-        rc = calc_device(H, H->st_slice[s0], p8, H->st_slice[s1], p8, w, h, du, dv, (size_t)w * 4, cs,
-                         io->stats ? &io->stats[k] : nullptr);
+        rc = calc_device(H, TVL1_FRAME_U8, H->st_slice[s0], p8, H->st_slice[s1], p8, w, h, nullptr, nullptr, 0, du, dv,
+                         (size_t)w * 4, cs, io->stats ? &io->stats[k] : nullptr);
         if (rc) return rc;
         if (io->apply_mask && (rc = launch_mask_flow(H->st_slice[s1], p8, w, h, du, dv, (size_t)w, 0, cs))) return rc;
         if (io->npoints >= 0) {
@@ -1362,6 +1443,13 @@ int tvl1_k_convert_u8(const uint8_t* d_src, size_t pitch_bytes, int w, int h, fl
     if (!d_src || !d_dst || w <= 0 || h <= 0 || pitch % 4 || pitch < w || pitch_bytes < (size_t)w)
         return fail(TVL1_ERR_INVALID, "bad argument");
     return launch_convert(d_src, pitch_bytes, w, h, d_dst, pitch, (cudaStream_t)stream);
+}
+
+int tvl1_k_convert_f32(const float* d_src, size_t pitch_bytes, int w, int h, float* d_dst, int pitch, void* stream)
+{
+    if (!d_src || !d_dst || w <= 0 || h <= 0 || pitch % 4 || pitch < w || pitch_bytes % 4 || pitch_bytes < (size_t)w * 4)
+        return fail(TVL1_ERR_INVALID, "bad argument");
+    return launch_convert_f32(d_src, pitch_bytes, w, h, d_dst, pitch, (cudaStream_t)stream);
 }
 
 int tvl1_k_resize(const float* d_src, int sw, int sh, int spitch, float* d_dst, int dw, int dh, int dpitch,

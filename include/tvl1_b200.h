@@ -10,6 +10,8 @@
  *                                          solve in TVL1_solve   src/optflow.cpp:518
  *   tvl1_calc_u8 / tvl1_calc_u8_host    <- TVL1_solve (solver->calc)
  *                                          src/optflow.h:31, src/optflow.cpp:516-520
+ *   tvl1_calc_ex / tvl1_calc_ex_host    <- the rest of the classes' calc(I0, I1, flow): CV_32FC1 frames and
+ *                                          useInitialFlow (the reference uses neither)
  *   tvl1_mask_flow_u8                   <- threshold + setTo in solve_wrapper
  *                                          src/optflow.cpp:471-473
  *   tvl1_sample_matches[_host]          <- mask build src/optflow.cpp:488-493 and
@@ -65,6 +67,9 @@ extern "C" {
 #define TVL1_SEMANTICS_CPU 0    /* tvl1_params.semantics: cv::DualTVL1OpticalFlow (default) */
 #define TVL1_SEMANTICS_CUDA 1   /* cv::cuda::OpticalFlowDual_TVL1's algorithm, see NUMERICS above */
 
+#define TVL1_FRAME_U8 0         /* tvl1_calc_ex frame_type: CV_8UC1 rows */
+#define TVL1_FRAME_F32 1        /* CV_32FC1 rows, scaled by 255 as the classes' convertTo does */
+
 #define TVL1_MAX_LEVELS 32
 #define TVL1_MAX_WARPS 64
 
@@ -87,7 +92,8 @@ typedef struct tvl1_params {
     int outer_iterations;   /* <= 0: derive from iterations */
     int median_filtering;   /* 5 (CPU class); 3; 1 = off */
     int use_initial_flow;   /* read by the reference but never forwarded
-                               (src/optflow.cpp:512,518); must be 0 */
+                               (src/optflow.cpp:512,518); must be 0 (TVL1_ERR_UNSUPPORTED).  An initial
+                               flow is an ARGUMENT of tvl1_calc_ex, not a handle parameter */
     int semantics;          /* TVL1_SEMANTICS_CPU (0, default) or TVL1_SEMANTICS_CUDA (1).  CUDA: `iterations`
                                is the flat count per (level, warp); inner/outer iterations must be <= 0
                                (TVL1_ERR_INVALID), gamma must be 0 (TVL1_ERR_UNSUPPORTED), median_filtering
@@ -141,6 +147,24 @@ int tvl1_calc_u8(tvl1_handle* h, const uint8_t* d_frame0, size_t pitch0,
 /* Same with host buffers: H2D of both frames, solve, D2H of both planes. */
 int tvl1_calc_u8_host(tvl1_handle* h, const uint8_t* h_frame0, size_t pitch0,
                       const uint8_t* h_frame1, size_t pitch1, int width, int height,
+                      float* h_u, float* h_v, size_t pitch_out, tvl1_stats* stats);
+
+/* cv::DualTVL1OpticalFlow::calc / cv::cuda::OpticalFlowDual_TVL1::calc with useInitialFlow, in the handle's semantics.
+ * frame_type TVL1_FRAME_U8: 8-bit rows, as tvl1_calc_u8.  TVL1_FRAME_F32: fp32 rows whose byte pitch is a multiple
+ * of 4 and at least 4 * width; level 0 of the pyramid is x * 255.0f (convertTo(CV_32F, 255.0), exactly).
+ * d_u0 and d_v0 NULL: the solve starts from zero flow (tvl1_calc_u8 is this call with TVL1_FRAME_U8).  Both given:
+ * it starts from that flow (planar fp32, byte pitch pitch_init, a multiple of 4): level 0 is the flow, each coarser
+ * level the image pyramid's resize of the finer one times scaleStep (SURVEY.md A.2a / Appendix B); the values are
+ * not validated, as OpenCV does not validate them.  Only one of them given: TVL1_ERR_INVALID.  d_u0 == d_u and
+ * d_v0 == d_v are allowed (OpenCV's flow is in/out). */
+int tvl1_calc_ex(tvl1_handle* h, int frame_type,
+                 const void* d_frame0, size_t pitch0, const void* d_frame1, size_t pitch1, int width, int height,
+                 const float* d_u0, const float* d_v0, size_t pitch_init,
+                 float* d_u, float* d_v, size_t pitch_out, void* stream, tvl1_stats* stats);
+/* Same with host buffers: frames and initial flow are staged in device buffers the handle keeps. */
+int tvl1_calc_ex_host(tvl1_handle* h, int frame_type,
+                      const void* h_frame0, size_t pitch0, const void* h_frame1, size_t pitch1, int width, int height,
+                      const float* h_u0, const float* h_v0, size_t pitch_init,
                       float* h_u, float* h_v, size_t pitch_out, tvl1_stats* stats);
 
 /* flow = 0 where frame1 <= 1 (src/optflow.cpp:471-473). */
@@ -283,6 +307,8 @@ int tvl1_prescale_u8_host(int device, const uint8_t* src, size_t spitch, int w, 
  * Planes are fp32 with a pitch in ELEMENTS; pointers are device memory. ---- */
 int tvl1_k_convert_u8(const uint8_t* d_src, size_t pitch_bytes, int w, int h, float* d_dst,
                       int pitch, void* stream);
+/* fp32 frame -> level 0 (x * 255.0f); pitch_bytes a multiple of 4, >= 4 * w; pad columns of d_dst get 0 */
+int tvl1_k_convert_f32(const float* d_src, size_t pitch_bytes, int w, int h, float* d_dst, int pitch, void* stream);
 int tvl1_k_resize(const float* d_src, int sw, int sh, int spitch, float* d_dst, int dw, int dh,
                   int dpitch, double inv_scale /* <= 0: explicit size */, float mul, void* stream);
 int tvl1_k_centered_gradient(const float* d_src, int w, int h, int pitch, float* d_dx,
