@@ -621,14 +621,47 @@ def k_centered_gradient(src, device=0):
     return dx.get(), dy.get()
 
 
-def k_warp(I0, I1, u1, u2, device=0):
-    """Returns I1w, I1wx, I1wy, grad, rho_c (the centred gradients of I1 are formed in-kernel)."""
+POISON_ROWS = 3   # rows past h that a poisoned stage call allocates, NaN-filled, in every plane
+
+
+def _stage_bufs(arrays, h, w, pitch, poison, n_out, device):
+    """Device planes of `pitch` elements for a stage-level call: the inputs `arrays` (h x w each) and n_out
+    outputs.  poison=False: zero padding, zeroed outputs, exactly h rows.  poison=True: the pad columns and
+    POISON_ROWS extra rows of every input hold NaN, and the outputs are NaN everywhere -- a kernel that reads
+    padding or misses a store shows up in what it returns."""
+    rows = h + (POISON_ROWS if poison else 0)
+    fill = np.nan if poison else 0.0
+    ins = []
+    for a in arrays:
+        x = np.full((rows, pitch), fill, np.float32)
+        x[:h, :w] = a
+        ins.append(DevBuf(x.nbytes, device).upload(x))
+    outs = [DevBuf(rows * pitch * 4, device).upload(np.full((rows, pitch), fill, np.float32)) for _ in range(n_out)]
+    return ins, outs, rows
+
+
+def _stage_result(bufs, h, w, pitch, rows, full):
+    """Downloads and frees `bufs`: the whole (rows, pitch) buffers when full, else their h x w images"""
+    res = []
+    for b in bufs:
+        a = b.download((rows, pitch), np.float32)
+        res.append(a if full else a[:h, :w].copy())
+        b.free()
+    return tuple(res)
+
+
+def k_warp(I0, I1, u1, u2, device=0, pitch=None, poison=False, full=False):
+    """Returns I1w, I1wx, I1wy, grad, rho_c (the centred gradients of I1 are formed in-kernel).  pitch: of all
+    device planes, in elements (default: the width rounded up to 32); poison / full: see _stage_bufs /
+    _stage_result."""
     h, w = np.asarray(I0).shape
-    ins = [Plane(h, w, device, np.asarray(a, np.float32)) for a in (I0, I1, u1, u2)]
-    outs = [Plane(h, w, device) for _ in range(5)]
-    check(lib().tvl1_k_warp(*[p.ptr for p in ins], w, h, ins[0].pitch, *[p.ptr for p in outs], None))
+    p = int(pitch or pitch_of(w))
+    ins, outs, rows = _stage_bufs([np.asarray(a, np.float32) for a in (I0, I1, u1, u2)], h, w, p, poison, 5, device)
+    check(lib().tvl1_k_warp(*[b.ptr for b in ins], w, h, p, *[o.ptr for o in outs], None))
     check(lib().tvl1_dev_sync(device))
-    return tuple(p.get() for p in outs)
+    for b in ins:
+        b.free()
+    return _stage_result(outs, h, w, p, rows, full)
 
 
 def k_resize_cuda(src, dw=None, dh=None, inv_scale=0.0, mul=1.0, device=0, spitch=None, dpitch=None):
@@ -651,37 +684,36 @@ def k_resize_cuda(src, dw=None, dh=None, inv_scale=0.0, mul=1.0, device=0, spitc
     return out
 
 
-def k_warp_cuda(I0, I1, u1, u2, device=0, pitch=None):
+def k_warp_cuda(I0, I1, u1, u2, device=0, pitch=None, poison=False, full=False):
     """warpBackward of TVL1_SEMANTICS_CUDA (tvl1_k_warp_cuda): returns I1w, I1wx, I1wy, grad, rho_c.  pitch: of
-    all device planes, in elements (default: the width rounded up to 32)."""
+    all device planes, in elements (default: the width rounded up to 32); poison / full: see _stage_bufs /
+    _stage_result."""
     h, w = np.asarray(I0).shape
     p = int(pitch or pitch_of(w))
-    bufs = []
-    for a in (I0, I1, u1, u2):
-        x = np.zeros((h, p), np.float32)
-        x[:, :w] = a
-        bufs.append(DevBuf(x.nbytes, device).upload(x))
-    outs = [DevBuf(h * p * 4, device).zero() for _ in range(5)]
-    check(lib().tvl1_k_warp_cuda(*[b.ptr for b in bufs], w, h, p, *[o.ptr for o in outs], None))
+    ins, outs, rows = _stage_bufs([np.asarray(a, np.float32) for a in (I0, I1, u1, u2)], h, w, p, poison, 5, device)
+    check(lib().tvl1_k_warp_cuda(*[b.ptr for b in ins], w, h, p, *[o.ptr for o in outs], None))
     check(lib().tvl1_dev_sync(device))
-    res = tuple(o.download((h, p), np.float32)[:, :w].copy() for o in outs)
-    for b in bufs + outs:
+    for b in ins:
         b.free()
-    return res
+    return _stage_result(outs, h, w, p, rows, full)
 
 
 def k_iterate(I1wx, I1wy, grad, rho_c, u1, u2, p11, p12, p21, p22, l_t, theta, taut, n=1, device=0,
-              fused=False):
+              fused=False, pitch=None, poison=False, full=False):
     """n iterations; returns (u1,u2,p11,p12,p21,p22, errors[n]).  fused: two per launch;
-    fused="outer": all n in one cooperative k_outer launch (the shipped schedule)."""
+    fused="outer": all n in one cooperative k_outer launch (the shipped schedule).  pitch: of all device planes,
+    in elements (default: the width rounded up to 32); poison / full: see _stage_bufs / _stage_result (the state
+    planes are updated in place, so poison NaN-fills their padding like the other inputs')."""
     h, w = np.asarray(u1).shape
-    consts = [Plane(h, w, device, np.asarray(a, np.float32)) for a in (I1wx, I1wy, grad, rho_c)]
-    state = [Plane(h, w, device, np.asarray(a, np.float32)) for a in (u1, u2, p11, p12, p21, p22)]
+    p = int(pitch or pitch_of(w))
+    arrays = [np.asarray(a, np.float32) for a in (I1wx, I1wy, grad, rho_c, u1, u2, p11, p12, p21, p22)]
+    bufs, _, rows = _stage_bufs(arrays, h, w, p, poison, 0, device)
     errs = np.zeros(max(n, 1), np.float64)
     fn = lib().tvl1_k_outer if fused == "outer" else (lib().tvl1_k_iterate_fused2 if fused else lib().tvl1_k_iterate)
-    check(fn(*[p.ptr for p in consts], *[p.ptr for p in state], w, h,
-             state[0].pitch, l_t, theta, taut, n, errs.ctypes.data, None))
-    return tuple(p.get() for p in state) + (errs[:n],)
+    check(fn(*[b.ptr for b in bufs], w, h, p, l_t, theta, taut, n, errs.ctypes.data, None))
+    for b in bufs[:4]:
+        b.free()
+    return _stage_result(bufs[4:], h, w, p, rows, full) + (errs[:n],)
 
 
 def k_iterate_gamma(I1wx, I1wy, rho_c, u1, u2, u3, p11, p12, p21, p22, p31, p32, l_t, theta, taut, gamma, n=1, device=0):
@@ -827,21 +859,24 @@ def k_knn2(q, t, device=0):
     return res
 
 
-def k_median3(src, device=0):
+def _median(fn, src, device, pitch, poison, full):
     src = np.asarray(src, np.float32)
     h, w = src.shape
-    s = Plane(h, w, device, src)
-    d = Plane(h, w, device)
-    check(lib().tvl1_k_median3(s.ptr, w, h, s.pitch, d.ptr, None))
+    p = int(pitch or pitch_of(w))
+    ins, outs, rows = _stage_bufs([src], h, w, p, poison, 1, device)
+    check(fn(ins[0].ptr, w, h, p, outs[0].ptr, None))
     check(lib().tvl1_dev_sync(device))
-    return d.get()
+    ins[0].free()
+    return _stage_result(outs, h, w, p, rows, full)[0]
 
 
-def k_median5(src, device=0):
-    src = np.asarray(src, np.float32)
-    h, w = src.shape
-    s = Plane(h, w, device, src)
-    d = Plane(h, w, device)
-    check(lib().tvl1_k_median5(s.ptr, w, h, s.pitch, d.ptr, None))
-    check(lib().tvl1_dev_sync(device))
-    return d.get()
+def k_median3(src, device=0, pitch=None, poison=False, full=False):
+    """medianBlur(src, 3) (tvl1_k_median3).  pitch: in elements (default: the width rounded up to 32); poison /
+    full: see _stage_bufs / _stage_result."""
+    return _median(lib().tvl1_k_median3, src, device, pitch, poison, full)
+
+
+def k_median5(src, device=0, pitch=None, poison=False, full=False):
+    """medianBlur(src, 5) (tvl1_k_median5).  pitch: in elements (default: the width rounded up to 32); poison /
+    full: see _stage_bufs / _stage_result."""
+    return _median(lib().tvl1_k_median5, src, device, pitch, poison, full)

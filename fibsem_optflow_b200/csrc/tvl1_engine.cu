@@ -1573,13 +1573,15 @@ static int k_iterate_impl(int fused, const float* d_I1wx, const float* d_I1wy, c
     } else if (fused) { for (int i = 0; i + 1 < n && !rc; i += 2) rc = launch_iterate2(a, st); }
     else { for (int i = 0; i < n && !rc; i++) rc = launch_iterate(a, st); }
     stage_end(st);
-    // passes made = buffer flips: n single passes, n/2 fused ones, n/2 + n%2 inside k_outer
+    // passes made = buffer flips: n single passes, n/2 fused ones, n/2 + n%2 inside k_outer.  The copy back
+    // covers the kernels' write width (w rounded up to 4), so the caller's padding beyond it stays untouched
     const int flips = fused == 2 ? n / 2 + (n & 1) : (fused ? n / 2 : n);
     if (!rc && (fused || (flips & 1))) {
         const int t = flips & 1;
         float* const src[6] = {a.u1[t], a.u2[t], a.p11[t], a.p12[t], a.p21[t], a.p22[t]};
+        const size_t row = (size_t)pitch * sizeof(float), cols = (size_t)((w + 3) & ~3) * sizeof(float);
         for (int k = 0; k < 6 && !rc; k++)
-            if (cudaMemcpyAsync(user[k], src[k], pb, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+            if (cudaMemcpy2DAsync(user[k], row, src[k], row, cols, h, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
                 rc = fail(TVL1_ERR_CUDA, "copy back failed");
     }
     if (!rc && errors && n > 0 &&

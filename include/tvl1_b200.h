@@ -314,13 +314,15 @@ int tvl1_k_resize(const float* d_src, int sw, int sh, int spitch, float* d_dst, 
 int tvl1_k_centered_gradient(const float* d_src, int w, int h, int pitch, float* d_dx,
                              float* d_dy, void* stream);
 /* warp step; I1's centred gradients are formed inside (A.3 fused into A.4).  d_I1w and d_grad
- * may be NULL. */
+ * may be NULL.  pitch (elements, all planes): a multiple of 4, >= w.  Reads and writes only x < w, y < h:
+ * the pad columns and any rows past h of the outputs are left as they were. */
 int tvl1_k_warp(const float* d_I0, const float* d_I1, const float* d_u1, const float* d_u2,
                 int w, int h, int pitch, float* d_I1w, float* d_I1wx, float* d_I1wy,
                 float* d_grad, float* d_rho_c, void* stream);
 /* TVL1_SEMANTICS_CUDA's stages: cuda::resize(INTER_LINEAR) (inv_scale > 0: by that factor, else to dw x dh;
  * then times mul) and warpBackward + calcGradRho (I1's centred gradients formed inside, clamped reads).  Same
- * arguments as tvl1_k_resize / tvl1_k_warp. */
+ * arguments as tvl1_k_resize / tvl1_k_warp, except that tvl1_k_warp_cuda takes any pitch >= w; like
+ * tvl1_k_warp it reads and writes only x < w, y < h. */
 int tvl1_k_resize_cuda(const float* d_src, int sw, int sh, int spitch, float* d_dst, int dw, int dh,
                        int dpitch, double inv_scale, float mul, void* stream);
 int tvl1_k_warp_cuda(const float* d_I0, const float* d_I1, const float* d_u1, const float* d_u2,
@@ -328,7 +330,9 @@ int tvl1_k_warp_cuda(const float* d_I0, const float* d_I1, const float* d_u1, co
                      float* d_grad, float* d_rho_c, void* stream);
 /* n inner iterations with no stop test; state planes are updated in place (the result
  * is copied back if it ends in the internal twin buffers).  errors (host, may be NULL)
- * receives the n per-iteration error sums. */
+ * receives the n per-iteration error sums.  pitch: a multiple of 4, >= w.  The state planes are
+ * written up to x < w rounded up to 4 (what lands in the pad columns below that is unspecified), never
+ * beyond it nor past row h; the same holds for tvl1_k_iterate_fused2 and tvl1_k_outer. */
 int tvl1_k_iterate(const float* d_I1wx, const float* d_I1wy, const float* d_grad,
                    const float* d_rho_c, float* d_u1, float* d_u2, float* d_p11, float* d_p12,
                    float* d_p21, float* d_p22, int w, int h, int pitch,
@@ -350,8 +354,12 @@ int tvl1_k_outer(const float* d_I1wx, const float* d_I1wy, const float* d_grad,
                  const float* d_rho_c, float* d_u1, float* d_u2, float* d_p11, float* d_p12,
                  float* d_p21, float* d_p22, int w, int h, int pitch,
                  float l_t, float theta, float taut, int n, double* errors, void* stream);
+/* medianBlur(src, 5), replicate border.  pitch: a multiple of 4, >= w.  d_dst is written up to x < w rounded
+ * up to 4 (4 outputs per store: the pad columns below that get unspecified values), never beyond it nor past
+ * row h. */
 int tvl1_k_median5(const float* d_src, int w, int h, int pitch, float* d_dst, void* stream);
-/* medianBlur(src, 3): the other fp32 aperture (medianFiltering = 3) */
+/* medianBlur(src, 3): the other fp32 aperture (medianFiltering = 3).  pitch: a multiple of 4, >= w; writes
+ * only x < w, y < h. */
 int tvl1_k_median3(const float* d_src, int w, int h, int pitch, float* d_dst, void* stream);
 /* The feature pre-alignment's kernels (8-bit images, pitches in BYTES; the score plane's in elements).
  * Candidates are {float harris; uint16_t x, y} (8 bytes), keypoints {float x, y, angle; int level}
