@@ -9,7 +9,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-SO_PATH = os.environ.get("TVL1_SO") or os.path.join(_HERE, "csrc", "libtvl1_b200.so")   # TVL1_SO: developer builds
+SO_PATH = os.path.join(_HERE, "csrc", "libtvl1_b200.so")
 
 MAX_LEVELS = 32
 MAX_WARPS = 64
@@ -111,13 +111,6 @@ def lib():
             "%s is missing: build it with `python fibsem_optflow_b200/csrc/build.py` "
             "(there is no CPU fallback)" % SO_PATH)
     L = C.CDLL(SO_PATH)
-    if os.environ.get("TVL1_SO"):
-        # developer A/B builds may predate newer entry points: give them inert placeholders
-        class _Missing:
-            argtypes = restype = None
-        for name in EXPORTS:
-            if not hasattr(L, name):
-                setattr(L, name, _Missing())
     L.tvl1_version.restype = C.c_char_p
     L.tvl1_last_error.restype = C.c_char_p
     L.tvl1_default_params.argtypes = [C.POINTER(Params)]

@@ -32,8 +32,7 @@ def stale():
 def build(force=False, verbose=False):
     if not force and not stale():
         return SO
-    extra = os.environ.get("TVL1_EXTRA_FLAGS", "").split()   # developer experiments only
-    cmd = [NVCC] + FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", SO] + [os.path.join(HERE, s) for s in SOURCES]
+    cmd = [NVCC] + FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", SO] + [os.path.join(HERE, s) for s in SOURCES]
     subprocess.check_call(cmd, cwd=HERE)
     return SO
 

@@ -283,10 +283,7 @@ int launch_warp_cuda(const WarpArgs& a, cudaStream_t st)
     return TVL1_OK;
 }
 
-#ifndef TVL1_ITER_NW
-#define TVL1_ITER_NW 4
-#endif
-static const int ITER_NW = TVL1_ITER_NW;
+static const int ITER_NW = 4;   // warps per block of the iteration kernels
 
 // resident blocks of the iteration kernels on the current device (SMs x occupancy), queried once
 // per device; the fused kernel's shared-memory ring needs the opt-in limit raised first
@@ -345,8 +342,7 @@ static int tile_rows_search(int w, int h, int strip, int halo, int rmin, int res
     double best = -1.0;
     int best_r = rmin;
     long long best_g = 1;
-    static const int rmax = getenv("TVL1_DEV_RMAX") ? atoi(getenv("TVL1_DEV_RMAX")) : 64;   // developer sweeps only
-    for (int R = rmin; R <= rmax; ++R) {
+    for (int R = rmin; R <= 64; ++R) {
         const long long ntiles = ns * cdiv(h, R);
         const long long G = ntiles < slots ? ntiles : slots;   // warps that get work
         const long long rounds = (ntiles + G - 1) / G;
@@ -354,15 +350,6 @@ static int tile_rows_search(int w, int h, int strip, int halo, int rmin, int res
         if (G < slots) eff *= (double)G / (double)slots;       // not even one tile per warp
         if (eff >= best) { best = eff; best_r = R; best_g = G; }
     }
-    static const char* dev_rows[2] = {getenv("TVL1_DEV_ROWS"), getenv("TVL1_DEV_ROWS2")};   // developer sweeps only
-    if (const char* e = dev_rows[halo == 1 ? 0 : 1]) {
-        best_r = atoi(e);
-        const long long ntiles = ns * cdiv(h, best_r);
-        best_g = ntiles < slots ? ntiles : slots;
-    }
-    static const bool verbose = getenv("TVL1_DEV_VERBOSE") != nullptr;
-    if (verbose)
-        fprintf(stderr, "tile_rows %dx%d strip %d: R=%d warps=%lld tiles=%lld\n", w, h, strip, best_r, best_g, ns * cdiv(h, best_r));
     *grid = (int)((best_g + ITER_NW - 1) / ITER_NW);
     return best_r;
 }
@@ -860,9 +847,6 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
 
     const size_t hdr = offsetof(Ctrl, iters);
     std::vector<int> counts((size_t)L * W, 0);   // iterations each (level, warp) needed
-    double* dev_errlog = nullptr;                // developer aid: per-iteration error sums to stderr
-    if (getenv("TVL1_DEV_ERRLOG")) cudaMalloc(&dev_errlog, sizeof(double) * L * W * H->inner * H->outer);
-    struct ErrlogGuard { double*& p; ~ErrlogGuard() { if (p) cudaFree(p); p = nullptr; } } errlog_guard{dev_errlog};
     for (int s = L - 1; s >= 0; --s) {
         const Level& lv = H->lv[s];
         const size_t pb = (size_t)lv.pitch * lv.h * sizeof(float);
@@ -913,7 +897,6 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
         for (int wi = 0; wi < W; ++wi) {
             const int slot = s * W + wi;
             ia.slot = slot;
-            if (dev_errlog) ia.errlog = dev_errlog + (size_t)slot * H->inner * H->outer;
             ma.slot = slot;
             // (2) warp I1 by the current flow; also re-arms the stop test (error = FLT_MAX)
             if ((rc = span_begin(1, s))) return rc;
@@ -947,7 +930,6 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
                     if (with_gamma) {
                         // the three-channel iteration: two plain launches each, no-ops once the stop flag is set
                         ga.slot = slot;
-                        ga.errlog = ia.errlog;
                         for (int k = 0; k < want; ++k)
                             if ((rc = launch_gamma_iteration(ga, st))) return rc;
                         launches += 2 * want;
@@ -993,13 +975,6 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
                 if (H->h_ctrl->done) break;
             }
             counts[slot] = done_total;
-            if (dev_errlog && done_total > 0) {
-                std::vector<double> e(done_total);
-                cudaMemcpy(e.data(), ia.errlog, sizeof(double) * done_total, cudaMemcpyDeviceToHost);
-                fprintf(stderr, "errlog L%d w%d n=%d e/eps:", s, wi, done_total);
-                for (int k = 0; k < done_total; k++) fprintf(stderr, " %.3g", e[k] / scaled_eps);
-                fprintf(stderr, "\n");
-            }
         }
         if (s == 0) break;
         // flow upsample to the next finer level (A.2): resize to its size, times 1/scaleStep

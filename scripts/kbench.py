@@ -55,8 +55,6 @@ def main():
             best = min(best, N.k_last_ms() / 40)
         dt = best * 1e-3
         print(f"k_iterate {n}^2: {dt*1e6:.1f} us/iter  {64*px/dt/1e9:.0f} GB/s (64 B/px model)")
-        if not callable(getattr(L, "tvl1_k_iterate_fused2", None)):
-            return
         best = 1e9
         for _ in range(3):
             N.check(L.tvl1_k_iterate_fused2(outs[0].ptr, outs[1].ptr, outs[0].ptr, outs[2].ptr, u1.ptr, u2.ptr, p[0].ptr, p[1].ptr,
