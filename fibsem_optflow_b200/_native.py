@@ -84,7 +84,7 @@ class StackIO(C.Structure):
 EXPORTS = [
     "tvl1_version", "tvl1_last_error", "tvl1_default_params", "tvl1_create", "tvl1_destroy",
     "tvl1_set_params", "tvl1_set_option", "tvl1_set_timing", "tvl1_calc_u8", "tvl1_calc_u8_host",
-    "tvl1_calc_ex", "tvl1_calc_ex_host",
+    "tvl1_calc_ex", "tvl1_calc_ex_host", "tvl1_calc_batch_u8", "tvl1_last_readbacks",
     "tvl1_prescaled_size", "tvl1_prescale_u8", "tvl1_prescale_u8_host",
     "tvl1_mask_flow_u8", "tvl1_finish_flow_u8", "tvl1_sample_matches", "tvl1_sample_matches_skip", "tvl1_sample_matches_ex",
     "tvl1_default_feature_params", "tvl1_find_alignment", "tvl1_warp_affine_u8", "tvl1_warp_affine_f32", "tvl1_stack_run", "tvl1_k_convert_u8", "tvl1_k_convert_f32", "tvl1_k_resize",
@@ -129,6 +129,9 @@ def lib():
                                C.POINTER(Stats)]
     L.tvl1_calc_ex_host.argtypes = [_vp, C.c_int, _vp, _sz, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, _vp, _vp, _sz,
                                     C.POINTER(Stats)]
+    L.tvl1_calc_batch_u8.argtypes = [_vp, C.c_int, _vp, _sz, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, _vp,
+                                     C.POINTER(Stats)]
+    L.tvl1_last_readbacks.argtypes = [_vp, C.POINTER(C.c_longlong)]
     L.tvl1_mask_flow_u8.argtypes = [_vp, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, _vp]
     L.tvl1_finish_flow_u8.argtypes = [_vp, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, C.c_int, _vp]
     L.tvl1_sample_matches.argtypes = [_vp, _vp, _sz, _vp, _sz, _vp, _vp, _sz, C.c_int, C.c_int,
@@ -272,6 +275,30 @@ def glibc_rand(seed, skip, n):
     return out
 
 
+def check_batch_frames(frames0, frames1):
+    """The frames of a batch as two lists of equal-size 2-D uint8 arrays (C-contiguous); raises Tvl1Error on
+    anything else, before the library is called."""
+    frames0, frames1 = list(frames0), list(frames1)   # an (n, h, w) stack is n frames
+    if not frames0 or len(frames0) != len(frames1):
+        raise Tvl1Error("a batch needs two equally long, non-empty lists of frames (%d and %d given)"
+                        % (len(frames0), len(frames1)))
+    out = []
+    for fl in (frames0, frames1):
+        arrs = []
+        for f in fl:
+            a = np.asarray(f)
+            if a.dtype != np.uint8 or a.ndim != 2:
+                raise Tvl1Error("batch frames must be 2-D uint8 arrays, not %s of shape %s" % (a.dtype, a.shape))
+            arrs.append(np.ascontiguousarray(a))
+        out.append(arrs)
+    shape = out[0][0].shape
+    if any(a.shape != shape for a in out[0] + out[1]):
+        raise Tvl1Error("the frames of a batch must all have one size")
+    if 0 in shape:
+        raise Tvl1Error("empty frames")
+    return out[0], out[1]
+
+
 class DevBuf:
     """A device allocation (tvl1_dev_alloc) with NumPy upload/download helpers."""
 
@@ -413,6 +440,49 @@ class Solver:
     def calc_device(self, d_f0, pitch0, d_f1, pitch1, w, h, d_u, d_v, pitch_out, stream=None):
         check(lib().tvl1_calc_u8(self.handle, d_f0, pitch0, d_f1, pitch1, w, h, d_u, d_v,
                                  pitch_out, stream, C.byref(self.stats)))
+
+    def calc_batch(self, frames0, frames1):
+        """n pairs of equal size in one solve (tvl1_calc_batch_u8): lists (or (n, h, w) stacks) of uint8 frames in, a
+        list of (u, v) float32 pairs out, each exactly what calc(frames0[k], frames1[k]) returns.  The per-pair stats
+        are in self.batch_stats (ms_total and launches are the batch's)."""
+        f0, f1 = check_batch_frames(frames0, frames1)
+        n = len(f0)
+        h, w = f0[0].shape
+        plane = h * w
+        frames = DevBuf(2 * n * plane, self.device)
+        flow = DevBuf(2 * n * plane * 4, self.device)
+        try:
+            frames.upload(np.stack(f0 + f1))
+            d0 = [frames.ptr + k * plane for k in range(n)]
+            d1 = [frames.ptr + (n + k) * plane for k in range(n)]
+            du = [flow.ptr + k * plane * 4 for k in range(n)]
+            dv = [flow.ptr + (n + k) * plane * 4 for k in range(n)]
+            self.calc_batch_device(d0, w, d1, w, w, h, du, dv, w * 4)
+            uv = flow.download((2, n, h, w), np.float32)
+        finally:
+            frames.free()
+            flow.free()
+        return [(uv[0, k].copy(), uv[1, k].copy()) for k in range(n)]
+
+    def calc_batch_device(self, d_f0, pitch0, d_f1, pitch1, w, h, d_u, d_v, pitch_out, stream=None):
+        """tvl1_calc_batch_u8 over lists of device pointers (pair k: d_f0[k], d_f1[k] -> d_u[k], d_v[k]); the per-pair
+        stats go to self.batch_stats"""
+        lists = [list(x) for x in (d_f0, d_f1, d_u, d_v)]
+        n = len(lists[0])
+        if n < 1 or any(len(x) != n for x in lists):
+            raise Tvl1Error("a batch needs four equally long, non-empty pointer lists (%s given)"
+                            % ", ".join(str(len(x)) for x in lists))
+        arrs = [(C.c_void_p * n)(*x) for x in lists]
+        stats = (Stats * n)()
+        check(lib().tvl1_calc_batch_u8(self.handle, n, arrs[0], pitch0, arrs[1], pitch1, w, h, arrs[2], arrs[3],
+                                       pitch_out, stream, stats))
+        self.batch_stats = list(stats)
+
+    def last_readbacks(self):
+        """host read-backs of the stop state made by the last calc on this handle"""
+        n = C.c_longlong(0)
+        check(lib().tvl1_last_readbacks(self.handle, C.byref(n)))
+        return n.value
 
     def calc_ex_device(self, frame_type, d_f0, pitch0, d_f1, pitch1, w, h, d_u0, d_v0, pitch_init, d_u, d_v,
                        pitch_out, stream=None):

@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 SO = os.path.join(HERE, "libtvl1_b200.so")
 SOURCES = ["tvl1_engine.cu", "tvl1_sampler.cu", "tvl1_features.cu"]
-DEPS = SOURCES + ["tvl1_kernels.cuh", "tvl1_internal.h", os.path.join("..", "..", "include", "tvl1_b200.h")]
+DEPS = SOURCES + ["tvl1_kernels.cuh", "tvl1_batch.cuh", "tvl1_internal.h", os.path.join("..", "..", "include", "tvl1_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -11,10 +11,12 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <algorithm>
 #include <mutex>
 #include <vector>
 
 #include "tvl1_kernels.cuh"
+#include "tvl1_batch.cuh"
 #include "tvl1_internal.h"
 
 namespace tvl1 {
@@ -515,6 +517,12 @@ struct Level {
     float *I0, *I1, *u1, *u2;   // u1/u2: buffer [0] of the twin pair; [1] is shared scratch
 };
 
+// Byte offsets of one pair's state in the batch arena (tvl1_calc_batch_u8); pair b's copy is at + b * stride
+struct BatchLayout {
+    size_t I0[TVL1_MAX_LEVELS], I1[TVL1_MAX_LEVELS], u1[TVL1_MAX_LEVELS], u2[TVL1_MAX_LEVELS];
+    size_t u1x, u2x, I1wx, I1wy, rho, p[4], part, ctrl;
+};
+
 }  // namespace tvl1
 
 using namespace tvl1;
@@ -568,6 +576,15 @@ struct tvl1_handle {
     int st_w = 0, st_h = 0;
     cudaStream_t st_in = nullptr, st_out = nullptr;
     cudaEvent_t st_up[TVL1_STACK_SLOTS] = {}, st_ready[2] = {nullptr, nullptr}, st_down[2] = {nullptr, nullptr};
+    // batch arena (tvl1_calc_batch_u8), apart from the single-pair one: bcap_n copies of a pair's state at
+    // bstride bytes, then the 2 * bcap_n frame pointers; pinned: bcap_n Ctrl read-backs, then the frame pointers
+    char* barena = nullptr;
+    char* bhost = nullptr;
+    size_t bstride = 0;
+    int bcap_n = 0, bcap_w = 0, bcap_h = 0, bcap_scales = 0;
+    double bcap_step = 0;
+    BatchLayout bl;
+    long long readbacks = 0;   // host read-backs of the stop state by the last calc
 };
 
 namespace tvl1 {
@@ -757,6 +774,31 @@ static int check_frames(int frame_type, size_t pitch0, size_t pitch1, int w, int
     return TVL1_OK;
 }
 
+// stats from a pair's final Ctrl: level sizes, iteration counts, totals and the byte model (zeroes the rest)
+static void stats_counts(tvl1_stats* stats, const Ctrl& c, int L, int W, const int* ws, const int* hs)
+{
+    memset(stats, 0, sizeof(*stats));
+    stats->levels = L;
+    stats->warps = W;
+    double bytes = 70.0 * (double)ws[0] * hs[0];
+    for (int s = 0; s < L; s++) {
+        stats->width[s] = ws[s];
+        stats->height[s] = hs[s];
+        const double px = (double)ws[s] * hs[s];
+        double per_px = 12.0;
+        for (int wi = 0; wi < W; wi++) {
+            const int n = c.iters[s * W + wi], o = c.outer[s * W + wi];
+            stats->iters[s * W + wi] = n;
+            stats->outer[s * W + wi] = o;
+            stats->total_iterations += n;
+            stats->px_iterations += (long long)px * n;
+            per_px += 40.0 + 64.0 * n + 16.0 * o;
+        }
+        bytes += px * per_px;
+    }
+    stats->algorithmic_bytes = bytes;
+}
+
 // the solve proper; everything is enqueued on `st`.  u0 / v0 (both or neither): the initial flow (useInitialFlow),
 // which may be d_u / d_v themselves
 static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pitch0, const void* f1, size_t pitch1,
@@ -780,6 +822,7 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
     const bool cs = P.semantics == TVL1_SEMANTICS_CUDA;
     long long launches = 0;
     H->ev_used = 0;
+    H->readbacks = 0;
 
     cudaEvent_t ev_begin, ev_pyr, ev_end;
     if ((rc = get_event(H, &ev_begin)) || (rc = get_event(H, &ev_pyr)) || (rc = get_event(H, &ev_end))) return rc;
@@ -967,6 +1010,7 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
                     }
                     if ((rc = copy_words(H->d_ctrl, H->h_ctrl, (int)(hdr / 4), st))) return rc;   // no copy engine: see copy_words
                     CK(cudaStreamSynchronize(st));
+                    H->readbacks++;
                     done_inner = H->h_ctrl->inner;
                     if (H->h_ctrl->done || done_inner >= H->inner) break;
                 }
@@ -1001,28 +1045,12 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
     CK(cudaEventRecord(ev_end, st));
     if ((rc = copy_words(H->d_ctrl, H->h_ctrl, (int)(sizeof(Ctrl) / 4), st))) return rc;
     CK(cudaStreamSynchronize(st));
+    H->readbacks++;
 
     if (stats) {
-        memset(stats, 0, sizeof(*stats));
-        stats->levels = L;
-        stats->warps = W;
-        double bytes = 70.0 * (double)w * h;
-        for (int s = 0; s < L; s++) {
-            stats->width[s] = H->lv[s].w;
-            stats->height[s] = H->lv[s].h;
-            const double px = (double)H->lv[s].w * H->lv[s].h;
-            double per_px = 12.0;
-            for (int wi = 0; wi < W; wi++) {
-                const int n = H->h_ctrl->iters[s * W + wi], o = H->h_ctrl->outer[s * W + wi];
-                stats->iters[s * W + wi] = n;
-                stats->outer[s * W + wi] = o;
-                stats->total_iterations += n;
-                stats->px_iterations += (long long)px * n;
-                per_px += 40.0 + 64.0 * n + 16.0 * o;
-            }
-            bytes += px * per_px;
-        }
-        stats->algorithmic_bytes = bytes;
+        int ws[TVL1_MAX_LEVELS], hs[TVL1_MAX_LEVELS];
+        for (int s = 0; s < L; s++) { ws[s] = H->lv[s].w; hs[s] = H->lv[s].h; }
+        stats_counts(stats, *H->h_ctrl, L, W, ws, hs);
         stats->launches = launches;
         float ms = 0.f;
         cudaEventElapsedTime(&ms, ev_begin, ev_end);
@@ -1037,6 +1065,273 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
                 case 2: stats->ms_median += ms; break;
                 default: stats->ms_other += ms; break;
             }
+        }
+    }
+    return TVL1_OK;
+}
+
+// ---------------------------------------------------------------- batches of equal-size pairs
+
+static void release_batch(tvl1_handle* H)
+{
+    if (H->barena) cudaFree(H->barena);
+    if (H->bhost) cudaFreeHost(H->bhost);
+    H->barena = nullptr;
+    H->bhost = nullptr;
+    H->bcap_n = H->bcap_w = H->bcap_h = 0;
+}
+
+// the batch arena for n pairs of w x h: kept while it has room for n pairs of this size and pyramid
+static int ensure_batch(tvl1_handle* H, int n, int w, int h, cudaStream_t st)
+{
+    if (H->barena && H->bcap_n >= n && H->bcap_w == w && H->bcap_h == h && H->bcap_scales == H->prm.nscales &&
+        H->bcap_step == H->prm.scale_step)
+        return TVL1_OK;
+    release_batch(H);
+    int ws[TVL1_MAX_LEVELS + 1], hs[TVL1_MAX_LEVELS + 1];
+    const int L = pyramid_sizes(w, h, H->prm.nscales, H->prm.scale_step, ws, hs);
+    BatchLayout& B = H->bl;
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    for (int s = 0; s < L; s++) {
+        const size_t b = (size_t)round_up(ws[s], 32) * hs[s] * sizeof(float);
+        B.I0[s] = carve(b); B.I1[s] = carve(b); B.u1[s] = carve(b); B.u2[s] = carve(b);
+    }
+    const size_t b0 = (size_t)round_up(w, 32) * h * sizeof(float);
+    B.u1x = carve(b0); B.u2x = carve(b0);
+    B.I1wx = carve(b0); B.I1wy = carve(b0); B.rho = carve(b0);
+    for (int k = 0; k < 4; k++) B.p[k] = carve(b0);
+    B.part = carve(TVL1_BATCH_MAX_BLOCKS * sizeof(double));
+    B.ctrl = carve(sizeof(Ctrl));
+    const size_t ptrs = ((size_t)2 * n * sizeof(void*) + 255) / 256 * 256;
+    if (off > (SIZE_MAX - ptrs) / (size_t)n)
+        return fail(TVL1_ERR_NOMEM, "a batch of %d pairs of %dx%d does not fit in the address space", n, w, h);
+    const size_t total = off * (size_t)n + ptrs;
+    cudaError_t e = cudaMalloc(&H->barena, total);
+    if (e != cudaSuccess) {
+        cudaGetLastError();   // an allocation failure is reported here, not by the next launch check
+        H->barena = nullptr;
+        return fail(TVL1_ERR_NOMEM, "cudaMalloc(%zu bytes) for a batch of %d pairs of %dx%d failed: %s", total, n, w, h,
+                    cudaGetErrorString(e));
+    }
+    e = cudaMallocHost(&H->bhost, (size_t)n * sizeof(Ctrl) + (size_t)2 * n * sizeof(void*));
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        H->bhost = nullptr;
+        release_batch(H);
+        return fail(TVL1_ERR_NOMEM, "cudaMallocHost for a batch of %d pairs failed: %s", n, cudaGetErrorString(e));
+    }
+    H->bstride = off;
+    H->bcap_n = n; H->bcap_w = w; H->bcap_h = h; H->bcap_scales = H->prm.nscales; H->bcap_step = H->prm.scale_step;
+    CK(cudaMemsetAsync(H->barena, 0, total, st));   // pad columns are read (never used): defined contents
+    return TVL1_OK;
+}
+
+// blocks per pair of a batched launch over `units` work items of `per_block` each: enough to fill the device
+// together with the other pairs, at most TVL1_BATCH_MAX_BLOCKS (the per-pair partial sums)
+static int batch_blocks(long long units, int per_block, int n)
+{
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    long long cap = ((long long)sms * 16 + n - 1) / n;
+    if (cap > TVL1_BATCH_MAX_BLOCKS) cap = TVL1_BATCH_MAX_BLOCKS;
+    const long long want = (units + per_block - 1) / per_block;
+    return (int)(want < 1 ? 1 : (want < cap ? want : cap));
+}
+
+// both planes of every pair: k_resize / k_resize_half with launch_resize2's arguments
+static int launch_bresize(BResizeArgs& a, double inv_scale, double mul, int apply_mul, int n, cudaStream_t st)
+{
+    const double inv_x = inv_scale > 0 ? inv_scale : (double)a.dw / a.sw;
+    const double inv_y = inv_scale > 0 ? inv_scale : (double)a.dh / a.sh;
+    a.scale_x = 1. / inv_x; a.scale_y = 1. / inv_y; a.mul = mul; a.apply_mul = apply_mul;
+    dim3 b(32, 8);
+    if (inv_scale == 0.5 && apply_mul != 1) k_bresize_half<<<dim3(cdiv(a.dw, 32), cdiv(a.dh, 8), 2 * n), b, 0, st>>>(a);
+    else k_bresize<<<dim3(cdiv(cdiv(a.dw, 4), 32), cdiv(a.dh, 8), 2 * n), b, 0, st>>>(a);
+    CK(cudaGetLastError());
+    return TVL1_OK;
+}
+
+// calc_device's loop in lockstep over n pairs of one size: the same (level, warp, outer iteration) for every pair,
+// each with its own stop state, so that every pair sees the kernel sequence of its own solve
+static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pitch0, const uint8_t* const* f1,
+                      size_t pitch1, int w, int h, float* const* d_u, float* const* d_v, size_t pitch_out,
+                      cudaStream_t st, tvl1_stats* stats)
+{
+    const tvl1_params& P = H->prm;
+    if (P.semantics == TVL1_SEMANTICS_CUDA)
+        return fail(TVL1_ERR_UNSUPPORTED, "tvl1_calc_batch_u8 solves in CPU-class semantics only, not cuda semantics");
+    if (P.gamma != 0.0) return fail(TVL1_ERR_UNSUPPORTED, "tvl1_calc_batch_u8 does not support gamma != 0");
+    if (n < 1 || n > TVL1_BATCH_MAX_PAIRS) return fail(TVL1_ERR_INVALID, "n must be in 1 .. %d, not %d", TVL1_BATCH_MAX_PAIRS, n);
+    if (!f0 || !f1 || !d_u || !d_v) return fail(TVL1_ERR_INVALID, "null pointer array");
+    for (int k = 0; k < n; k++)
+        if (!f0[k] || !f1[k] || !d_u[k] || !d_v[k]) return fail(TVL1_ERR_INVALID, "null image or flow pointer in entry %d", k);
+    int rc = check_frames(TVL1_FRAME_U8, pitch0, pitch1, w, h, nullptr, nullptr, 0, pitch_out);
+    if (rc) return rc;
+    if (w > 32767 || h > 32767) return fail(TVL1_ERR_INVALID, "image side > 32767 (remap uses int16 coordinates)");
+    CK(cudaSetDevice(H->device));
+    if ((rc = ensure_batch(H, n, w, h, st))) return rc;
+    if ((rc = upload_cubic_table(H->device))) return rc;
+    int ws[TVL1_MAX_LEVELS + 1], hs[TVL1_MAX_LEVELS + 1];
+    const int L = pyramid_sizes(w, h, P.nscales, P.scale_step, ws, hs), W = P.warps;
+    int pitch[TVL1_MAX_LEVELS];
+    for (int s = 0; s < L; s++) pitch[s] = round_up(ws[s], 32);
+    const float l_t = (float)(P.lambda * P.theta), taut = (float)(P.tau / P.theta), theta = (float)P.theta;
+    const BatchLayout& B = H->bl;
+    const size_t S = H->bstride;
+    char* const base = H->barena;
+    auto plane = [&](size_t o) { return (float*)(base + o); };
+    Ctrl* const ctrl = (Ctrl*)(base + B.ctrl);
+    Ctrl* const hc = (Ctrl*)H->bhost;                                          // pair b's read-back: hc[b]
+    const uint8_t** const hptr = (const uint8_t**)(H->bhost + (size_t)n * sizeof(Ctrl));
+    const uint8_t** const dptr = (const uint8_t**)(base + (size_t)H->bcap_n * S);
+    const size_t hdr = offsetof(Ctrl, iters);
+    long long launches = 0;
+    H->ev_used = 0;
+    H->readbacks = 0;
+    auto read_ctrl = [&](size_t bytes) -> int {   // every pair's first `bytes` of Ctrl -> hc[], then wait for them
+        const int words = (int)(bytes / 4);
+        const long long total = (long long)n * words;
+        k_bctrl_read<<<(unsigned)(total < 256 * 32 ? (total + 255) / 256 : 32), 256, 0, st>>>(ctrl, S, words, n, (int*)hc);
+        CK(cudaGetLastError());
+        CK(cudaStreamSynchronize(st));
+        H->readbacks++;
+        return TVL1_OK;
+    };
+
+    cudaEvent_t ev_begin, ev_end;
+    if ((rc = get_event(H, &ev_begin)) || (rc = get_event(H, &ev_end))) return rc;
+    CK(cudaEventRecord(ev_begin, st));
+    CK(cudaMemset2DAsync(ctrl, S, 0, sizeof(Ctrl), n, st));
+    // (1) pyramid of every pair
+    for (int k = 0; k < n; k++) { hptr[k] = f0[k]; hptr[n + k] = f1[k]; }
+    CK(cudaMemcpyAsync(dptr, hptr, (size_t)2 * n * sizeof(void*), cudaMemcpyHostToDevice, st));
+    k_bconvert_u8<<<dim3(cdiv(cdiv(w, 4), 32), cdiv(h, 8), 2 * n), dim3(32, 8), 0, st>>>(
+        dptr, pitch0, pitch1, w, h, plane(B.I0[0]), plane(B.I1[0]), pitch[0], S);
+    CK(cudaGetLastError());
+    launches += 1;
+    for (int s = 1; s < L; s++) {
+        BResizeArgs ra = {};
+        ra.src[0][0] = ra.src[0][1] = plane(B.I0[s - 1]);
+        ra.src[1][0] = ra.src[1][1] = plane(B.I1[s - 1]);
+        ra.dst[0] = plane(B.I0[s]); ra.dst[1] = plane(B.I1[s]);
+        ra.sw = ws[s - 1]; ra.sh = hs[s - 1]; ra.sp = pitch[s - 1]; ra.dw = ws[s]; ra.dh = hs[s]; ra.dp = pitch[s];
+        ra.stride = S;
+        if ((rc = launch_bresize(ra, P.scale_step, 1.f, 0, n, st))) return rc;
+        launches += 1;
+    }
+    {   // the coarsest level starts from zero flow
+        const size_t b = (size_t)pitch[L - 1] * hs[L - 1] * sizeof(float);
+        CK(cudaMemset2DAsync(plane(B.u1[L - 1]), S, 0, b, n, st));
+        CK(cudaMemset2DAsync(plane(B.u2[L - 1]), S, 0, b, n, st));
+    }
+
+    std::vector<int> counts((size_t)L * W, 0);   // the most iterations any pair needed per (level, warp)
+    std::vector<int> total(n);
+    for (int s = L - 1; s >= 0; --s) {
+        const int lw = ws[s], lh = hs[s];
+        BIterArgs ia;
+        ia.I1wx = plane(B.I1wx); ia.I1wy = plane(B.I1wy); ia.rho_c = plane(B.rho);
+        ia.u1[0] = plane(B.u1[s]); ia.u1[1] = plane(B.u1x); ia.u2[0] = plane(B.u2[s]); ia.u2[1] = plane(B.u2x);
+        ia.p11 = plane(B.p[0]); ia.p12 = plane(B.p[1]); ia.p21 = plane(B.p[2]); ia.p22 = plane(B.p[3]);
+        ia.w = lw; ia.h = lh; ia.pitch = pitch[s];
+        ia.l_t = l_t; ia.theta = theta; ia.taut = taut;
+        ia.scaled_eps = (float)(P.epsilon * P.epsilon * (double)(lw * lh));
+        ia.level = s; ia.inner_max = H->inner; ia.ctrl = ctrl; ia.partials = (double*)(base + B.part); ia.stride = S;
+        const dim3 gi(batch_blocks((long long)cdiv(lw, 128) * lh, TVL1_BITER_NW, n), 1, n);
+        BMedianArgs ma;
+        ma.u1[0] = ia.u1[0]; ma.u1[1] = ia.u1[1]; ma.u2[0] = ia.u2[0]; ma.u2[1] = ia.u2[1];
+        ma.ctrl = ctrl; ma.w = lw; ma.h = lh; ma.pitch = pitch[s]; ma.level = s; ma.stride = S;
+        const int per_thread = P.median_filtering == 3 ? 4 : 8;
+        const dim3 gm(batch_blocks(2LL * cdiv(lw, per_thread) * lh, 256, n), 1, n);
+        BWarpArgs wa;
+        wa.I0 = plane(B.I0[s]); wa.I1 = plane(B.I1[s]);
+        wa.u1[0] = ia.u1[0]; wa.u1[1] = ia.u1[1]; wa.u2[0] = ia.u2[0]; wa.u2[1] = ia.u2[1];
+        wa.I1wx = plane(B.I1wx); wa.I1wy = plane(B.I1wy); wa.rho_c = plane(B.rho);
+        wa.ctrl = ctrl; wa.w = lw; wa.h = lh; wa.pitch = pitch[s]; wa.level = s; wa.stride = S;
+        const dim3 gw(cdiv(lw, 32), cdiv(lh, 8), n);
+
+        for (int wi = 0; wi < W; ++wi) {
+            const int slot = s * W + wi;
+            ia.slot = slot;
+            ma.slot = slot;
+            // (2) warp; the level's first warp also zeroes p11 .. p22 and every warp re-arms the stop test
+            for (int k = 0; k < 4; k++) wa.pz[k] = wi == 0 ? plane(B.p[k]) : nullptr;
+            k_bwarp<<<gw, dim3(32, 8), 0, st>>>(wa);
+            CK(cudaGetLastError());
+            launches++;
+            // (3) outer iterations, as calc_device: chunks of iterations enqueued without knowing how many run,
+            // sized from the count the previous (level, warp) needed, one read-back of all pairs per chunk.  An
+            // outer iteration ends when every pair is done or has used its inner budget.
+            const int pred_total = wi > 0 ? counts[slot - 1] : (s < L - 1 ? counts[(s + 1) * W] : H->inner);
+            std::fill(total.begin(), total.end(), 0);
+            int least_total = 0;   // fewest iterations any pair not yet done has made in this (level, warp)
+            for (int no = 0; no < H->outer; ++no) {
+                if (P.median_filtering > 1) {
+                    if (P.median_filtering == 3) k_bmedian3<<<gm, 256, 0, st>>>(ma);
+                    else k_bmedian5<<<gm, 256, 0, st>>>(ma);
+                    CK(cudaGetLastError());
+                    launches++;
+                }
+                CK(cudaMemset2DAsync(&ctrl->inner, S, 0, sizeof(int), n, st));
+                int least_inner = 0, want = 0;   // fewest inner iterations of a pair still iterating
+                for (;;) {
+                    const int left_pred = pred_total - least_total - least_inner;
+                    want = want == 0 ? (left_pred + 1 > 4 ? left_pred + 1 : 4) : 2 * want;
+                    if (want > H->inner - least_inner) want = H->inner - least_inner;
+                    for (int k = 0; k < want; ++k) {
+                        k_biter_u<<<gi, dim3(32, TVL1_BITER_NW), 0, st>>>(ia);
+                        k_biter_p<<<gi, dim3(32, TVL1_BITER_NW), 0, st>>>(ia);
+                    }
+                    CK(cudaGetLastError());
+                    launches += 2 * want;
+                    if ((rc = read_ctrl(hdr))) return rc;
+                    least_inner = H->inner;
+                    for (int b = 0; b < n; b++)
+                        if (!hc[b].done && hc[b].inner < least_inner) least_inner = hc[b].inner;
+                    if (least_inner >= H->inner) break;
+                }
+                bool all_done = true;
+                least_total = INT32_MAX;
+                for (int b = 0; b < n; b++) {
+                    total[b] += hc[b].inner;   // 0 for a pair that was done before this outer iteration
+                    if (!hc[b].done) { all_done = false; if (total[b] < least_total) least_total = total[b]; }
+                }
+                if (all_done) break;
+            }
+            counts[slot] = *std::max_element(total.begin(), total.end());
+        }
+        if (s == 0) break;
+        // flow upsample to the next finer level, from the twin that holds each pair's flow
+        BResizeArgs ra = {};
+        ra.src[0][0] = ia.u1[0]; ra.src[0][1] = ia.u1[1]; ra.src[1][0] = ia.u2[0]; ra.src[1][1] = ia.u2[1];
+        ra.dst[0] = plane(B.u1[s - 1]); ra.dst[1] = plane(B.u2[s - 1]);
+        ra.ctrl = ctrl; ra.level = s;
+        ra.sw = lw; ra.sh = lh; ra.sp = pitch[s]; ra.dw = ws[s - 1]; ra.dh = hs[s - 1]; ra.dp = pitch[s - 1];
+        ra.stride = S;
+        if ((rc = launch_bresize(ra, 0.0, (float)(1 / P.scale_step), 1, n, st))) return rc;
+        launches += 1;
+    }
+    // A.8: planar output of every pair, from the twin its final Ctrl names
+    if ((rc = read_ctrl(sizeof(Ctrl)))) return rc;
+    for (int b = 0; b < n; b++) {
+        const size_t o = (size_t)b * S;
+        const int uc = hc[b].ucur[0];
+        CK(cudaMemcpy2DAsync(d_u[b], pitch_out, base + (uc ? B.u1x : B.u1[0]) + o, (size_t)pitch[0] * 4, (size_t)w * 4, h,
+                             cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpy2DAsync(d_v[b], pitch_out, base + (uc ? B.u2x : B.u2[0]) + o, (size_t)pitch[0] * 4, (size_t)w * 4, h,
+                             cudaMemcpyDeviceToDevice, st));
+    }
+    CK(cudaEventRecord(ev_end, st));
+    CK(cudaStreamSynchronize(st));
+    if (stats) {
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, ev_begin, ev_end);
+        for (int b = 0; b < n; b++) {
+            stats_counts(&stats[b], hc[b], L, W, ws, hs);
+            stats[b].ms_total = ms;
+            stats[b].launches = launches;
         }
     }
     return TVL1_OK;
@@ -1096,6 +1391,7 @@ void tvl1_destroy(tvl1_handle* H)
     if (!H) return;
     cudaSetDevice(H->device);
     tvl1::release_arena(H);
+    tvl1::release_batch(H);
     if (H->h_ctrl) cudaFreeHost(H->h_ctrl);
     if (H->d_f0) cudaFree(H->d_f0);
     if (H->d_f1) cudaFree(H->d_f1);
@@ -1200,6 +1496,22 @@ int tvl1_calc_ex_host(tvl1_handle* H, int frame_type, const void* h_frame0, size
     CK(cudaMemcpy2DAsync(h_u, pitch_out, H->d_uo, (size_t)width * 4, (size_t)width * 4, height, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpy2DAsync(h_v, pitch_out, H->d_vo, (size_t)width * 4, (size_t)width * 4, height, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
+    return TVL1_OK;
+}
+
+int tvl1_calc_batch_u8(tvl1_handle* H, int n, const uint8_t* const* d_frame0, size_t pitch0,
+                       const uint8_t* const* d_frame1, size_t pitch1, int width, int height,
+                       float* const* d_u, float* const* d_v, size_t pitch_out, void* stream, tvl1_stats* stats)
+{
+    if (!H) return fail(TVL1_ERR_INVALID, "handle is null");
+    return calc_batch(H, n, d_frame0, pitch0, d_frame1, pitch1, width, height, d_u, d_v, pitch_out, (cudaStream_t)stream,
+                      stats);
+}
+
+int tvl1_last_readbacks(const tvl1_handle* H, long long* n)
+{
+    if (!H || !n) return fail(TVL1_ERR_INVALID, "null handle or output");
+    *n = H->readbacks;
     return TVL1_OK;
 }
 

@@ -10,6 +10,7 @@
  *                                          solve in TVL1_solve   src/optflow.cpp:518
  *   tvl1_calc_u8 / tvl1_calc_u8_host    <- TVL1_solve (solver->calc)
  *                                          src/optflow.h:31, src/optflow.cpp:516-520
+ *   tvl1_calc_batch_u8                  <- TVL1_solve of many equal-size pairs in one call (no counterpart)
  *   tvl1_calc_ex / tvl1_calc_ex_host    <- the rest of the classes' calc(I0, I1, flow): CV_32FC1 frames and
  *                                          useInitialFlow (the reference uses neither)
  *   tvl1_mask_flow_u8                   <- threshold + setTo in solve_wrapper
@@ -143,6 +144,27 @@ int tvl1_set_timing(tvl1_handle* h, int enabled);
 int tvl1_calc_u8(tvl1_handle* h, const uint8_t* d_frame0, size_t pitch0,
                  const uint8_t* d_frame1, size_t pitch1, int width, int height,
                  float* d_u, float* d_v, size_t pitch_out, void* stream, tvl1_stats* stats);
+
+/* n pairs of equal size in one solve, in the handle's parameters: many small pairs (ROI strips) keep the GPU busy
+ * where one alone leaves it idle.  Pair k: frames d_frame0[k] / d_frame1[k] (8-bit rows, byte pitches pitch0 /
+ * pitch1, the same for every pair), flow into d_u[k] / d_v[k] (planar fp32, byte pitch pitch_out); the pointer
+ * arrays are host memory, their entries device pointers, and entries may repeat.  Every pair's flow and iteration
+ * counts are bit-identical to tvl1_calc_u8 of that pair alone.  stats: NULL or n entries (per-pair iters[] / outer[]
+ * / totals; ms_total and launches are the batch's).  Synchronises `stream`, as tvl1_calc_u8 does.
+ * CPU-class semantics only: TVL1_SEMANTICS_CUDA and gamma != 0 give TVL1_ERR_UNSUPPORTED.  n outside
+ * 1 .. TVL1_BATCH_MAX_PAIRS, a NULL entry or the pitch rules of tvl1_calc_u8: TVL1_ERR_INVALID.  A batch whose
+ * state does not fit on the device: TVL1_ERR_NOMEM, with nothing of it left allocated.  The handle keeps the
+ * batch's state apart from a single pair's; either call may follow the other. */
+#define TVL1_BATCH_MAX_PAIRS 32767
+int tvl1_calc_batch_u8(tvl1_handle* h, int n,
+                       const uint8_t* const* d_frame0, size_t pitch0,
+                       const uint8_t* const* d_frame1, size_t pitch1, int width, int height,
+                       float* const* d_u, float* const* d_v, size_t pitch_out,
+                       void* stream, tvl1_stats* stats);
+
+/* Host read-backs of the device-side stop state made by the last tvl1_calc_* call on this handle (one per chunk of
+ * enqueued iterations -- for a batch, one covers every pair -- plus the final one). */
+int tvl1_last_readbacks(const tvl1_handle* h, long long* n);
 
 /* Same with host buffers: H2D of both frames, solve, D2H of both planes. */
 int tvl1_calc_u8_host(tvl1_handle* h, const uint8_t* h_frame0, size_t pitch0,
