@@ -193,47 +193,46 @@ int launch_convert_f32(const float* src, size_t pitch_bytes, int w, int h, float
     return TVL1_OK;
 }
 
-// one or two planes (srcB / dstB may be null) resized alike in one launch; apply_mul: see scale_px
-int launch_resize2(const float* srcA, const float* srcB, int sw, int sh, int sp, float* dstA, float* dstB, int dw, int dh,
-                   int dp, double inv_scale, double mul, int apply_mul, cudaStream_t st)
+// one or two planes (srcB / dstB null: one) of one pair, the source in twin 0
+static ResizeArgs resize_args(const float* srcA, const float* srcB, int sw, int sh, int sp, float* dstA, float* dstB, int dw,
+                              int dh, int dp)
+{
+    ResizeArgs a = {};
+    a.src[0][0] = srcA; a.src[1][0] = srcB; a.dst[0] = dstA; a.dst[1] = dstB;
+    a.sw = sw; a.sh = sh; a.sp = sp; a.dw = dw; a.dh = dh; a.dp = dp;
+    return a;
+}
+
+// a's planes of n pairs (two planes each; one plane: n is 1) resized alike in one launch.  inv_scale > 0:
+// resize(src, Size(), inv_scale, inv_scale); otherwise the explicit size dw x dh.  apply_mul: see scale_px
+int launch_resize(ResizeArgs a, int n, double inv_scale, double mul, int apply_mul, cudaStream_t st)
 {
     double inv_x, inv_y;
     if (inv_scale > 0) { inv_x = inv_scale; inv_y = inv_scale; }
-    else { inv_x = (double)dw / sw; inv_y = (double)dh / sh; }
-    const double scale_x = 1. / inv_x, scale_y = 1. / inv_y;
+    else { inv_x = (double)a.dw / a.sw; inv_y = (double)a.dh / a.sh; }
+    a.scale_x = 1. / inv_x; a.scale_y = 1. / inv_y; a.mul = mul; a.apply_mul = apply_mul;
+    const unsigned nz = a.dst[1] ? 2 * n : 1;
     dim3 b(32, 8);
     // resize(src, Size(), 0.5, 0.5): OpenCV's INTER_AREA fast path.  The fp32 multiply (tvl1_k_resize with mul != 1)
     // has always taken the bilinear kernel at 0.5 and keeps doing so; the fp64 one (an initial flow's downscale) is
     // cv::resize followed by cv::multiply and so takes the area path like the image pyramid
-    if (inv_scale == 0.5 && apply_mul != 1) {
-        dim3 gh(cdiv(dw, 32), cdiv(dh, 8), srcB ? 2 : 1);
-        k_resize_half<<<gh, b, 0, st>>>(srcA, srcB, sw, sh, sp, dstA, dstB, dw, dh, dp, mul, apply_mul);
-        CK(cudaGetLastError());
-        return TVL1_OK;
-    }
-    dim3 g(cdiv(cdiv(dw, 4), 32), cdiv(dh, 8), srcB ? 2 : 1);
-    k_resize<<<g, b, 0, st>>>(srcA, srcB, sw, sh, sp, dstA, dstB, dw, dh, dp, scale_x, scale_y, mul, apply_mul);
+    if (inv_scale == 0.5 && apply_mul != 1) k_resize_half<<<dim3(cdiv(a.dw, 32), cdiv(a.dh, 8), nz), b, 0, st>>>(a);
+    else k_resize<<<dim3(cdiv(cdiv(a.dw, 4), 32), cdiv(a.dh, 8), nz), b, 0, st>>>(a);
     CK(cudaGetLastError());
     return TVL1_OK;
 }
 
-int launch_resize(const float* src, int sw, int sh, int sp, float* dst, int dw, int dh, int dp,
-                  double inv_scale, double mul, int apply_mul, cudaStream_t st)
-{
-    return launch_resize2(src, nullptr, sw, sh, sp, dst, nullptr, dw, dh, dp, inv_scale, mul, apply_mul, st);
-}
-
-// cv::cuda semantics: cuda::resize(INTER_LINEAR) of one or two planes (srcB / dstB may be null).  inv_scale > 0:
+// cv::cuda semantics: cuda::resize(INTER_LINEAR) of a's planes (one pair, twin 0).  inv_scale > 0:
 // resize(src, Size(), inv_scale, inv_scale); otherwise the explicit size dw x dh (factor dw / sw in fp64).
-int launch_resize_cuda2(const float* srcA, const float* srcB, int sw, int sh, int sp, float* dstA, float* dstB, int dw,
-                        int dh, int dp, double inv_scale, double mul, int apply_mul, cudaStream_t st)
+int launch_resize_cuda(const ResizeArgs& a, double inv_scale, double mul, int apply_mul, cudaStream_t st)
 {
-    const double f_x = inv_scale > 0 ? inv_scale : (double)dw / sw;
-    const double f_y = inv_scale > 0 ? inv_scale : (double)dh / sh;
+    const double f_x = inv_scale > 0 ? inv_scale : (double)a.dw / a.sw;
+    const double f_y = inv_scale > 0 ? inv_scale : (double)a.dh / a.sh;
     const float fx = (float)(1.0 / f_x), fy = (float)(1.0 / f_y);
     dim3 b(32, 8);
-    dim3 g(cdiv(dw, 32), cdiv(dh, 8), srcB ? 2 : 1);
-    k_resize_cuda<<<g, b, 0, st>>>(srcA, srcB, sw, sh, sp, dstA, dstB, dw, dh, dp, fx, fy, (float)mul, apply_mul);
+    dim3 g(cdiv(a.dw, 32), cdiv(a.dh, 8), a.dst[1] ? 2 : 1);
+    k_resize_cuda<<<g, b, 0, st>>>(a.src[0][0], a.src[1][0], a.sw, a.sh, a.sp, a.dst[0], a.dst[1], a.dw, a.dh, a.dp, fx, fy,
+                                   (float)mul, apply_mul);
     CK(cudaGetLastError());
     return TVL1_OK;
 }
@@ -453,8 +452,8 @@ int launch_iterate2(IterArgs& a, cudaStream_t st, bool cs = false)
     return TVL1_OK;
 }
 
-// gamma != 0: one inner iteration = estimateU launch + dual-update launch (persistent blocks over row segments)
-int launch_gamma_iteration(const GammaArgs& a, cudaStream_t st)
+// gamma != 0: one inner iteration = k_plain_u<3> + k_plain_p<3> (persistent blocks over row segments)
+int launch_gamma_iteration(const PlainIterArgs& a, cudaStream_t st)
 {
     static int cached[64] = {};
     int dev = 0;
@@ -466,11 +465,11 @@ int launch_gamma_iteration(const GammaArgs& a, cudaStream_t st)
         resident = sms * 8;
     }
     const long long ntiles = (long long)cdiv(a.w, 128) * a.h;
-    const long long want = (ntiles + ITER_NW - 1) / ITER_NW;
+    const long long want = (ntiles + TVL1_PLAIN_NW - 1) / TVL1_PLAIN_NW;
     const unsigned grid = (unsigned)(want < resident ? want : resident);
-    dim3 b(32, ITER_NW);
-    k_gamma_u<ITER_NW><<<grid, b, 0, st>>>(a);
-    k_gamma_p<ITER_NW><<<grid, b, 0, st>>>(a);
+    dim3 b(32, TVL1_PLAIN_NW);
+    k_plain_u<3><<<grid, b, 0, st>>>(a);
+    k_plain_p<3><<<grid, b, 0, st>>>(a);
     CK(cudaGetLastError());
     return TVL1_OK;
 }
@@ -482,7 +481,7 @@ int launch_median3(const MedianArgs& a, int planes, cudaStream_t st)
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const long long n = (long long)cdiv(a.w, 4) * a.h * planes;
     const long long want = (n + 255) / 256;
-    k_median3<<<(unsigned)(want < sms * 8 ? want : sms * 8), 256, 0, st>>>(a, planes);
+    k_median3<<<(unsigned)(want < sms * 8 ? want : sms * 8), 256, 0, st>>>(a, planes, 0);
     CK(cudaGetLastError());
     return TVL1_OK;
 }
@@ -855,8 +854,9 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
     launches += 2;
     for (int s = 1; s < L; s++) {
         const Level &a = H->lv[s - 1], &b = H->lv[s];
-        if ((rc = (cs ? launch_resize_cuda2 : launch_resize2)(a.I0, a.I1, a.w, a.h, a.pitch, b.I0, b.I1, b.w, b.h, b.pitch,
-                                                              P.scale_step, 1.f, 0, st))) return rc;
+        const ResizeArgs ra = resize_args(a.I0, a.I1, a.w, a.h, a.pitch, b.I0, b.I1, b.w, b.h, b.pitch);
+        if ((rc = cs ? launch_resize_cuda(ra, P.scale_step, 1.f, 0, st) : launch_resize(ra, 1, P.scale_step, 1.f, 0, st)))
+            return rc;
         launches += 1;
     }
     if (u0) {
@@ -869,10 +869,9 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
         CK(cudaMemcpy2DAsync(l0.u2, (size_t)l0.pitch * 4, v0, pitch_init, (size_t)w * 4, h, cudaMemcpyDeviceToDevice, st));
         for (int s = 1; s < L; s++) {
             const Level &a = H->lv[s - 1], &b = H->lv[s];
-            rc = cs ? launch_resize_cuda2(a.u1, a.u2, a.w, a.h, a.pitch, b.u1, b.u2, b.w, b.h, b.pitch, P.scale_step,
-                                          (float)P.scale_step, 1, st)
-                    : launch_resize2(a.u1, a.u2, a.w, a.h, a.pitch, b.u1, b.u2, b.w, b.h, b.pitch, P.scale_step,
-                                     P.scale_step, 2, st);
+            const ResizeArgs ra = resize_args(a.u1, a.u2, a.w, a.h, a.pitch, b.u1, b.u2, b.w, b.h, b.pitch);
+            rc = cs ? launch_resize_cuda(ra, P.scale_step, (float)P.scale_step, 1, st)
+                    : launch_resize(ra, 1, P.scale_step, P.scale_step, 2, st);
             if (rc) return rc;
             launches += 1;
         }
@@ -911,17 +910,17 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
         ia.eps_d = P.epsilon * P.epsilon * (double)(lv.w * lv.h);
         ia.err_on = P.epsilon > 0.0;
         const bool with_gamma = P.gamma != 0.0;
-        GammaArgs ga;
+        PlainIterArgs ga = {};
         if (with_gamma) {
             ga.I1wx = H->I1wx; ga.I1wy = H->I1wy; ga.rho_c = H->rho;
-            for (int k = 0; k < 2; k++) {
-                ga.u1[k] = ia.u1[k]; ga.u2[k] = ia.u2[k];
-                ga.p11[k] = ia.p11[k]; ga.p12[k] = ia.p12[k]; ga.p21[k] = ia.p21[k]; ga.p22[k] = ia.p22[k];
-            }
-            ga.u3 = H->u3[s]; ga.p31 = H->p31; ga.p32 = H->p32;
+            ga.u1[0] = ia.u1[0]; ga.u1[1] = ia.u1[1]; ga.u2[0] = ia.u2[0]; ga.u2[1] = ia.u2[1]; ga.u3 = H->u3[s];
+            // in place in H->p[k][0], the planes the level's first warp zeroes: only the k_iterate* / k_outer kernels
+            // flip pcur, so this solve never leaves them
+            ga.p11 = H->p[0][0]; ga.p12 = H->p[1][0]; ga.p21 = H->p[2][0]; ga.p22 = H->p[3][0];
+            ga.p31 = H->p31; ga.p32 = H->p32;
             ga.w = lv.w; ga.h = lv.h; ga.pitch = lv.pitch;
             ga.l_t = l_t; ga.theta = theta; ga.taut = taut; ga.gamma = (float)P.gamma; ga.scaled_eps = scaled_eps;
-            ga.level = s; ga.slot = 0; ga.inner_max = H->inner; ga.mode = 1;
+            ga.level = s; ga.slot = 0; ga.inner_max = H->inner;
             ga.ctrl = H->d_ctrl; ga.partials = H->d_partials; ga.errlog = nullptr;
         }
         const bool fused = (long long)lv.w * lv.h >= H->fused_min_px && H->inner >= 2;
@@ -1026,11 +1025,13 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
         const int uc = H->h_ctrl->ucur[s];
         const float mul = (float)(1 / P.scale_step);
         if ((rc = span_begin(3, s))) return rc;
-        if ((rc = (cs ? launch_resize_cuda2 : launch_resize2)(uc ? H->u1x : lv.u1, uc ? H->u2x : lv.u2, lv.w, lv.h, lv.pitch,
-                                                              up.u1, up.u2, up.w, up.h, up.pitch, 0.0, mul, 1, st))) return rc;
+        const ResizeArgs ra = resize_args(uc ? H->u1x : lv.u1, uc ? H->u2x : lv.u2, lv.w, lv.h, lv.pitch, up.u1, up.u2, up.w,
+                                          up.h, up.pitch);
+        if ((rc = cs ? launch_resize_cuda(ra, 0.0, mul, 1, st) : launch_resize(ra, 1, 0.0, mul, 1, st))) return rc;
         launches += 1;
         if (with_gamma) {   // u3 is zoomed like the flow but not scaled
-            if ((rc = launch_resize(H->u3[s], lv.w, lv.h, lv.pitch, H->u3[s - 1], up.w, up.h, up.pitch, 0.0, 1.f, 0, st))) return rc;
+            if ((rc = launch_resize(resize_args(H->u3[s], nullptr, lv.w, lv.h, lv.pitch, H->u3[s - 1], nullptr, up.w, up.h,
+                                                up.pitch), 1, 0.0, 1.f, 0, st))) return rc;
             launches += 1;
         }
         span_end();
@@ -1140,19 +1141,6 @@ static int batch_blocks(long long units, int per_block, int n)
     return (int)(want < 1 ? 1 : (want < cap ? want : cap));
 }
 
-// both planes of every pair: k_resize / k_resize_half with launch_resize2's arguments
-static int launch_bresize(BResizeArgs& a, double inv_scale, double mul, int apply_mul, int n, cudaStream_t st)
-{
-    const double inv_x = inv_scale > 0 ? inv_scale : (double)a.dw / a.sw;
-    const double inv_y = inv_scale > 0 ? inv_scale : (double)a.dh / a.sh;
-    a.scale_x = 1. / inv_x; a.scale_y = 1. / inv_y; a.mul = mul; a.apply_mul = apply_mul;
-    dim3 b(32, 8);
-    if (inv_scale == 0.5 && apply_mul != 1) k_bresize_half<<<dim3(cdiv(a.dw, 32), cdiv(a.dh, 8), 2 * n), b, 0, st>>>(a);
-    else k_bresize<<<dim3(cdiv(cdiv(a.dw, 4), 32), cdiv(a.dh, 8), 2 * n), b, 0, st>>>(a);
-    CK(cudaGetLastError());
-    return TVL1_OK;
-}
-
 // calc_device's loop in lockstep over n pairs of one size: the same (level, warp, outer iteration) for every pair,
 // each with its own stop state, so that every pair sees the kernel sequence of its own solve
 static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pitch0, const uint8_t* const* f1,
@@ -1212,13 +1200,10 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
     CK(cudaGetLastError());
     launches += 1;
     for (int s = 1; s < L; s++) {
-        BResizeArgs ra = {};
-        ra.src[0][0] = ra.src[0][1] = plane(B.I0[s - 1]);
-        ra.src[1][0] = ra.src[1][1] = plane(B.I1[s - 1]);
-        ra.dst[0] = plane(B.I0[s]); ra.dst[1] = plane(B.I1[s]);
-        ra.sw = ws[s - 1]; ra.sh = hs[s - 1]; ra.sp = pitch[s - 1]; ra.dw = ws[s]; ra.dh = hs[s]; ra.dp = pitch[s];
+        ResizeArgs ra = resize_args(plane(B.I0[s - 1]), plane(B.I1[s - 1]), ws[s - 1], hs[s - 1], pitch[s - 1], plane(B.I0[s]),
+                                    plane(B.I1[s]), ws[s], hs[s], pitch[s]);
         ra.stride = S;
-        if ((rc = launch_bresize(ra, P.scale_step, 1.f, 0, n, st))) return rc;
+        if ((rc = launch_resize(ra, n, P.scale_step, 1.f, 0, st))) return rc;
         launches += 1;
     }
     {   // the coarsest level starts from zero flow
@@ -1231,7 +1216,7 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
     std::vector<int> total(n);
     for (int s = L - 1; s >= 0; --s) {
         const int lw = ws[s], lh = hs[s];
-        BIterArgs ia;
+        PlainIterArgs ia = {};
         ia.I1wx = plane(B.I1wx); ia.I1wy = plane(B.I1wy); ia.rho_c = plane(B.rho);
         ia.u1[0] = plane(B.u1[s]); ia.u1[1] = plane(B.u1x); ia.u2[0] = plane(B.u2[s]); ia.u2[1] = plane(B.u2x);
         ia.p11 = plane(B.p[0]); ia.p12 = plane(B.p[1]); ia.p21 = plane(B.p[2]); ia.p22 = plane(B.p[3]);
@@ -1239,10 +1224,10 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
         ia.l_t = l_t; ia.theta = theta; ia.taut = taut;
         ia.scaled_eps = (float)(P.epsilon * P.epsilon * (double)(lw * lh));
         ia.level = s; ia.inner_max = H->inner; ia.ctrl = ctrl; ia.partials = (double*)(base + B.part); ia.stride = S;
-        const dim3 gi(batch_blocks((long long)cdiv(lw, 128) * lh, TVL1_BITER_NW, n), 1, n);
-        BMedianArgs ma;
+        const dim3 gi(batch_blocks((long long)cdiv(lw, 128) * lh, TVL1_PLAIN_NW, n), 1, n);
+        MedianArgs ma = {};
         ma.u1[0] = ia.u1[0]; ma.u1[1] = ia.u1[1]; ma.u2[0] = ia.u2[0]; ma.u2[1] = ia.u2[1];
-        ma.ctrl = ctrl; ma.w = lw; ma.h = lh; ma.pitch = pitch[s]; ma.level = s; ma.stride = S;
+        ma.ctrl = ctrl; ma.w = lw; ma.h = lh; ma.pitch = pitch[s]; ma.level = s;
         const int per_thread = P.median_filtering == 3 ? 4 : 8;
         const dim3 gm(batch_blocks(2LL * cdiv(lw, per_thread) * lh, 256, n), 1, n);
         BWarpArgs wa;
@@ -1269,8 +1254,8 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
             int least_total = 0;   // fewest iterations any pair not yet done has made in this (level, warp)
             for (int no = 0; no < H->outer; ++no) {
                 if (P.median_filtering > 1) {
-                    if (P.median_filtering == 3) k_bmedian3<<<gm, 256, 0, st>>>(ma);
-                    else k_bmedian5<<<gm, 256, 0, st>>>(ma);
+                    if (P.median_filtering == 3) k_median3<<<gm, 256, 0, st>>>(ma, 2, S);
+                    else k_bmedian5<<<gm, 256, 0, st>>>(ma, S);
                     CK(cudaGetLastError());
                     launches++;
                 }
@@ -1281,8 +1266,8 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
                     want = want == 0 ? (left_pred + 1 > 4 ? left_pred + 1 : 4) : 2 * want;
                     if (want > H->inner - least_inner) want = H->inner - least_inner;
                     for (int k = 0; k < want; ++k) {
-                        k_biter_u<<<gi, dim3(32, TVL1_BITER_NW), 0, st>>>(ia);
-                        k_biter_p<<<gi, dim3(32, TVL1_BITER_NW), 0, st>>>(ia);
+                        k_plain_u<2><<<gi, dim3(32, TVL1_PLAIN_NW), 0, st>>>(ia);
+                        k_plain_p<2><<<gi, dim3(32, TVL1_PLAIN_NW), 0, st>>>(ia);
                     }
                     CK(cudaGetLastError());
                     launches += 2 * want;
@@ -1304,13 +1289,11 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
         }
         if (s == 0) break;
         // flow upsample to the next finer level, from the twin that holds each pair's flow
-        BResizeArgs ra = {};
-        ra.src[0][0] = ia.u1[0]; ra.src[0][1] = ia.u1[1]; ra.src[1][0] = ia.u2[0]; ra.src[1][1] = ia.u2[1];
-        ra.dst[0] = plane(B.u1[s - 1]); ra.dst[1] = plane(B.u2[s - 1]);
-        ra.ctrl = ctrl; ra.level = s;
-        ra.sw = lw; ra.sh = lh; ra.sp = pitch[s]; ra.dw = ws[s - 1]; ra.dh = hs[s - 1]; ra.dp = pitch[s - 1];
-        ra.stride = S;
-        if ((rc = launch_bresize(ra, 0.0, (float)(1 / P.scale_step), 1, n, st))) return rc;
+        ResizeArgs ra = resize_args(ia.u1[0], ia.u2[0], lw, lh, pitch[s], plane(B.u1[s - 1]), plane(B.u2[s - 1]), ws[s - 1],
+                                    hs[s - 1], pitch[s - 1]);
+        ra.src[0][1] = ia.u1[1]; ra.src[1][1] = ia.u2[1];
+        ra.ctrl = ctrl; ra.level = s; ra.stride = S;
+        if ((rc = launch_resize(ra, n, 0.0, (float)(1 / P.scale_step), 1, st))) return rc;
         launches += 1;
     }
     // A.8: planar output of every pair, from the twin its final Ctrl names
@@ -1743,7 +1726,8 @@ int tvl1_k_resize(const float* d_src, int sw, int sh, int spitch, float* d_dst, 
                   double inv_scale, float mul, void* stream)
 {
     if (!d_src || !d_dst || sw <= 0 || sh <= 0 || dw <= 0 || dh <= 0) return fail(TVL1_ERR_INVALID, "bad argument");
-    return launch_resize(d_src, sw, sh, spitch, d_dst, dw, dh, dpitch, inv_scale, mul, mul != 1.f, (cudaStream_t)stream);
+    return launch_resize(resize_args(d_src, nullptr, sw, sh, spitch, d_dst, nullptr, dw, dh, dpitch), 1, inv_scale, mul,
+                         mul != 1.f, (cudaStream_t)stream);
 }
 
 int tvl1_k_resize_cuda(const float* d_src, int sw, int sh, int spitch, float* d_dst, int dw, int dh, int dpitch,
@@ -1751,8 +1735,8 @@ int tvl1_k_resize_cuda(const float* d_src, int sw, int sh, int spitch, float* d_
 {
     if (!d_src || !d_dst || sw <= 0 || sh <= 0 || dw <= 0 || dh <= 0 || spitch < sw || dpitch < dw)
         return fail(TVL1_ERR_INVALID, "bad argument");
-    return launch_resize_cuda2(d_src, nullptr, sw, sh, spitch, d_dst, nullptr, dw, dh, dpitch, inv_scale, mul, mul != 1.f,
-                               (cudaStream_t)stream);
+    return launch_resize_cuda(resize_args(d_src, nullptr, sw, sh, spitch, d_dst, nullptr, dw, dh, dpitch), inv_scale, mul,
+                              mul != 1.f, (cudaStream_t)stream);
 }
 
 int tvl1_k_centered_gradient(const float* d_src, int w, int h, int pitch, float* d_dx, float* d_dy, void* stream)
@@ -1925,14 +1909,13 @@ int tvl1_k_iterate_gamma(const float* d_I1wx, const float* d_I1wy, const float* 
     CK(cudaMalloc(&tmp, total));
     cudaError_t e = cudaMemsetAsync(tmp, 0, total, st);
     if (e != cudaSuccess) { cudaFree(tmp); return fail(TVL1_ERR_CUDA, "memset: %s", cudaGetErrorString(e)); }
-    GammaArgs a;
+    PlainIterArgs a = {};
     a.I1wx = d_I1wx; a.I1wy = d_I1wy; a.rho_c = d_rho_c;
-    for (int k = 0; k < 2; k++) {
-        a.u1[k] = d_u1; a.u2[k] = d_u2; a.p11[k] = d_p11; a.p12[k] = d_p12; a.p21[k] = d_p21; a.p22[k] = d_p22;
-    }
-    a.u3 = d_u3; a.p31 = d_p31; a.p32 = d_p32;
+    a.u1[0] = a.u1[1] = d_u1; a.u2[0] = a.u2[1] = d_u2; a.u3 = d_u3;
+    a.p11 = d_p11; a.p12 = d_p12; a.p21 = d_p21; a.p22 = d_p22; a.p31 = d_p31; a.p32 = d_p32;
     a.w = w; a.h = h; a.pitch = pitch; a.l_t = l_t; a.theta = theta; a.taut = taut; a.gamma = gamma;
-    a.scaled_eps = -1.f; a.level = 0; a.slot = 0; a.inner_max = 1 << 30; a.mode = 0;
+    a.scaled_eps = -1.f;   // never stops
+    a.level = 0; a.slot = 0; a.inner_max = 1 << 30;
     a.ctrl = (Ctrl*)tmp; a.partials = (double*)(tmp + part_off); a.errlog = (double*)(tmp + log_off);
     int rc = TVL1_OK;
     stage_begin(st);
