@@ -84,7 +84,7 @@ class StackIO(C.Structure):
 EXPORTS = [
     "tvl1_version", "tvl1_last_error", "tvl1_default_params", "tvl1_create", "tvl1_destroy",
     "tvl1_set_params", "tvl1_set_option", "tvl1_set_timing", "tvl1_calc_u8", "tvl1_calc_u8_host",
-    "tvl1_calc_ex", "tvl1_calc_ex_host", "tvl1_calc_batch_u8", "tvl1_last_readbacks",
+    "tvl1_calc_ex", "tvl1_calc_ex_host", "tvl1_calc_batch_u8", "tvl1_calc_batch_ex", "tvl1_last_readbacks",
     "tvl1_prescaled_size", "tvl1_prescale_u8", "tvl1_prescale_u8_host",
     "tvl1_mask_flow_u8", "tvl1_finish_flow_u8", "tvl1_sample_matches", "tvl1_sample_matches_skip", "tvl1_sample_matches_ex",
     "tvl1_default_feature_params", "tvl1_find_alignment", "tvl1_warp_affine_u8", "tvl1_warp_affine_f32", "tvl1_stack_run", "tvl1_k_convert_u8", "tvl1_k_convert_f32", "tvl1_k_resize",
@@ -131,6 +131,8 @@ def lib():
                                     C.POINTER(Stats)]
     L.tvl1_calc_batch_u8.argtypes = [_vp, C.c_int, _vp, _sz, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, _vp,
                                      C.POINTER(Stats)]
+    L.tvl1_calc_batch_ex.argtypes = [_vp, C.c_int, C.c_int, _vp, _sz, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, _vp,
+                                     _vp, _sz, _vp, C.POINTER(Stats)]
     L.tvl1_last_readbacks.argtypes = [_vp, C.POINTER(C.c_longlong)]
     L.tvl1_mask_flow_u8.argtypes = [_vp, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, _vp]
     L.tvl1_finish_flow_u8.argtypes = [_vp, _vp, _sz, C.c_int, C.c_int, _vp, _vp, _sz, C.c_int, _vp]
@@ -297,6 +299,47 @@ def check_batch_frames(frames0, frames1):
     if 0 in shape:
         raise Tvl1Error("empty frames")
     return out[0], out[1]
+
+
+def check_batch_ex(frames0, frames1, init=None):
+    """The frames and initial flows of calc_batch_ex: two equally long, non-empty lists of 2-D frames of one size, all
+    uint8 or all float32, and init None or a list of one (u0, v0) float32 pair per pair, of the frames' size.  Returns
+    (frames0, frames1, init) as lists of C-contiguous arrays (init: None or [(u0, v0), ...]); raises Tvl1Error on
+    anything else, before the library is called."""
+    frames0, frames1 = list(frames0), list(frames1)   # an (n, h, w) stack is n frames
+    if not frames0 or len(frames0) != len(frames1):
+        raise Tvl1Error("a batch needs two equally long, non-empty lists of frames (%d and %d given)"
+                        % (len(frames0), len(frames1)))
+    f0 = [np.asarray(f) for f in frames0]
+    f1 = [np.asarray(f) for f in frames1]
+    dtype = f0[0].dtype
+    for a in f0 + f1:
+        if a.dtype not in (np.uint8, np.float32) or a.ndim != 2:
+            raise Tvl1Error("batch frames must be 2-D uint8 or float32 arrays, not %s of shape %s" % (a.dtype, a.shape))
+        if a.dtype != dtype:
+            raise Tvl1Error("the frames of a batch must all be uint8 or all float32 (%s and %s given)" % (dtype, a.dtype))
+    shape = f0[0].shape
+    if any(a.shape != shape for a in f0 + f1):
+        raise Tvl1Error("the frames of a batch must all have one size")
+    if 0 in shape:
+        raise Tvl1Error("empty frames")
+    f0 = [np.ascontiguousarray(a) for a in f0]
+    f1 = [np.ascontiguousarray(a) for a in f1]
+    if init is None:
+        return f0, f1, None
+    init = list(init)
+    if len(init) != len(f0):
+        raise Tvl1Error("init needs one (u0, v0) pair per pair of frames (%d for %d pairs)" % (len(init), len(f0)))
+    flows = []
+    for k, uv in enumerate(init):
+        uv = list(uv)
+        if len(uv) != 2:
+            raise Tvl1Error("init entry %d is not a (u0, v0) pair" % k)
+        u0, v0 = (np.asarray(a) for a in uv)
+        if u0.dtype != np.float32 or v0.dtype != np.float32 or u0.shape != shape or v0.shape != shape:
+            raise Tvl1Error("init entry %d: the initial flow planes must be float32 of the frames' size %s" % (k, shape))
+        flows.append((np.ascontiguousarray(u0), np.ascontiguousarray(v0)))
+    return f0, f1, flows
 
 
 class DevBuf:
@@ -476,6 +519,55 @@ class Solver:
         stats = (Stats * n)()
         check(lib().tvl1_calc_batch_u8(self.handle, n, arrs[0], pitch0, arrs[1], pitch1, w, h, arrs[2], arrs[3],
                                        pitch_out, stream, stats))
+        self.batch_stats = list(stats)
+
+    def calc_batch_ex(self, frames0, frames1, init=None):
+        """calc_ex for n pairs of equal size in one solve (tvl1_calc_batch_ex), in the handle's parameters whatever
+        they are (either semantics, gamma): lists (or (n, h, w) stacks) of frames, all uint8 or all float32, and init
+        None or a list of n (u0, v0) float32 planes the pairs start from.  Returns a list of (u, v) float32 pairs,
+        each exactly what calc_ex(frames0[k], frames1[k], init[k]) returns; the per-pair stats are in
+        self.batch_stats (ms_total and launches are the batch's)."""
+        f0, f1, flows = check_batch_ex(frames0, frames1, init)
+        n = len(f0)
+        h, w = f0[0].shape
+        e = f0[0].itemsize
+        ft = FRAME_U8 if e == 1 else FRAME_F32
+        plane = h * w
+        frames = DevBuf(2 * n * plane * e, self.device)
+        flow = DevBuf(2 * n * plane * 4, self.device)
+        try:
+            frames.upload(np.stack(f0 + f1))
+            d0 = [frames.ptr + k * plane * e for k in range(n)]
+            d1 = [frames.ptr + (n + k) * plane * e for k in range(n)]
+            du = [flow.ptr + k * plane * 4 for k in range(n)]
+            dv = [flow.ptr + (n + k) * plane * 4 for k in range(n)]
+            d_u0 = d_v0 = None
+            if flows is not None:   # the flow buffers start as the initial flows (in/out, as OpenCV's flow)
+                flow.upload(np.stack([f[0] for f in flows] + [f[1] for f in flows]))
+                d_u0, d_v0 = du, dv
+            self.calc_batch_ex_device(ft, d0, w * e, d1, w * e, w, h, d_u0, d_v0, w * 4, du, dv, w * 4)
+            uv = flow.download((2, n, h, w), np.float32)
+        finally:
+            frames.free()
+            flow.free()
+        return [(uv[0, k].copy(), uv[1, k].copy()) for k in range(n)]
+
+    def calc_batch_ex_device(self, frame_type, d_f0, pitch0, d_f1, pitch1, w, h, d_u0, d_v0, pitch_init, d_u, d_v,
+                             pitch_out, stream=None):
+        """tvl1_calc_batch_ex over lists of device pointers (pair k: d_f0[k], d_f1[k], from d_u0[k], d_v0[k] ->
+        d_u[k], d_v[k]; d_u0 and d_v0 None: zero start); the per-pair stats go to self.batch_stats"""
+        lists = [list(x) for x in (d_f0, d_f1, d_u, d_v)]
+        if d_u0 is not None or d_v0 is not None:
+            lists += [list(x) if x is not None else [] for x in (d_u0, d_v0)]
+        n = len(lists[0])
+        if n < 1 or any(len(x) != n for x in lists):
+            raise Tvl1Error("a batch needs equally long, non-empty pointer lists (%s given)"
+                            % ", ".join(str(len(x)) for x in lists))
+        arrs = [(C.c_void_p * n)(*x) for x in lists]
+        init = (arrs[4], arrs[5]) if len(arrs) == 6 else (None, None)
+        stats = (Stats * n)()
+        check(lib().tvl1_calc_batch_ex(self.handle, n, frame_type, arrs[0], pitch0, arrs[1], pitch1, w, h, init[0],
+                                       init[1], pitch_init, arrs[2], arrs[3], pitch_out, stream, stats))
         self.batch_stats = list(stats)
 
     def last_readbacks(self):

@@ -6,7 +6,8 @@ NumPy arrays in place of cv::Mat / GpuMat:
 
     generate_TV_args(im_args, args)            src/optflow.cpp:500-514
     TVL1_solve(frame0, frame1, TV_args)        src/optflow.cpp:516-520
-    TVL1_solve_batch(frame0s, frame1s, TV_args) many equal-size pairs in one call (no counterpart)
+    TVL1_solve_batch(frame0s, frame1s, TV_args, init_flows=None)
+                                               many equal-size pairs in one call (no counterpart)
     find_alignment(frame0, frame1, ...)        src/features.cpp:46-167
     solve_rois(frame0, frame1, rois, ...)      src/optflow.cpp:312-392
     solve_wrapper(frame0, frame1, ...)         src/optflow.cpp:395-497
@@ -123,11 +124,13 @@ def TVL1_solve(frame0, frame1, TV_args, device=0, init_flow=None):
     return s.calc_ex(frame0, frame1, init=init_flow)
 
 
-def TVL1_solve_batch(frame0s, frame1s, TV_args, device=0):
-    """TVL1_solve of many pairs of one size in one call: lists of uint8 frames in, a list of (flow_x, flow_y) float32
-    planes out, each exactly what TVL1_solve of that pair returns.  Solving equal-size ROI strips a batch at a time
-    keeps the GPU busy where one small pair leaves it mostly idle."""
-    return _solver_for(TV_args, device).calc_batch(frame0s, frame1s)
+def TVL1_solve_batch(frame0s, frame1s, TV_args, device=0, init_flows=None):
+    """TVL1_solve of many pairs of one size in one call: lists of frames (all uint8, or all float32 -- scaled by 255,
+    as TVL1_solve does with an init_flow) in, a list of (flow_x, flow_y) float32 planes out, each exactly what
+    TVL1_solve of that pair returns, in either "semantics" and with any gamma.  init_flows: None, or one (flow_x,
+    flow_y) pair of float32 planes per pair, as TVL1_solve's init_flow.  Solving equal-size ROI strips a batch at a time keeps the GPU busy where one small pair leaves it
+    mostly idle."""
+    return _solver_for(TV_args, device).calc_batch_ex(frame0s, frame1s, init=init_flows)
 
 
 # orb_defaults (src/features.cpp:19-32) and the matcher / RANSAC keys (:107, :133)

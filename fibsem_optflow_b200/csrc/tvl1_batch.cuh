@@ -1,12 +1,13 @@
-// tvl1_batch.cuh -- the kernels only tvl1_calc_batch_u8 launches: n pairs of one size per launch.
+// tvl1_batch.cuh -- the kernels only batches (tvl1_calc_batch_ex, tvl1_calc_batch_u8) launch: n pairs of one size
+// per launch.
 //
 // The batch arena holds n copies of a pair's state at one fixed distance, `stride` bytes (a multiple of 256): pair b's
 // copy of a plane -- and its Ctrl -- is the pair-0 pointer plus b * stride (at_pair).  blockIdx.z is the pair
 // everywhere.  These kernels serve the small-frame regime, where a pair alone leaves most of the GPU idle and the
 // launch latency dominates: no TMA staging, plain global loads.  A batch also launches the kernels of tvl1_kernels.cuh
-// that take a pair stride: k_resize / k_resize_half, k_median3 and the plain iteration k_plain_u<2> / k_plain_p<2>.
-// Every value is computed with the operations, and in the order, of the single-pair kernels, so each pair's flow and
-// iteration counts are those of tvl1_calc_u8.  Each pair keeps its own stop state in its own Ctrl; every kernel but
+// that take a pair: k_resize / k_resize_half / k_resize_cuda, k_median3, k_warp_cuda and the plain iteration
+// k_plain_u / k_plain_p.  Every value is computed with the operations, and in the order, of the single-pair kernels,
+// so each pair's flow and iteration counts are those of tvl1_calc_ex.  Each pair keeps its own stop state in its own Ctrl; every kernel but
 // the warp returns at once for a pair whose `done` is set.
 #pragma once
 #include "tvl1_kernels.cuh"
@@ -34,6 +35,32 @@ __global__ void __launch_bounds__(256) k_bconvert_u8(const uint8_t* const* __res
         o.w = x + 3 < w ? (float)s[3] : 0.f;
     }
     *reinterpret_cast<float4*>(at_pair(f ? I1 : I0, stride, b) + (size_t)y * dpitch + x) = o;
+}
+
+// A.2 for fp32 frames, as k_convert_f32 (convert_f32_px); pitch0 / pitch1 in elements; src and blockIdx.z as
+// k_bconvert_u8's
+__global__ void __launch_bounds__(256) k_bconvert_f32(const float* const* __restrict__ src, size_t pitch0, size_t pitch1,
+                                                      int w, int h, float* I0, float* I1, int dpitch, size_t stride)
+{
+    const int b = blockIdx.z >> 1, f = blockIdx.z & 1;
+    const int x = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
+    const int y = blockIdx.y * blockDim.y + threadIdx.y;
+    if (y >= h || x >= w) return;
+    const float* s = src[f * (gridDim.z >> 1) + b] + (size_t)y * (f ? pitch1 : pitch0) + x;
+    *reinterpret_cast<float4*>(at_pair(f ? I1 : I0, stride, b) + (size_t)y * dpitch + x) = convert_f32_px(s, x, w);
+}
+
+// useInitialFlow: every pair's (u0, v0) -> its level-0 twin 0 (u1, u2), columns 0 .. w - 1 as the single pair's
+// row copy.  src: the 2n plane pointers, u0 of every pair then v0 of every pair; spitch in elements;
+// blockIdx.z = 2 * pair + plane
+__global__ void __launch_bounds__(256) k_bload_flow(const float* const* __restrict__ src, size_t spitch, int w, int h,
+                                                    float* u1, float* u2, int dpitch, size_t stride)
+{
+    const int b = blockIdx.z >> 1, f = blockIdx.z & 1;
+    const int x = blockIdx.x * blockDim.x + threadIdx.x;
+    const int y = blockIdx.y * blockDim.y + threadIdx.y;
+    if (y >= h || x >= w) return;
+    at_pair(f ? u2 : u1, stride, b)[(size_t)y * dpitch + x] = __ldg(src[f * (gridDim.z >> 1) + b] + (size_t)y * spitch + x);
 }
 
 struct BWarpArgs {

@@ -203,7 +203,19 @@ static ResizeArgs resize_args(const float* srcA, const float* srcB, int sw, int 
     return a;
 }
 
-// a's planes of n pairs (two planes each; one plane: n is 1) resized alike in one launch.  inv_scale > 0:
+// gridDim.z of a resize of a's planes of n pairs.  One plane (dst[1] null) of n > 1 pairs, without a ctrl: pair k's
+// plane is taken as plane k & 1 of pair k >> 1 at twice the stride
+static unsigned resize_z(ResizeArgs& a, int n)
+{
+    if (a.dst[1]) return 2 * n;
+    if (n == 1) return 1;
+    a.src[1][0] = (const float*)((const char*)a.src[0][0] + a.stride);
+    a.dst[1] = (float*)((char*)a.dst[0] + a.stride);
+    a.stride *= 2;
+    return n;
+}
+
+// a's planes of n pairs (two planes each, or one: see resize_z) resized alike in one launch.  inv_scale > 0:
 // resize(src, Size(), inv_scale, inv_scale); otherwise the explicit size dw x dh.  apply_mul: see scale_px
 int launch_resize(ResizeArgs a, int n, double inv_scale, double mul, int apply_mul, cudaStream_t st)
 {
@@ -211,7 +223,7 @@ int launch_resize(ResizeArgs a, int n, double inv_scale, double mul, int apply_m
     if (inv_scale > 0) { inv_x = inv_scale; inv_y = inv_scale; }
     else { inv_x = (double)a.dw / a.sw; inv_y = (double)a.dh / a.sh; }
     a.scale_x = 1. / inv_x; a.scale_y = 1. / inv_y; a.mul = mul; a.apply_mul = apply_mul;
-    const unsigned nz = a.dst[1] ? 2 * n : 1;
+    const unsigned nz = resize_z(a, n);
     dim3 b(32, 8);
     // resize(src, Size(), 0.5, 0.5): OpenCV's INTER_AREA fast path.  The fp32 multiply (tvl1_k_resize with mul != 1)
     // has always taken the bilinear kernel at 0.5 and keeps doing so; the fp64 one (an initial flow's downscale) is
@@ -222,17 +234,17 @@ int launch_resize(ResizeArgs a, int n, double inv_scale, double mul, int apply_m
     return TVL1_OK;
 }
 
-// cv::cuda semantics: cuda::resize(INTER_LINEAR) of a's planes (one pair, twin 0).  inv_scale > 0:
-// resize(src, Size(), inv_scale, inv_scale); otherwise the explicit size dw x dh (factor dw / sw in fp64).
-int launch_resize_cuda(const ResizeArgs& a, double inv_scale, double mul, int apply_mul, cudaStream_t st)
+// cv::cuda semantics: cuda::resize(INTER_LINEAR) of a's planes of n pairs, as launch_resize.  inv_scale > 0:
+// resize(src, Size(), inv_scale, inv_scale); otherwise the explicit size dw x dh (factor dw / sw in fp64).  The
+// source step fx = (float)(1 / factor) and the multiply by (float)mul (apply_mul != 0) are fp32.
+int launch_resize_cuda(ResizeArgs a, int n, double inv_scale, double mul, int apply_mul, cudaStream_t st)
 {
     const double f_x = inv_scale > 0 ? inv_scale : (double)a.dw / a.sw;
     const double f_y = inv_scale > 0 ? inv_scale : (double)a.dh / a.sh;
-    const float fx = (float)(1.0 / f_x), fy = (float)(1.0 / f_y);
+    a.scale_x = 1.0 / f_x; a.scale_y = 1.0 / f_y; a.mul = mul; a.apply_mul = apply_mul;
     dim3 b(32, 8);
-    dim3 g(cdiv(a.dw, 32), cdiv(a.dh, 8), a.dst[1] ? 2 : 1);
-    k_resize_cuda<<<g, b, 0, st>>>(a.src[0][0], a.src[1][0], a.sw, a.sh, a.sp, a.dst[0], a.dst[1], a.dw, a.dh, a.dp, fx, fy,
-                                   (float)mul, apply_mul);
+    dim3 g(cdiv(a.dw, 32), cdiv(a.dh, 8), resize_z(a, n));
+    k_resize_cuda<<<g, b, 0, st>>>(a);
     CK(cudaGetLastError());
     return TVL1_OK;
 }
@@ -275,11 +287,11 @@ int launch_warp_cuda(const WarpArgs& a, cudaStream_t st)
     if (!resident) {
         int sms = 148, occ = 0;
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_warp_cuda, 256, 0) != cudaSuccess || occ < 1) occ = 2;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_warp_cuda<false>, 256, 0) != cudaSuccess || occ < 1) occ = 2;
         resident = sms * occ;
     }
     const long long ntiles = (long long)cdiv(a.w, TVL1_WC_TW) * cdiv(a.h, TVL1_WC_TH);
-    k_warp_cuda<<<(unsigned)(ntiles < resident ? ntiles : resident), dim3(32, 8), 0, st>>>(a);
+    k_warp_cuda<false><<<(unsigned)(ntiles < resident ? ntiles : resident), dim3(32, 8), 0, st>>>(a, 0);
     CK(cudaGetLastError());
     return TVL1_OK;
 }
@@ -516,10 +528,11 @@ struct Level {
     float *I0, *I1, *u1, *u2;   // u1/u2: buffer [0] of the twin pair; [1] is shared scratch
 };
 
-// Byte offsets of one pair's state in the batch arena (tvl1_calc_batch_u8); pair b's copy is at + b * stride
+// Byte offsets of one pair's state in the batch arena (tvl1_calc_batch_ex); pair b's copy is at + b * stride.
+// u3, p31, p32: only in an arena made for gamma != 0
 struct BatchLayout {
-    size_t I0[TVL1_MAX_LEVELS], I1[TVL1_MAX_LEVELS], u1[TVL1_MAX_LEVELS], u2[TVL1_MAX_LEVELS];
-    size_t u1x, u2x, I1wx, I1wy, rho, p[4], part, ctrl;
+    size_t I0[TVL1_MAX_LEVELS], I1[TVL1_MAX_LEVELS], u1[TVL1_MAX_LEVELS], u2[TVL1_MAX_LEVELS], u3[TVL1_MAX_LEVELS];
+    size_t u1x, u2x, I1wx, I1wy, rho, p[4], p31, p32, part, ctrl;
 };
 
 }  // namespace tvl1
@@ -575,12 +588,14 @@ struct tvl1_handle {
     int st_w = 0, st_h = 0;
     cudaStream_t st_in = nullptr, st_out = nullptr;
     cudaEvent_t st_up[TVL1_STACK_SLOTS] = {}, st_ready[2] = {nullptr, nullptr}, st_down[2] = {nullptr, nullptr};
-    // batch arena (tvl1_calc_batch_u8), apart from the single-pair one: bcap_n copies of a pair's state at
-    // bstride bytes, then the 2 * bcap_n frame pointers; pinned: bcap_n Ctrl read-backs, then the frame pointers
+    // batch arena (tvl1_calc_batch_ex), apart from the single-pair one: bcap_n copies of a pair's state at
+    // bstride bytes, then the 4 * bcap_n pointers of the frames and initial flows; pinned: bcap_n Ctrl read-backs,
+    // then those pointers.  bcap_gamma: the pairs' state includes the planes of the third channel
     char* barena = nullptr;
     char* bhost = nullptr;
     size_t bstride = 0;
     int bcap_n = 0, bcap_w = 0, bcap_h = 0, bcap_scales = 0;
+    bool bcap_gamma = false;
     double bcap_step = 0;
     BatchLayout bl;
     long long readbacks = 0;   // host read-backs of the stop state by the last calc
@@ -855,7 +870,7 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
     for (int s = 1; s < L; s++) {
         const Level &a = H->lv[s - 1], &b = H->lv[s];
         const ResizeArgs ra = resize_args(a.I0, a.I1, a.w, a.h, a.pitch, b.I0, b.I1, b.w, b.h, b.pitch);
-        if ((rc = cs ? launch_resize_cuda(ra, P.scale_step, 1.f, 0, st) : launch_resize(ra, 1, P.scale_step, 1.f, 0, st)))
+        if ((rc = cs ? launch_resize_cuda(ra, 1, P.scale_step, 1.f, 0, st) : launch_resize(ra, 1, P.scale_step, 1.f, 0, st)))
             return rc;
         launches += 1;
     }
@@ -870,7 +885,7 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
         for (int s = 1; s < L; s++) {
             const Level &a = H->lv[s - 1], &b = H->lv[s];
             const ResizeArgs ra = resize_args(a.u1, a.u2, a.w, a.h, a.pitch, b.u1, b.u2, b.w, b.h, b.pitch);
-            rc = cs ? launch_resize_cuda(ra, P.scale_step, (float)P.scale_step, 1, st)
+            rc = cs ? launch_resize_cuda(ra, 1, P.scale_step, (float)P.scale_step, 1, st)
                     : launch_resize(ra, 1, P.scale_step, P.scale_step, 2, st);
             if (rc) return rc;
             launches += 1;
@@ -1027,7 +1042,7 @@ static int calc_device(tvl1_handle* H, int frame_type, const void* f0, size_t pi
         if ((rc = span_begin(3, s))) return rc;
         const ResizeArgs ra = resize_args(uc ? H->u1x : lv.u1, uc ? H->u2x : lv.u2, lv.w, lv.h, lv.pitch, up.u1, up.u2, up.w,
                                           up.h, up.pitch);
-        if ((rc = cs ? launch_resize_cuda(ra, 0.0, mul, 1, st) : launch_resize(ra, 1, 0.0, mul, 1, st))) return rc;
+        if ((rc = cs ? launch_resize_cuda(ra, 1, 0.0, mul, 1, st) : launch_resize(ra, 1, 0.0, mul, 1, st))) return rc;
         launches += 1;
         if (with_gamma) {   // u3 is zoomed like the flow but not scaled
             if ((rc = launch_resize(resize_args(H->u3[s], nullptr, lv.w, lv.h, lv.pitch, H->u3[s - 1], nullptr, up.w, up.h,
@@ -1082,11 +1097,13 @@ static void release_batch(tvl1_handle* H)
     H->bcap_n = H->bcap_w = H->bcap_h = 0;
 }
 
-// the batch arena for n pairs of w x h: kept while it has room for n pairs of this size and pyramid
+// the batch arena for n pairs of w x h: kept while it has room for n pairs of this size and pyramid, and the planes of
+// the third channel when gamma != 0
 static int ensure_batch(tvl1_handle* H, int n, int w, int h, cudaStream_t st)
 {
+    const bool gamma = H->prm.gamma != 0.0;
     if (H->barena && H->bcap_n >= n && H->bcap_w == w && H->bcap_h == h && H->bcap_scales == H->prm.nscales &&
-        H->bcap_step == H->prm.scale_step)
+        H->bcap_step == H->prm.scale_step && (H->bcap_gamma || !gamma))
         return TVL1_OK;
     release_batch(H);
     int ws[TVL1_MAX_LEVELS + 1], hs[TVL1_MAX_LEVELS + 1];
@@ -1102,9 +1119,13 @@ static int ensure_batch(tvl1_handle* H, int n, int w, int h, cudaStream_t st)
     B.u1x = carve(b0); B.u2x = carve(b0);
     B.I1wx = carve(b0); B.I1wy = carve(b0); B.rho = carve(b0);
     for (int k = 0; k < 4; k++) B.p[k] = carve(b0);
+    if (gamma) {
+        for (int s = 0; s < L; s++) B.u3[s] = carve((size_t)round_up(ws[s], 32) * hs[s] * sizeof(float));
+        B.p31 = carve(b0); B.p32 = carve(b0);
+    }
     B.part = carve(TVL1_BATCH_MAX_BLOCKS * sizeof(double));
     B.ctrl = carve(sizeof(Ctrl));
-    const size_t ptrs = ((size_t)2 * n * sizeof(void*) + 255) / 256 * 256;
+    const size_t ptrs = ((size_t)4 * n * sizeof(void*) + 255) / 256 * 256;
     if (off > (SIZE_MAX - ptrs) / (size_t)n)
         return fail(TVL1_ERR_NOMEM, "a batch of %d pairs of %dx%d does not fit in the address space", n, w, h);
     const size_t total = off * (size_t)n + ptrs;
@@ -1115,7 +1136,7 @@ static int ensure_batch(tvl1_handle* H, int n, int w, int h, cudaStream_t st)
         return fail(TVL1_ERR_NOMEM, "cudaMalloc(%zu bytes) for a batch of %d pairs of %dx%d failed: %s", total, n, w, h,
                     cudaGetErrorString(e));
     }
-    e = cudaMallocHost(&H->bhost, (size_t)n * sizeof(Ctrl) + (size_t)2 * n * sizeof(void*));
+    e = cudaMallocHost(&H->bhost, (size_t)n * sizeof(Ctrl) + (size_t)4 * n * sizeof(void*));
     if (e != cudaSuccess) {
         cudaGetLastError();
         H->bhost = nullptr;
@@ -1124,6 +1145,7 @@ static int ensure_batch(tvl1_handle* H, int n, int w, int h, cudaStream_t st)
     }
     H->bstride = off;
     H->bcap_n = n; H->bcap_w = w; H->bcap_h = h; H->bcap_scales = H->prm.nscales; H->bcap_step = H->prm.scale_step;
+    H->bcap_gamma = gamma;
     CK(cudaMemsetAsync(H->barena, 0, total, st));   // pad columns are read (never used): defined contents
     return TVL1_OK;
 }
@@ -1142,20 +1164,24 @@ static int batch_blocks(long long units, int per_block, int n)
 }
 
 // calc_device's loop in lockstep over n pairs of one size: the same (level, warp, outer iteration) for every pair,
-// each with its own stop state, so that every pair sees the kernel sequence of its own solve
-static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pitch0, const uint8_t* const* f1,
-                      size_t pitch1, int w, int h, float* const* d_u, float* const* d_v, size_t pitch_out,
-                      cudaStream_t st, tvl1_stats* stats)
+// each with its own stop state, so that every pair sees the kernel sequence of its own solve.  Its choices are
+// calc_device's: in cuda semantics cv::cuda's resize and warp, no median and one outer iteration of `iterations`;
+// with gamma != 0 the three-channel iteration.  u0 / v0 (both or neither): each pair's initial flow, whose entries
+// may be those of d_u / d_v
+static int calc_batch(tvl1_handle* H, int n, int frame_type, const void* const* f0, size_t pitch0, const void* const* f1,
+                      size_t pitch1, int w, int h, const float* const* u0, const float* const* v0, size_t pitch_init,
+                      float* const* d_u, float* const* d_v, size_t pitch_out, cudaStream_t st, tvl1_stats* stats)
 {
     const tvl1_params& P = H->prm;
-    if (P.semantics == TVL1_SEMANTICS_CUDA)
-        return fail(TVL1_ERR_UNSUPPORTED, "tvl1_calc_batch_u8 solves in CPU-class semantics only, not cuda semantics");
-    if (P.gamma != 0.0) return fail(TVL1_ERR_UNSUPPORTED, "tvl1_calc_batch_u8 does not support gamma != 0");
     if (n < 1 || n > TVL1_BATCH_MAX_PAIRS) return fail(TVL1_ERR_INVALID, "n must be in 1 .. %d, not %d", TVL1_BATCH_MAX_PAIRS, n);
     if (!f0 || !f1 || !d_u || !d_v) return fail(TVL1_ERR_INVALID, "null pointer array");
-    for (int k = 0; k < n; k++)
+    if ((u0 == nullptr) != (v0 == nullptr))
+        return fail(TVL1_ERR_INVALID, "the initial flow needs both pointer arrays (or neither)");
+    for (int k = 0; k < n; k++) {
         if (!f0[k] || !f1[k] || !d_u[k] || !d_v[k]) return fail(TVL1_ERR_INVALID, "null image or flow pointer in entry %d", k);
-    int rc = check_frames(TVL1_FRAME_U8, pitch0, pitch1, w, h, nullptr, nullptr, 0, pitch_out);
+        if (u0 && (!u0[k] || !v0[k])) return fail(TVL1_ERR_INVALID, "null initial-flow pointer in entry %d", k);
+    }
+    int rc = check_frames(frame_type, pitch0, pitch1, w, h, u0 ? u0[0] : nullptr, v0 ? v0[0] : nullptr, pitch_init, pitch_out);
     if (rc) return rc;
     if (w > 32767 || h > 32767) return fail(TVL1_ERR_INVALID, "image side > 32767 (remap uses int16 coordinates)");
     CK(cudaSetDevice(H->device));
@@ -1166,14 +1192,15 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
     int pitch[TVL1_MAX_LEVELS];
     for (int s = 0; s < L; s++) pitch[s] = round_up(ws[s], 32);
     const float l_t = (float)(P.lambda * P.theta), taut = (float)(P.tau / P.theta), theta = (float)P.theta;
+    const bool cs = P.semantics == TVL1_SEMANTICS_CUDA, with_gamma = P.gamma != 0.0;
     const BatchLayout& B = H->bl;
     const size_t S = H->bstride;
     char* const base = H->barena;
     auto plane = [&](size_t o) { return (float*)(base + o); };
     Ctrl* const ctrl = (Ctrl*)(base + B.ctrl);
     Ctrl* const hc = (Ctrl*)H->bhost;                                          // pair b's read-back: hc[b]
-    const uint8_t** const hptr = (const uint8_t**)(H->bhost + (size_t)n * sizeof(Ctrl));
-    const uint8_t** const dptr = (const uint8_t**)(base + (size_t)H->bcap_n * S);
+    const void** const hptr = (const void**)(H->bhost + (size_t)n * sizeof(Ctrl));   // f0[], f1[], u0[], v0[]
+    const void** const dptr = (const void**)(base + (size_t)H->bcap_n * S);
     const size_t hdr = offsetof(Ctrl, iters);
     long long launches = 0;
     H->ev_used = 0;
@@ -1193,23 +1220,53 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
     CK(cudaEventRecord(ev_begin, st));
     CK(cudaMemset2DAsync(ctrl, S, 0, sizeof(Ctrl), n, st));
     // (1) pyramid of every pair
-    for (int k = 0; k < n; k++) { hptr[k] = f0[k]; hptr[n + k] = f1[k]; }
-    CK(cudaMemcpyAsync(dptr, hptr, (size_t)2 * n * sizeof(void*), cudaMemcpyHostToDevice, st));
-    k_bconvert_u8<<<dim3(cdiv(cdiv(w, 4), 32), cdiv(h, 8), 2 * n), dim3(32, 8), 0, st>>>(
-        dptr, pitch0, pitch1, w, h, plane(B.I0[0]), plane(B.I1[0]), pitch[0], S);
+    const int nptr = u0 ? 4 * n : 2 * n;
+    for (int k = 0; k < n; k++) {
+        hptr[k] = f0[k]; hptr[n + k] = f1[k];
+        if (u0) { hptr[2 * n + k] = u0[k]; hptr[3 * n + k] = v0[k]; }
+    }
+    CK(cudaMemcpyAsync(dptr, hptr, (size_t)nptr * sizeof(void*), cudaMemcpyHostToDevice, st));
+    const dim3 gc(cdiv(cdiv(w, 4), 32), cdiv(h, 8), 2 * n);
+    if (frame_type == TVL1_FRAME_F32)
+        k_bconvert_f32<<<gc, dim3(32, 8), 0, st>>>((const float* const*)dptr, pitch0 / 4, pitch1 / 4, w, h, plane(B.I0[0]),
+                                                   plane(B.I1[0]), pitch[0], S);
+    else
+        k_bconvert_u8<<<gc, dim3(32, 8), 0, st>>>((const uint8_t* const*)dptr, pitch0, pitch1, w, h, plane(B.I0[0]),
+                                                  plane(B.I1[0]), pitch[0], S);
     CK(cudaGetLastError());
     launches += 1;
     for (int s = 1; s < L; s++) {
         ResizeArgs ra = resize_args(plane(B.I0[s - 1]), plane(B.I1[s - 1]), ws[s - 1], hs[s - 1], pitch[s - 1], plane(B.I0[s]),
                                     plane(B.I1[s]), ws[s], hs[s], pitch[s]);
         ra.stride = S;
-        if ((rc = launch_resize(ra, n, P.scale_step, 1.f, 0, st))) return rc;
+        if ((rc = cs ? launch_resize_cuda(ra, n, P.scale_step, 1.f, 0, st) : launch_resize(ra, n, P.scale_step, 1.f, 0, st)))
+            return rc;
         launches += 1;
     }
-    {   // the coarsest level starts from zero flow
+    if (u0) {
+        // useInitialFlow, as calc_device: level 0 is each pair's flow, each coarser level the finer one resized and
+        // times scaleStep (fp64 in the CPU class, fp32 in cv::cuda).  Into twin 0; the coarsest level is not zeroed
+        k_bload_flow<<<dim3(cdiv(w, 32), cdiv(h, 8), 2 * n), dim3(32, 8), 0, st>>>(
+            (const float* const*)(dptr + 2 * n), pitch_init / 4, w, h, plane(B.u1[0]), plane(B.u2[0]), pitch[0], S);
+        CK(cudaGetLastError());
+        launches += 1;
+        for (int s = 1; s < L; s++) {
+            ResizeArgs ra = resize_args(plane(B.u1[s - 1]), plane(B.u2[s - 1]), ws[s - 1], hs[s - 1], pitch[s - 1],
+                                        plane(B.u1[s]), plane(B.u2[s]), ws[s], hs[s], pitch[s]);
+            ra.stride = S;
+            rc = cs ? launch_resize_cuda(ra, n, P.scale_step, (float)P.scale_step, 1, st)
+                    : launch_resize(ra, n, P.scale_step, P.scale_step, 2, st);
+            if (rc) return rc;
+            launches += 1;
+        }
+    }
+    {   // the coarsest level starts from zero flow (without an initial one), u3 from zero
         const size_t b = (size_t)pitch[L - 1] * hs[L - 1] * sizeof(float);
-        CK(cudaMemset2DAsync(plane(B.u1[L - 1]), S, 0, b, n, st));
-        CK(cudaMemset2DAsync(plane(B.u2[L - 1]), S, 0, b, n, st));
+        if (!u0) {
+            CK(cudaMemset2DAsync(plane(B.u1[L - 1]), S, 0, b, n, st));
+            CK(cudaMemset2DAsync(plane(B.u2[L - 1]), S, 0, b, n, st));
+        }
+        if (with_gamma) CK(cudaMemset2DAsync(plane(B.u3[L - 1]), S, 0, b, n, st));
     }
 
     std::vector<int> counts((size_t)L * W, 0);   // the most iterations any pair needed per (level, warp)
@@ -1224,6 +1281,15 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
         ia.l_t = l_t; ia.theta = theta; ia.taut = taut;
         ia.scaled_eps = (float)(P.epsilon * P.epsilon * (double)(lw * lh));
         ia.level = s; ia.inner_max = H->inner; ia.ctrl = ctrl; ia.partials = (double*)(base + B.part); ia.stride = S;
+        ia.eps_d = P.epsilon * P.epsilon * (double)(lw * lh);
+        ia.err_on = P.epsilon > 0.0;
+        if (with_gamma) {
+            ia.u3 = plane(B.u3[s]); ia.p31 = plane(B.p31); ia.p32 = plane(B.p32); ia.gamma = (float)P.gamma;
+            // p31 / p32 start the level at zero (the warp zeroes p11 .. p22)
+            const size_t pb = (size_t)pitch[s] * lh * sizeof(float);
+            CK(cudaMemset2DAsync(ia.p31, S, 0, pb, n, st));
+            CK(cudaMemset2DAsync(ia.p32, S, 0, pb, n, st));
+        }
         const dim3 gi(batch_blocks((long long)cdiv(lw, 128) * lh, TVL1_PLAIN_NW, n), 1, n);
         MedianArgs ma = {};
         ma.u1[0] = ia.u1[0]; ma.u1[1] = ia.u1[1]; ma.u2[0] = ia.u2[0]; ma.u2[1] = ia.u2[1];
@@ -1236,14 +1302,22 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
         wa.I1wx = plane(B.I1wx); wa.I1wy = plane(B.I1wy); wa.rho_c = plane(B.rho);
         wa.ctrl = ctrl; wa.w = lw; wa.h = lh; wa.pitch = pitch[s]; wa.level = s; wa.stride = S;
         const dim3 gw(cdiv(lw, 32), cdiv(lh, 8), n);
+        WarpArgs wc;   // cuda semantics: k_warp_cuda, persistent blocks per pair over its 32 x 16 tiles
+        memset(wc.tmI1, 0, sizeof(wc.tmI1));   // not read by k_warp_cuda
+        wc.I0 = wa.I0; wc.I1 = wa.I1;
+        wc.u1[0] = ia.u1[0]; wc.u1[1] = ia.u1[1]; wc.u2[0] = ia.u2[0]; wc.u2[1] = ia.u2[1];
+        wc.I1w = nullptr; wc.I1wx = wa.I1wx; wc.I1wy = wa.I1wy; wc.grad = nullptr; wc.rho_c = wa.rho_c;
+        wc.w = lw; wc.h = lh; wc.pitch = pitch[s]; wc.level = s; wc.one = 1.0f; wc.ctrl = ctrl;
+        const dim3 gwc(batch_blocks((long long)cdiv(lw, TVL1_WC_TW) * cdiv(lh, TVL1_WC_TH), 1, n), 1, n);
 
         for (int wi = 0; wi < W; ++wi) {
             const int slot = s * W + wi;
             ia.slot = slot;
             ma.slot = slot;
             // (2) warp; the level's first warp also zeroes p11 .. p22 and every warp re-arms the stop test
-            for (int k = 0; k < 4; k++) wa.pz[k] = wi == 0 ? plane(B.p[k]) : nullptr;
-            k_bwarp<<<gw, dim3(32, 8), 0, st>>>(wa);
+            for (int k = 0; k < 4; k++) wa.pz[k] = wc.pz[k] = wi == 0 ? plane(B.p[k]) : nullptr;
+            if (cs) k_warp_cuda<true><<<gwc, dim3(32, 8), 0, st>>>(wc, S);
+            else k_bwarp<<<gw, dim3(32, 8), 0, st>>>(wa);
             CK(cudaGetLastError());
             launches++;
             // (3) outer iterations, as calc_device: chunks of iterations enqueued without knowing how many run,
@@ -1253,7 +1327,7 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
             std::fill(total.begin(), total.end(), 0);
             int least_total = 0;   // fewest iterations any pair not yet done has made in this (level, warp)
             for (int no = 0; no < H->outer; ++no) {
-                if (P.median_filtering > 1) {
+                if (P.median_filtering > 1 && !cs) {
                     if (P.median_filtering == 3) k_median3<<<gm, 256, 0, st>>>(ma, 2, S);
                     else k_bmedian5<<<gm, 256, 0, st>>>(ma, S);
                     CK(cudaGetLastError());
@@ -1266,8 +1340,11 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
                     want = want == 0 ? (left_pred + 1 > 4 ? left_pred + 1 : 4) : 2 * want;
                     if (want > H->inner - least_inner) want = H->inner - least_inner;
                     for (int k = 0; k < want; ++k) {
-                        k_plain_u<2><<<gi, dim3(32, TVL1_PLAIN_NW), 0, st>>>(ia);
-                        k_plain_p<2><<<gi, dim3(32, TVL1_PLAIN_NW), 0, st>>>(ia);
+                        if (cs) k_plain_u<2, true><<<gi, dim3(32, TVL1_PLAIN_NW), 0, st>>>(ia);
+                        else if (with_gamma) k_plain_u<3><<<gi, dim3(32, TVL1_PLAIN_NW), 0, st>>>(ia);
+                        else k_plain_u<2><<<gi, dim3(32, TVL1_PLAIN_NW), 0, st>>>(ia);
+                        if (with_gamma) k_plain_p<3><<<gi, dim3(32, TVL1_PLAIN_NW), 0, st>>>(ia);
+                        else k_plain_p<2><<<gi, dim3(32, TVL1_PLAIN_NW), 0, st>>>(ia);
                     }
                     CK(cudaGetLastError());
                     launches += 2 * want;
@@ -1288,13 +1365,21 @@ static int calc_batch(tvl1_handle* H, int n, const uint8_t* const* f0, size_t pi
             counts[slot] = *std::max_element(total.begin(), total.end());
         }
         if (s == 0) break;
-        // flow upsample to the next finer level, from the twin that holds each pair's flow
+        // flow upsample to the next finer level, from the twin that holds each pair's flow, times 1/scaleStep
         ResizeArgs ra = resize_args(ia.u1[0], ia.u2[0], lw, lh, pitch[s], plane(B.u1[s - 1]), plane(B.u2[s - 1]), ws[s - 1],
                                     hs[s - 1], pitch[s - 1]);
         ra.src[0][1] = ia.u1[1]; ra.src[1][1] = ia.u2[1];
         ra.ctrl = ctrl; ra.level = s; ra.stride = S;
-        if ((rc = launch_resize(ra, n, 0.0, (float)(1 / P.scale_step), 1, st))) return rc;
+        const float mul = (float)(1 / P.scale_step);
+        if ((rc = cs ? launch_resize_cuda(ra, n, 0.0, mul, 1, st) : launch_resize(ra, n, 0.0, mul, 1, st))) return rc;
         launches += 1;
+        if (with_gamma) {   // u3 is zoomed like the flow but not scaled (one buffer: no ctrl)
+            ResizeArgs r3 = resize_args(ia.u3, nullptr, lw, lh, pitch[s], plane(B.u3[s - 1]), nullptr, ws[s - 1], hs[s - 1],
+                                        pitch[s - 1]);
+            r3.stride = S;
+            if ((rc = launch_resize(r3, n, 0.0, 1.f, 0, st))) return rc;
+            launches += 1;
+        }
     }
     // A.8: planar output of every pair, from the twin its final Ctrl names
     if ((rc = read_ctrl(sizeof(Ctrl)))) return rc;
@@ -1482,13 +1567,26 @@ int tvl1_calc_ex_host(tvl1_handle* H, int frame_type, const void* h_frame0, size
     return TVL1_OK;
 }
 
+int tvl1_calc_batch_ex(tvl1_handle* H, int n, int frame_type, const void* const* d_frame0, size_t pitch0,
+                       const void* const* d_frame1, size_t pitch1, int width, int height,
+                       const float* const* d_u0, const float* const* d_v0, size_t pitch_init,
+                       float* const* d_u, float* const* d_v, size_t pitch_out, void* stream, tvl1_stats* stats)
+{
+    if (!H) return fail(TVL1_ERR_INVALID, "handle is null");
+    return calc_batch(H, n, frame_type, d_frame0, pitch0, d_frame1, pitch1, width, height, d_u0, d_v0, pitch_init, d_u, d_v,
+                      pitch_out, (cudaStream_t)stream, stats);
+}
+
 int tvl1_calc_batch_u8(tvl1_handle* H, int n, const uint8_t* const* d_frame0, size_t pitch0,
                        const uint8_t* const* d_frame1, size_t pitch1, int width, int height,
                        float* const* d_u, float* const* d_v, size_t pitch_out, void* stream, tvl1_stats* stats)
 {
     if (!H) return fail(TVL1_ERR_INVALID, "handle is null");
-    return calc_batch(H, n, d_frame0, pitch0, d_frame1, pitch1, width, height, d_u, d_v, pitch_out, (cudaStream_t)stream,
-                      stats);
+    if (H->prm.semantics == TVL1_SEMANTICS_CUDA)
+        return fail(TVL1_ERR_UNSUPPORTED, "tvl1_calc_batch_u8 solves in CPU-class semantics only, not cuda semantics");
+    if (H->prm.gamma != 0.0) return fail(TVL1_ERR_UNSUPPORTED, "tvl1_calc_batch_u8 does not support gamma != 0");
+    return calc_batch(H, n, TVL1_FRAME_U8, (const void* const*)d_frame0, pitch0, (const void* const*)d_frame1, pitch1, width,
+                      height, nullptr, nullptr, 0, d_u, d_v, pitch_out, (cudaStream_t)stream, stats);
 }
 
 int tvl1_last_readbacks(const tvl1_handle* H, long long* n)
@@ -1735,7 +1833,7 @@ int tvl1_k_resize_cuda(const float* d_src, int sw, int sh, int spitch, float* d_
 {
     if (!d_src || !d_dst || sw <= 0 || sh <= 0 || dw <= 0 || dh <= 0 || spitch < sw || dpitch < dw)
         return fail(TVL1_ERR_INVALID, "bad argument");
-    return launch_resize_cuda(resize_args(d_src, nullptr, sw, sh, spitch, d_dst, nullptr, dw, dh, dpitch), inv_scale, mul,
+    return launch_resize_cuda(resize_args(d_src, nullptr, sw, sh, spitch, d_dst, nullptr, dw, dh, dpitch), 1, inv_scale, mul,
                               mul != 1.f, (cudaStream_t)stream);
 }
 

@@ -11,6 +11,8 @@
  *   tvl1_calc_u8 / tvl1_calc_u8_host    <- TVL1_solve (solver->calc)
  *                                          src/optflow.h:31, src/optflow.cpp:516-520
  *   tvl1_calc_batch_u8                  <- TVL1_solve of many equal-size pairs in one call (no counterpart)
+ *   tvl1_calc_batch_ex                  <- the same for tvl1_calc_ex: either semantics, gamma, fp32 frames and
+ *                                          initial flows
  *   tvl1_calc_ex / tvl1_calc_ex_host    <- the rest of the classes' calc(I0, I1, flow): CV_32FC1 frames and
  *                                          useInitialFlow (the reference uses neither)
  *   tvl1_mask_flow_u8                   <- threshold + setTo in solve_wrapper
@@ -151,7 +153,8 @@ int tvl1_calc_u8(tvl1_handle* h, const uint8_t* d_frame0, size_t pitch0,
  * arrays are host memory, their entries device pointers, and entries may repeat.  Every pair's flow and iteration
  * counts are bit-identical to tvl1_calc_u8 of that pair alone.  stats: NULL or n entries (per-pair iters[] / outer[]
  * / totals; ms_total and launches are the batch's).  Synchronises `stream`, as tvl1_calc_u8 does.
- * CPU-class semantics only: TVL1_SEMANTICS_CUDA and gamma != 0 give TVL1_ERR_UNSUPPORTED.  n outside
+ * This is tvl1_calc_batch_ex with TVL1_FRAME_U8 and no initial flow, restricted to CPU-class semantics:
+ * TVL1_SEMANTICS_CUDA and gamma != 0 give TVL1_ERR_UNSUPPORTED here (tvl1_calc_batch_ex solves both).  n outside
  * 1 .. TVL1_BATCH_MAX_PAIRS, a NULL entry or the pitch rules of tvl1_calc_u8: TVL1_ERR_INVALID.  A batch whose
  * state does not fit on the device: TVL1_ERR_NOMEM, with nothing of it left allocated.  The handle keeps the
  * batch's state apart from a single pair's; either call may follow the other. */
@@ -159,6 +162,21 @@ int tvl1_calc_u8(tvl1_handle* h, const uint8_t* d_frame0, size_t pitch0,
 int tvl1_calc_batch_u8(tvl1_handle* h, int n,
                        const uint8_t* const* d_frame0, size_t pitch0,
                        const uint8_t* const* d_frame1, size_t pitch1, int width, int height,
+                       float* const* d_u, float* const* d_v, size_t pitch_out,
+                       void* stream, tvl1_stats* stats);
+
+/* tvl1_calc_batch_u8 for tvl1_calc_ex: n pairs of equal size in the handle's parameters, whatever they are (either
+ * semantics, any gamma).  frame_type and the frames' pitch rules are tvl1_calc_ex's, the same for every pair.
+ * d_u0 and d_v0: both NULL, every pair starts from zero flow; both given, n entries each (none NULL), pair k starts
+ * from d_u0[k] / d_v0[k] (planar fp32, byte pitch pitch_init, a multiple of 4, the same for every pair); an entry may
+ * equal d_u[k] / d_v[k] (OpenCV's flow is in/out) and entries may repeat.  Only one of them given, or a NULL entry:
+ * TVL1_ERR_INVALID.  Pair k's flow, iters[] and outer[] are bit-identical to tvl1_calc_ex of that pair alone, with the
+ * same frame type and initial flow, on a handle with the same parameters; in cuda semantics outer[] is 0, as there.
+ * Everything else is as tvl1_calc_batch_u8: n, NULL entries, TVL1_ERR_NOMEM, stats and the synchronised stream. */
+int tvl1_calc_batch_ex(tvl1_handle* h, int n, int frame_type,
+                       const void* const* d_frame0, size_t pitch0,
+                       const void* const* d_frame1, size_t pitch1, int width, int height,
+                       const float* const* d_u0, const float* const* d_v0, size_t pitch_init,
                        float* const* d_u, float* const* d_v, size_t pitch_out,
                        void* stream, tvl1_stats* stats);
 
